@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Jaccard edges/s of the Phenograph graph-weighting path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json `metric`: "Jaccard edges/s at 4M cells k=30"): a synthetic 4M x 30
@@ -70,7 +70,13 @@ def parse():
     ap.add_argument("--no-traffic-probe", action="store_true", help="do not re-run the kernel under ncu for roofline.traffic")
     ap.add_argument("--traffic-probe", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     shapes = {"cfg1": (10_000, 15), "cfg2": (100_000, 30), "cfg3": (1_000_000, 30), "cfg4": (4_000_000, 30),
               "cfg5": (10_000_000, 100)}
     if a.config != "cfg4":
@@ -307,6 +313,32 @@ def run_traffic_probe(a):
 
 
 # --------------------------------------------------------------------------- GPU arm
+DUMP_EDGE_COLUMNS = 1_500_000  # 36 MB of edges + 12 MB of their positions: a dump stays under 64 MB
+
+
+def dump_outputs(path, out, flags):
+    """--dump-outputs: what the timed path returned in its last step, as .npy files under `path`, so
+    that two builds of the project can be compared output for output on the same seeded input.
+      edges.npy         float64 (3, m): the from / to / weight rows of the (3, E) result; all E columns
+                        when E <= DUMP_EDGE_COLUMNS, else a sample of DUMP_EDGE_COLUMNS columns drawn
+                        with a fixed seed (the same columns in every run with the same E)
+      edge_columns.npy  float64 (m,): the column of the result each edges.npy column is
+      flags.npy         float64: the flag words the path sets (0 = no repeated or invalid ids)"""
+    import numpy as np
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    E = out.shape[1]
+    if E <= DUMP_EDGE_COLUMNS:
+        cols = np.arange(E, dtype=np.int64)
+    else:
+        cols = np.sort(np.random.default_rng(20261020).choice(E, DUMP_EDGE_COLUMNS, replace=False))
+    edges = out[:, torch.from_numpy(cols).to(out.device)].cpu().numpy().astype(np.float64)
+    np.save(os.path.join(path, "edges.npy"), edges)
+    np.save(os.path.join(path, "edge_columns.npy"), cols.astype(np.float64))
+    np.save(os.path.join(path, "flags.npy"), flags.cpu().numpy().astype(np.float64))
+
+
 def network_record(colptr, srows, sw, n, k, a, dev, flush):
     """The bulk steps of the community detection on the device-resident graph (SURVEY 8f row 3): CSR
     network, quality function, reduced network -- timed once each and, unless --no-parity, checked bit
@@ -549,6 +581,8 @@ def run_ours(a):
     else:
         kern_avg_ms = float(step_ms.mean())
     assert int(flags[0]) == 0 and gather_flags == 0, "fast kernel flagged the synthetic input"
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, out, flags)
     total_ms = float(step_ms.sum())
     ms_per_step = total_ms / a.steps
     value = E / (ms_per_step * 1e-3)

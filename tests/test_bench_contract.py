@@ -31,6 +31,43 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr
+
+
+def test_dump_outputs_files(tmp_path):
+    """bench.dump_outputs on CPU tensors: the whole result when it is small, a fixed sample of
+    columns (the same in every run, under 64 MB) when it is large."""
+    import numpy as np
+    import torch
+
+    import bench
+
+    flags = torch.zeros(2, dtype=torch.int32)
+    small = torch.arange(3 * 1000, dtype=torch.float64).reshape(3, 1000)
+    bench.dump_outputs(str(tmp_path / "small"), small, flags)
+    assert np.array_equal(np.load(tmp_path / "small" / "edges.npy"), small.numpy())
+    assert np.array_equal(np.load(tmp_path / "small" / "edge_columns.npy"), np.arange(1000.0))
+    assert np.load(tmp_path / "small" / "flags.npy").dtype == np.float64
+
+    E = 3 * bench.DUMP_EDGE_COLUMNS
+    big = torch.arange(E, dtype=torch.float64).expand(3, E)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), big, flags)
+    total = 0
+    for name in ("edges", "edge_columns", "flags"):
+        x, y = np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy"))
+        assert x.dtype == np.float64 and np.array_equal(x, y)
+        total += os.path.getsize(tmp_path / "a" / (name + ".npy"))
+    assert total < 64e6
+    cols = np.load(tmp_path / "a" / "edge_columns.npy")
+    edges = np.load(tmp_path / "a" / "edges.npy")
+    assert edges.shape == (3, bench.DUMP_EDGE_COLUMNS) and np.unique(cols).size == cols.size
+    assert np.array_equal(edges[0], cols)
+
+
 def test_network_record_of_the_bench_line(monkeypatch, tmp_path):
     """bench.network_record (the `network_next_row` object) driven on CPU tensors through the emulated
     network library: keys, parity record and the planted-community clustering, without a GPU."""

@@ -115,6 +115,26 @@ def test_labels_from_device_graph(cuda, oracle):
     assert np.array_equal(lab_gpu, lab_ref)
 
 
+def test_device_graph_is_the_input_of_the_stored_reference_labels(cuda, oracle):
+    """Label parity with nothing outside the repository: tests/golden/net_snn_900_k12_louvain.npz holds
+    the lower-triangle edge list of this seeded 900 x 12 matrix and the Louvain labels the reference's
+    own ModularityOptimizer returned for it (tests/golden/make_golden.py).  The graph built on the
+    device is that edge list bit for bit, so the reference's optimiser returns those labels for it, and
+    the network of the device graph gives the stored quality value for them."""
+    from gficf_b200 import modularity
+
+    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "net_snn_900_k12_louvain.npz"))
+    n, k = 900, 12
+    idx0 = synth.knn_index(n, k, family="planted", scramble=True)
+    names = louvain.lower_triangle_edges(oracle.parallel(synth.to_r_matrix(idx0)))[0]
+    colptr, rows, w, vcell, flags = _gpu_triangle(n, k, idx0)
+    assert flags & ~16 == 0 and np.array_equal(vcell, names.astype(np.int64))
+    assert np.array_equal(np.repeat(np.arange(vcell.size), np.diff(colptr)), g["node1"])
+    assert np.array_equal(rows, g["node2"]) and np.array_equal(w, g["w"])
+    net = modularity.matrix_to_network(*(torch.from_numpy(x).cuda() for x in (colptr, rows, w)))
+    assert net.calc_quality_function(g["cluster"], float(g["resolution"])) == float(g["quality"])
+
+
 def test_snn_timing_record(cuda):
     """Not a pass/fail gate: prints the device time of the whole step at 1M x 30."""
     from gficf_b200 import device as D, snn
