@@ -1944,6 +1944,109 @@ int gficf_cuda_wmu_test(const double* mat_x, const double* mat_y, int64_t n_gene
   API_END
 }
 
+// One-vs-rest Mann-Whitney U for every cluster in one call: one upload, one sort per gene
+int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, const int32_t* cluster,
+                           int32_t n_clusters, double* out, char* err, size_t errlen) {
+  API_BEGIN
+  if (err && errlen) err[0] = 0;
+  if (n_genes < 0 || n_cells < 0) throw Err{GFICF_E_ARG, "negative matrix dimension"};
+  if (n_clusters < 2) throw Err{GFICF_E_ARG, "one-vs-rest needs at least two clusters"};
+  if (n_clusters > kWmuMaxClusters)
+    throw Err{GFICF_E_LIMIT, fmt("more than %d clusters (the per-CTA rank-sum accumulators)", kWmuMaxClusters)};
+  if (n_cells >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 cells per gene"};
+  if (n_genes == 0) return GFICF_OK;
+  if (!mat || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  std::vector<long long> size((size_t)n_clusters, 0);
+  for (int64_t i = 0; i < n_cells; ++i) {
+    const int32_t c = cluster[i];
+    if (c < 0 || c >= n_clusters)
+      throw Err{GFICF_E_ARG, fmt("cluster id %d of cell %lld is outside [0, %d)", c, (long long)i, n_clusters)};
+    ++size[(size_t)c];
+  }
+  for (int32_t c = 0; c < n_clusters; ++c)
+    if (!size[(size_t)c]) throw Err{GFICF_E_ARG, fmt("cluster %d has no cells", c)};
+  if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
+  std::lock_guard<std::mutex> lk(g_call_mu);
+  int prev_dev = 0;
+  cudaGetDevice(&prev_dev);
+  const auto t0 = std::chrono::steady_clock::now();
+  DeviceWs& ws = g_ws[0];
+  CU_TRY(cudaSetDevice(0));
+  ws.ensure(0);
+  g_active_devices.store(1);
+  const long long N = n_cells, C = n_clusters;
+  const size_t acc_smem = (size_t)C * kWmuClusterSmemBytes;
+  CU_TRY(cudaFuncSetAttribute(wmu_markers_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              kWmuMaxClusters * kWmuClusterSmemBytes));
+  int per_sm = 0;
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_rank_kernel, kWmuThreads, acc_smem));
+  const int grid = (int)std::min<long long>(n_genes, (long long)std::max(1, per_sm) * sm_count());
+  // device buffers: the matrix in in_raw; cluster ids | cluster sizes in idx; per-CTA sort scratch in
+  // scratch (keys) and counts (payload); z | ratio per (gene, cluster) and the per-gene single flags in out
+  const size_t bm = (size_t)n_genes * N * 8, bid = ((size_t)N * 4 + 255) / 256 * 256;
+  ws.in_raw.need(bm);
+  ws.idx.need(bid + (size_t)C * 8);
+  ws.scratch.need((size_t)grid * 2 * N * sizeof(unsigned long long));
+  ws.counts.need((size_t)grid * (3 * N + 2) * sizeof(unsigned));
+  const size_t zc = (size_t)n_genes * C;
+  ws.out.need(zc * 16 + (size_t)n_genes * 4 + 64);
+  double* d_mat = (double*)ws.in_raw.p;
+  int* d_cl = (int*)ws.idx.p;
+  long long* d_size = (long long*)((char*)ws.idx.p + bid);
+  double* d_z = (double*)ws.out.p;
+  double* d_ratio = d_z + zc;
+  int* d_single = (int*)(d_ratio + zc);
+  CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
+  h2d_block(ws, mat, n_genes * N, d_mat, n_genes * N, 1, 8, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, cluster, N, d_cl, N, 1, 4, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, size.data(), C, d_size, C, 1, 8, ws.s_comp, /*ids=*/false);
+  CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
+  wmu_markers_rank_kernel<<<grid, kWmuThreads, acc_smem, ws.s_comp>>>(
+      d_mat, n_genes, N, d_cl, d_size, n_clusters, (unsigned long long*)ws.scratch.p, (unsigned*)ws.counts.p, d_z,
+      d_single);
+  const dim3 mgrid((unsigned)((n_genes + kMeanGenes - 1) / kMeanGenes), (unsigned)((C + kMarkClusters - 1) / kMarkClusters));
+  wmu_markers_means_kernel<<<mgrid, kMarkThreads, 0, ws.s_comp>>>(d_mat, n_genes, N, d_cl, d_size, n_clusters, d_ratio);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
+  std::vector<double> h(zc * 2);
+  std::vector<int> hs((size_t)n_genes);
+  CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaStreamSynchronize(ws.s_comp));
+  // the two transcendental steps per (gene, cluster), as in gficf_cuda_wmu_test; block c of out is
+  // cluster c's n_genes x 2 result.  Clusters are spread over host threads when there are many values.
+  auto finish = [&](long long c_lo, long long c_hi) {
+    for (long long c = c_lo; c < c_hi; ++c) {
+      const double* z = h.data() + (size_t)c * n_genes;
+      const double* ratio = h.data() + zc + (size_t)c * n_genes;
+      double* o = out + (size_t)c * 2 * n_genes;
+      for (int64_t g = 0; g < n_genes; ++g) {
+        o[g] = hs[(size_t)g] ? 1.0 : gficf_host::wmu_pvalue(z[g]);
+        o[n_genes + g] = log2(ratio[g]);
+      }
+    }
+  };
+  const long long nthreads =
+      std::min<long long>({C, (long long)std::max(1u, std::thread::hardware_concurrency()), 16LL,
+                           std::max(1LL, (long long)zc / 16384)});
+  if (nthreads <= 1) {
+    finish(0, C);
+  } else {
+    std::vector<std::thread> th;
+    for (long long t = 0; t < nthreads; ++t) th.emplace_back(finish, C * t / nthreads, C * (t + 1) / nthreads);
+    for (auto& x : th) x.join();
+  }
+  float ms0 = 0, ms1 = 0;
+  CU_TRY(cudaEventElapsedTime(&ms0, ws.ev[0], ws.ev[1]));
+  CU_TRY(cudaEventElapsedTime(&ms1, ws.ev[1], ws.ev[2]));
+  cudaSetDevice(prev_dev);
+  double tm[8] = {ms0, 0, ms1, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
+                  0, 2, (double)zc * 16 + (double)n_genes * 4};
+  memcpy(tl_timings, tm, sizeof tm);
+  return GFICF_OK;
+  API_END
+}
+
 }  // extern "C"
 
 // ---------------------------------------------------------------- network pieces of the community detection (next row 3)

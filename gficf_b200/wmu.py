@@ -41,3 +41,32 @@ def rcpp_parallel_WMU_test(matX, matY, printOutput: bool = False) -> np.ndarray:
     if printOutput:
         sys.stdout.write(_BANNER_DONE)
     return out
+
+
+def rcpp_parallel_WMU_markers(mat, cluster, printOutput: bool = False) -> np.ndarray:
+    """Every cluster's one-vs-rest test in one call: a genes x cells matrix and one 0-based cluster id
+    per cell -> (n_genes, 2, n_clusters) float64 (Fortran order).  out[:, :, c] equals, bit for bit,
+    rcpp_parallel_WMU_test(mat[:, cluster == c], mat[:, cluster != c]); n_clusters = max id + 1, and
+    every id in [0, n_clusters) must have cells."""
+    m = np.asfortranarray(np.asarray(mat), dtype=np.float64)
+    if m.ndim != 2:
+        raise TypeError("a numeric matrix (2-D) is required")
+    cl = np.asarray(cluster)
+    if cl.ndim != 1 or cl.shape[0] != m.shape[1]:
+        raise ValueError("cluster must hold one id per column (cell) of mat")
+    if cl.size and not np.issubdtype(cl.dtype, np.integer):
+        raise TypeError("cluster ids must be integers")
+    if cl.size and (cl.min() < 0 or cl.max() >= 2 ** 31 - 1):
+        raise ValueError("cluster ids must be 0-based and below 2^31 - 1")
+    ids = np.ascontiguousarray(cl, dtype=np.int32)
+    k = int(ids.max()) + 1 if ids.size else 0
+    if printOutput:
+        sys.stdout.write(_BANNER)
+    g = m.shape[0]
+    out = np.empty((g, 2, k), dtype=np.float64, order="F")
+    err = C.create_string_buffer(512)
+    rc = _lib.lib().gficf_cuda_wmu_markers(m.ctypes.data, g, m.shape[1], ids.ctypes.data, k, out.ctypes.data, err, 512)
+    _lib.check(rc, err)
+    if printOutput:
+        sys.stdout.write(_BANNER_DONE)
+    return out

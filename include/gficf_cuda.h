@@ -324,6 +324,19 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
 int gficf_cuda_wmu_test(const double* mat_x, const double* mat_y, int64_t n_genes, int64_t n1, int64_t n2,
                         double* out, char* err, size_t errlen);
 
+/* The loop of findClusterMarkers (R/deGenes.R:44-54) in one call: for every cluster c, cluster c's cells
+ * against all other cells.  mat: n_genes x n_cells doubles, COLUMN-major; cluster: n_cells 0-based ids
+ * in [0, n_clusters); out: n_genes x 2 x n_clusters doubles, column-major.  Block c (out + c*2*n_genes)
+ * is, bit for bit, what gficf_cuda_wmu_test returns for mat[, cluster == c] against
+ * mat[, cluster != c] (both with the cells in ascending order).  The matrix is uploaded once and each
+ * gene sorted once: its ranks, tie groups, tie term and distinct count do not depend on the split,
+ * only the per-cluster rank sums and the two fold-change means do.
+ * GFICF_E_ARG: negative size, null pointer, n_clusters < 2, an id outside [0, n_clusters) or a cluster
+ * without cells.  GFICF_E_LIMIT: more than 8192 clusters (12 bytes of rank-sum accumulators per cluster
+ * in each CTA's shared memory) or n_cells >= 2^31.  Timings as for gficf_cuda_wmu_test.  One device. */
+int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, const int32_t* cluster,
+                           int32_t n_clusters, double* out, char* err, size_t errlen);
+
 /* ---- the data-parallel pieces of the community detection that reads the graph (SURVEY 8f row 3;
  * reference src/ModularityOptimizer.cpp).  The sequential, RNG-ordered local moving loop (:484-583)
  * stays on the host; these are the steps around it that touch every edge:
