@@ -136,6 +136,10 @@ radix_scatter_kernel(const unsigned long long* __restrict__ keys_in, const unsig
 // walking the block pairs.  That one element is added with a real floating-point add, the binade
 // changes, and the walk goes on.  The doubles produced are exactly the sequential chain's.
 //   domain: x[t] >= 0 (0 = skipped element), finite; anything else raises kFlagNetWeight.
+// s == 0 needs no case of its own: it is S = 0 in binade e = -1022, where a zero element is the
+// identity pair and every non-zero element (shift <= 0) saturates, so the walk below finds the first
+// non-zero element and its real addition gives 0 + x = x.  A run of leading zeros (masked sums whose
+// first entries are all masked out) is thus consumed a window at a time like any other stretch.
 // A window of up to 1024 blocks x 4096 elements is processed per step; the window grows while no
 // binade boundary is met.  State lives on the device; the host only reads the position back
 // every few dozen steps.
@@ -246,7 +250,7 @@ seq_blocks_kernel(const double* __restrict__ x, long long n, const SeqState* __r
                   SeqFn* __restrict__ block_fn, unsigned* __restrict__ flags) {
   __shared__ SeqFn s_warp[kSeqThreads / 32];
   const long long t0 = st->t0;
-  if (t0 >= n || st->S == 0) return;  // finished, or s == 0: the next element is added by seq_advance_kernel
+  if (t0 >= n) return;  // finished
   const int nb = st->win_blocks, e = st->e;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   bool bad = false;
@@ -293,20 +297,6 @@ seq_advance_kernel(const double* __restrict__ x, long long n, SeqState* __restri
     return;
   }
   bool bad = false;
-  if (S0 == 0) {  // s == 0: 0.0 + x is x itself
-    if (threadIdx.x == 0) {
-      const double v = x[t0];
-      if (v > 0.0 && v <= 1.7976931348623157e308) {
-        seq_split(v, &st->S, &st->e);
-        st->value = v;
-      } else if (v != 0.0) {
-        atomicOr(flags, kFlagNetWeight);
-      }
-      st->t0 = t0 + 1;
-      if (t0 + 1 >= n) out[0] = st->value * scale;
-    }
-    return;
-  }
   for (int b = threadIdx.x; b < nb; b += kSeqThreads) s_fn[b] = block_fn[b];
   __syncthreads();
   if (threadIdx.x == 0) {
