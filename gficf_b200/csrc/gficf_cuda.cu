@@ -1944,18 +1944,20 @@ int gficf_cuda_wmu_test(const double* mat_x, const double* mat_y, int64_t n_gene
   API_END
 }
 
-// One-vs-rest Mann-Whitney U for every cluster in one call: one upload, one sort per gene
-int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, const int32_t* cluster,
-                           int32_t n_clusters, double* out, char* err, size_t errlen) {
-  API_BEGIN
-  if (err && errlen) err[0] = 0;
+}  // extern "C"
+
+namespace {
+// Argument checks shared by both markers entries: sizes and cluster cap, then every id and every cluster's
+// size (each cluster needs cells).
+void markers_check_sizes(int64_t n_genes, int64_t n_cells, int32_t n_clusters) {
   if (n_genes < 0 || n_cells < 0) throw Err{GFICF_E_ARG, "negative matrix dimension"};
   if (n_clusters < 2) throw Err{GFICF_E_ARG, "one-vs-rest needs at least two clusters"};
   if (n_clusters > kWmuMaxClusters)
     throw Err{GFICF_E_LIMIT, fmt("more than %d clusters (the per-CTA rank-sum accumulators)", kWmuMaxClusters)};
   if (n_cells >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 cells per gene"};
-  if (n_genes == 0) return GFICF_OK;
-  if (!mat || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
+}
+
+std::vector<long long> markers_cluster_sizes(const int32_t* cluster, int64_t n_cells, int32_t n_clusters) {
   std::vector<long long> size((size_t)n_clusters, 0);
   for (int64_t i = 0; i < n_cells; ++i) {
     const int32_t c = cluster[i];
@@ -1965,6 +1967,51 @@ int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, 
   }
   for (int32_t c = 0; c < n_clusters; ++c)
     if (!size[(size_t)c]) throw Err{GFICF_E_ARG, fmt("cluster %d has no cells", c)};
+  return size;
+}
+
+// Host finish of both markers entries: the two transcendental steps per (gene, cluster), as in
+// gficf_cuda_wmu_test.  h = z | ratio, each n_clusters blocks of n_genes; block c of out is cluster c's
+// n_genes x 2 result.  Clusters are spread over host threads when there are many values.
+void markers_finish(const std::vector<double>& h, const std::vector<int>& hs, int64_t n_genes, int32_t n_clusters,
+                    double* out) {
+  const long long C = n_clusters;
+  const size_t zc = (size_t)n_genes * C;
+  auto finish = [&](long long c_lo, long long c_hi) {
+    for (long long c = c_lo; c < c_hi; ++c) {
+      const double* z = h.data() + (size_t)c * n_genes;
+      const double* ratio = h.data() + zc + (size_t)c * n_genes;
+      double* o = out + (size_t)c * 2 * n_genes;
+      for (int64_t g = 0; g < n_genes; ++g) {
+        o[g] = hs[(size_t)g] ? 1.0 : gficf_host::wmu_pvalue(z[g]);
+        o[n_genes + g] = log2(ratio[g]);
+      }
+    }
+  };
+  const long long nthreads =
+      std::min<long long>({C, (long long)std::max(1u, std::thread::hardware_concurrency()), 16LL,
+                           std::max(1LL, (long long)zc / 16384)});
+  if (nthreads <= 1) {
+    finish(0, C);
+  } else {
+    std::vector<std::thread> th;
+    for (long long t = 0; t < nthreads; ++t) th.emplace_back(finish, C * t / nthreads, C * (t + 1) / nthreads);
+    for (auto& x : th) x.join();
+  }
+}
+}  // namespace
+
+extern "C" {
+
+// One-vs-rest Mann-Whitney U for every cluster in one call: one upload, one sort per gene
+int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, const int32_t* cluster,
+                           int32_t n_clusters, double* out, char* err, size_t errlen) {
+  API_BEGIN
+  if (err && errlen) err[0] = 0;
+  markers_check_sizes(n_genes, n_cells, n_clusters);
+  if (n_genes == 0) return GFICF_OK;
+  if (!mat || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  const std::vector<long long> size = markers_cluster_sizes(cluster, n_cells, n_clusters);
   if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
   std::lock_guard<std::mutex> lk(g_call_mu);
   int prev_dev = 0;
@@ -2013,29 +2060,7 @@ int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, 
   CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
   CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
   CU_TRY(cudaStreamSynchronize(ws.s_comp));
-  // the two transcendental steps per (gene, cluster), as in gficf_cuda_wmu_test; block c of out is
-  // cluster c's n_genes x 2 result.  Clusters are spread over host threads when there are many values.
-  auto finish = [&](long long c_lo, long long c_hi) {
-    for (long long c = c_lo; c < c_hi; ++c) {
-      const double* z = h.data() + (size_t)c * n_genes;
-      const double* ratio = h.data() + zc + (size_t)c * n_genes;
-      double* o = out + (size_t)c * 2 * n_genes;
-      for (int64_t g = 0; g < n_genes; ++g) {
-        o[g] = hs[(size_t)g] ? 1.0 : gficf_host::wmu_pvalue(z[g]);
-        o[n_genes + g] = log2(ratio[g]);
-      }
-    }
-  };
-  const long long nthreads =
-      std::min<long long>({C, (long long)std::max(1u, std::thread::hardware_concurrency()), 16LL,
-                           std::max(1LL, (long long)zc / 16384)});
-  if (nthreads <= 1) {
-    finish(0, C);
-  } else {
-    std::vector<std::thread> th;
-    for (long long t = 0; t < nthreads; ++t) th.emplace_back(finish, C * t / nthreads, C * (t + 1) / nthreads);
-    for (auto& x : th) x.join();
-  }
+  markers_finish(h, hs, n_genes, n_clusters, out);
   float ms0 = 0, ms1 = 0;
   CU_TRY(cudaEventElapsedTime(&ms0, ws.ev[0], ws.ev[1]));
   CU_TRY(cudaEventElapsedTime(&ms1, ws.ev[1], ws.ev[2]));
@@ -2094,6 +2119,121 @@ int gficf_cuda_network_reduce_dev(const int64_t* d_first, const int32_t* d_neigh
                           d_r_first, d_r_neighbor, d_r_edge_w, r_cap, d_r_node_w, d_r_self_links, d_r_total_w,
                           n_reduced_edges, d_scratch, scratch_bytes, d_flags, (cudaStream_t)stream, sm_count() * 8);
   DEV_END
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------- Mann-Whitney markers from a sparse matrix
+#include "wmu_csc_plan.h"
+
+extern "C" {
+
+// gficf_cuda_wmu_markers on a compressed-column matrix: the stored values are uploaded, made gene-major on
+// the device (wmu_csc_to_genes) and only they are read by the rank and means kernels.
+int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const double* x, int64_t n_genes,
+                               int64_t n_cells, const int32_t* cluster, int32_t n_clusters, double* out, char* err,
+                               size_t errlen) {
+  API_BEGIN
+  if (err && errlen) err[0] = 0;
+  markers_check_sizes(n_genes, n_cells, n_clusters);
+  if (n_genes == 0) return GFICF_OK;
+  if (n_genes >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 genes (R's int row ids)"};
+  if (!colptr || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  if (colptr[0] != 0) throw Err{GFICF_E_ARG, fmt("colptr[0] is %d, not 0", colptr[0])};
+  for (int64_t j = 0; j < n_cells; ++j)
+    if (colptr[j + 1] < colptr[j])
+      throw Err{GFICF_E_ARG, fmt("colptr decreases at column %lld (%d after %d)", (long long)j, colptr[j + 1], colptr[j])};
+  const long long nnz = colptr[n_cells];
+  if (nnz > 0 && (!row || !x)) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  const std::vector<long long> size = markers_cluster_sizes(cluster, n_cells, n_clusters);
+  if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
+  std::lock_guard<std::mutex> lk(g_call_mu);
+  int prev_dev = 0;
+  cudaGetDevice(&prev_dev);
+  const auto t0 = std::chrono::steady_clock::now();
+  DeviceWs& ws = g_ws[0];
+  CU_TRY(cudaSetDevice(0));
+  ws.ensure(0);
+  g_active_devices.store(1);
+  const long long N = n_cells, C = n_clusters;
+  const WmuClusterLists cl = wmu_cluster_lists(cluster, N, n_clusters);
+  // device buffers: colptr | row | x in in_raw; cluster ids | crank | members | cluster sizes | cptr in idx;
+  // the transpose's scratch in scratch (the gene-major values end up there); per-CTA sort scratch of the
+  // rank kernel in counts; z | ratio per (gene, cluster) and the per-gene single flags in out
+  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
+  const size_t b_cp = al((size_t)(N + 1) * 4), b_row = al((size_t)nnz * 4), b_x = (size_t)nnz * 8;
+  ws.in_raw.need(b_cp + b_row + b_x + 8);
+  const size_t b_cell = al((size_t)N * 4), b_size = al((size_t)C * 8);
+  ws.idx.need(3 * b_cell + b_size + (size_t)(C + 1) * 8);
+  ws.scratch.need(wmu_csc_layout(nullptr, n_genes, nnz).bytes);
+  const WmuCscScratch sc = wmu_csc_layout((char*)ws.scratch.p, n_genes, nnz);
+  const size_t zc = (size_t)n_genes * C;
+  ws.out.need(zc * 16 + (size_t)n_genes * 4 + 64);
+  int* d_colptr = (int*)ws.in_raw.p;
+  int* d_row = (int*)((char*)ws.in_raw.p + b_cp);
+  double* d_x = (double*)((char*)ws.in_raw.p + b_cp + b_row);
+  int* d_cl = (int*)ws.idx.p;
+  int* d_crank = (int*)((char*)ws.idx.p + b_cell);
+  int* d_members = (int*)((char*)ws.idx.p + 2 * b_cell);
+  long long* d_size = (long long*)((char*)ws.idx.p + 3 * b_cell);
+  long long* d_cptr = (long long*)((char*)ws.idx.p + 3 * b_cell + b_size);
+  double* d_z = (double*)ws.out.p;
+  double* d_ratio = d_z + zc;
+  int* d_single = (int*)(d_ratio + zc);
+  CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
+  h2d_block(ws, colptr, N + 1, d_colptr, N + 1, 1, 4, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, row, nnz, d_row, nnz, 1, 4, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, x, nnz, d_x, nnz, 1, 8, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, cluster, N, d_cl, N, 1, 4, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, cl.crank.data(), N, d_crank, N, 1, 4, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, cl.members.data(), N, d_members, N, 1, 4, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, size.data(), C, d_size, C, 1, 8, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, cl.cptr.data(), C + 1, d_cptr, C + 1, 1, 8, ws.s_comp, /*ids=*/false);
+  CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
+  const WmuGeneMajor gm = wmu_csc_to_genes(ws.s_comp, sc, sm_count() * 8, d_colptr, d_row, d_x, n_genes, N, nnz);
+  CU_TRY(cudaGetLastError());
+  // the row-id flag and the gene pointers (they size the rank kernel's scratch) before anything reads them
+  unsigned flags = 0;
+  std::vector<long long> gptr((size_t)n_genes + 1);
+  CU_TRY(cudaMemcpyAsync(&flags, sc.flags, 4, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaMemcpyAsync(gptr.data(), sc.gene_ptr, gptr.size() * 8, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaStreamSynchronize(ws.s_comp));
+  if (flags & kFlagCscRow)
+    throw Err{GFICF_E_ARG, "a row id is outside [0, n_genes) or row ids are not strictly increasing in a column"};
+  long long cap = 1;
+  for (int64_t g = 0; g < n_genes; ++g) cap = std::max(cap, gptr[(size_t)g + 1] - gptr[(size_t)g]);
+  const size_t acc_smem = (size_t)C * kWmuClusterSmemBytes;
+  CU_TRY(cudaFuncSetAttribute(wmu_markers_csr_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              kWmuMaxClusters * kWmuClusterSmemBytes));
+  int per_sm = 0;
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_csr_rank_kernel, kWmuThreads, acc_smem));
+  const int grid = (int)std::min<long long>(n_genes, (long long)std::max(1, per_sm) * sm_count());
+  ws.counts.need((size_t)grid * 2 * cap * (sizeof(unsigned long long) + sizeof(unsigned)));
+  unsigned long long* d_keys = (unsigned long long*)ws.counts.p;
+  unsigned* d_pay = (unsigned*)(d_keys + (size_t)grid * 2 * cap);
+  wmu_markers_csr_rank_kernel<<<grid, kWmuThreads, acc_smem, ws.s_comp>>>(
+      gm.ent_x, gm.ent_cell, sc.gene_ptr, n_genes, N, d_cl, d_size, n_clusters, cap, d_keys, d_pay, d_z, d_single);
+  const int mthreads = wmu_csr_means_threads(n_clusters);
+  const dim3 mgrid((unsigned)n_genes, (unsigned)((C + mthreads - 1) / mthreads));
+  wmu_markers_csr_means_kernel<<<mgrid, mthreads, 0, ws.s_comp>>>(gm.ent_x, gm.ent_cell, sc.gene_ptr, n_genes, N, d_cl,
+                                                                  d_crank, d_members, d_cptr, n_clusters, d_ratio);
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
+  std::vector<double> h(zc * 2);
+  std::vector<int> hs((size_t)n_genes);
+  CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaStreamSynchronize(ws.s_comp));
+  markers_finish(h, hs, n_genes, n_clusters, out);
+  float ms0 = 0, ms1 = 0;
+  CU_TRY(cudaEventElapsedTime(&ms0, ws.ev[0], ws.ev[1]));
+  CU_TRY(cudaEventElapsedTime(&ms1, ws.ev[1], ws.ev[2]));
+  cudaSetDevice(prev_dev);
+  double tm[8] = {ms0, 0, ms1, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
+                  0, (double)(7 + 5 * ((bits_for(n_genes - 1) + 7) / 8)), (double)zc * 16 + (double)n_genes * 4 + 4 + (double)gptr.size() * 8};
+  memcpy(tl_timings, tm, sizeof tm);
+  return GFICF_OK;
+  API_END
 }
 
 }  // extern "C"

@@ -92,7 +92,7 @@ __device__ __forceinline__ double wmu_z(const WmuGeneOut& o, long long n1, long 
 // simply has M = N.
 // ---------------------------------------------------------------------------
 
-// Shared memory of the per-gene sort and tie-group pass (wmu_load_sort, wmu_tie_groups).
+// Shared memory of the per-gene sort and tie-group pass (wmu_load, wmu_sort, wmu_tie_groups).
 struct WmuSortSmem {
   unsigned hist[256];
   unsigned base[256];
@@ -103,20 +103,21 @@ struct WmuSortSmem {
   unsigned carry, flag, m, z1, neg, negties;
 };
 
-// A gene after wmu_load_sort: its M non-zero values sorted (keys, payload = position in the row) in
-// buffer `cur`; nz = N - M zeros, n_neg negative values, z1 zeros among positions [0, n1).
+// A gene after wmu_load (and wmu_sort): its M non-zero values sorted (keys, payload = the value's position)
+// in buffer `cur`; nz = N - M zeros, n_neg negative values, z1 zeros among positions [0, n1).
 struct WmuSorted {
   long long M, nz, n_neg, z1;
   int cur;
 };
 
-// Gene g's row of N values -- positions [0, n1) from mat_x, the rest from mat_y -- with its non-zero
-// values compacted and radix-sorted.  Called by every thread of the CTA; ends on a barrier.
-__device__ __forceinline__ WmuSorted wmu_load_sort(const double* __restrict__ mat_x, const double* __restrict__ mat_y,
-                                                   long long n_genes, long long g, long long n1, long long N,
-                                                   unsigned long long* k0, unsigned long long* k1, unsigned* p0,
-                                                   unsigned* p1, WmuSortSmem& sm) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+// Load step: the n_items values item(i, &pos) of a gene of N cells (n_items == N for a dense row; the
+// stored values for a sparse one, the other N - n_items cells being zeros) -- non-zero values are appended
+// in any order to k0 / p0 as (key, position); zeros, stored or not, are counted.  Called by every thread
+// of the CTA; ends on a barrier.
+template <class Item>
+__device__ __forceinline__ WmuSorted wmu_load(long long n_items, long long n1, long long N, unsigned long long* k0,
+                                              unsigned* p0, WmuSortSmem& sm, Item item) {
+  const int tid = threadIdx.x, lane = tid & 31;
   const unsigned lt_mask = (1u << lane) - 1u;
   if (tid == 0) {
     sm.m = 0;
@@ -124,16 +125,15 @@ __device__ __forceinline__ WmuSorted wmu_load_sort(const double* __restrict__ ma
     sm.neg = 0;
   }
   __syncthreads();
-  // ---- the gene's row: element (g, c) of a column-major matrix sits at g + c * n_genes.
-  //      Non-zero values are appended (any order) as (key, original position); zeros are counted.
-  for (long long t0 = 0; t0 < N; t0 += kWmuThreads) {
+  for (long long t0 = 0; t0 < n_items; t0 += kWmuThreads) {
     const long long i = t0 + tid;
     double v = 0.0;
-    const bool in = i < N;
-    if (in) v = i < n1 ? __ldg(mat_x + g + i * n_genes) : __ldg(mat_y + g + (i - n1) * n_genes);
+    unsigned p = 0;
+    const bool in = i < n_items;
+    if (in) v = item(i, &p);
     const bool nzv = in && v != 0.0;  // -0.0 == 0.0: same tie group as +0.0, like in the reference
     const unsigned m_nz = __ballot_sync(0xffffffffu, nzv);
-    const unsigned m_z1 = __ballot_sync(0xffffffffu, in && !nzv && i < n1);
+    const unsigned m_z1 = __ballot_sync(0xffffffffu, in && !nzv && (long long)p < n1);
     const unsigned m_neg = __ballot_sync(0xffffffffu, nzv && v < 0.0);
     unsigned wbase = 0;
     if (lane == 0) {
@@ -145,7 +145,7 @@ __device__ __forceinline__ WmuSorted wmu_load_sort(const double* __restrict__ ma
     if (nzv) {
       const unsigned pos = wbase + __popc(m_nz & lt_mask);
       k0[pos] = wmu_key(v);
-      p0[pos] = (unsigned)i;
+      p0[pos] = p;
     }
   }
   __syncthreads();
@@ -154,9 +154,28 @@ __device__ __forceinline__ WmuSorted wmu_load_sort(const double* __restrict__ ma
   s.nz = N - s.M;
   s.z1 = sm.z1;
   s.n_neg = sm.neg;
+  s.cur = 0;
+  return s;
+}
+
+// Gene g's dense row of N values -- positions [0, n1) from mat_x, the rest from mat_y; element (g, c) of a
+// column-major matrix sits at g + c * n_genes.
+__device__ __forceinline__ WmuSorted wmu_load_dense(const double* __restrict__ mat_x, const double* __restrict__ mat_y,
+                                                    long long n_genes, long long g, long long n1, long long N,
+                                                    unsigned long long* k0, unsigned* p0, WmuSortSmem& sm) {
+  return wmu_load(N, n1, N, k0, p0, sm, [&](long long i, unsigned* p) {
+    *p = (unsigned)i;
+    return i < n1 ? __ldg(mat_x + g + i * n_genes) : __ldg(mat_y + g + (i - n1) * n_genes);
+  });
+}
+
+// Sort step: LSD radix sort of the M loaded keys, 8 bits per pass; sets s.cur.  Ends on a barrier.
+__device__ __forceinline__ void wmu_sort(WmuSorted& s, unsigned long long* k0, unsigned long long* k1, unsigned* p0,
+                                         unsigned* p1, WmuSortSmem& sm) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const unsigned lt_mask = (1u << lane) - 1u;
   const long long M = s.M;
   int cur = 0;
-  // ---- LSD radix sort of the M non-zero keys, 8 bits per pass
   for (int pass = 0; pass < 8 && M > 1; ++pass) {
     const int shift = pass * 8;
     if (tid < 256) sm.hist[tid] = 0;
@@ -237,7 +256,6 @@ __device__ __forceinline__ WmuSorted wmu_load_sort(const double* __restrict__ ma
     __syncthreads();
   }
   s.cur = cur;
-  return s;
 }
 
 // The tie groups of a sorted gene: the thread that sits on the first element of a group finds the
@@ -361,7 +379,8 @@ wmu_rank_kernel(const double* __restrict__ mat_x, const double* __restrict__ mat
   unsigned* const px = p0 + 2 * N;  // [M+1]
 
   for (long long g = blockIdx.x; g < n_genes; g += gridDim.x) {
-    const WmuSorted s = wmu_load_sort(mat_x, mat_y, n_genes, g, n1, N, k0, k1, p0, p1, sm);
+    WmuSorted s = wmu_load_dense(mat_x, mat_y, n_genes, g, n1, N, k0, p0, sm);
+    wmu_sort(s, k0, k1, p0, p1, sm);
     const long long M = s.M;
     const unsigned long long* keys = s.cur ? k1 : k0;
     const unsigned* pays = s.cur ? p1 : p0;
@@ -429,6 +448,61 @@ wmu_rank_kernel(const double* __restrict__ mat_x, const double* __restrict__ mat
 constexpr int kWmuClusterSmemBytes = 12;
 constexpr int kWmuMaxClusters = 8192;  // 96 KiB of accumulators: two CTAs still fit an SM's shared memory
 
+// Everything of one gene after its load step, shared by both markers kernels: sort, every cluster's rank
+// sum, tie groups, z per (gene, cluster).  The payload of a loaded value is its cell.  s_tr / s_nnz must
+// be zero on entry.  Called by every thread; ends on a barrier.
+__device__ __forceinline__ void wmu_markers_gene(WmuSorted s, long long g, long long n_genes, long long N,
+                                                 const int* __restrict__ cluster,
+                                                 const long long* __restrict__ cluster_size, int n_clusters,
+                                                 unsigned long long* k0, unsigned long long* k1, unsigned* p0,
+                                                 unsigned* p1, unsigned long long* s_tr, unsigned* s_nnz,
+                                                 WmuSortSmem& sm, WmuGeneOut& s_out, double* __restrict__ out_z,
+                                                 int* __restrict__ out_single) {
+  const int tid = threadIdx.x;
+  const unsigned long long kZeroKey = 0x8000000000000000ull;  // wmu_key(0.0)
+  wmu_sort(s, k0, k1, p0, p1, sm);
+  const long long M = s.M;
+  const unsigned long long* keys = s.cur ? k1 : k0;
+  const unsigned* pays = s.cur ? p1 : p0;
+  for (long long i = tid; i < M; i += kWmuThreads) {
+    const unsigned long long key = keys[i];
+    long long lo = i, hi = i + 1;
+    if (i > 0 && keys[i - 1] == key) {  // first position whose key equals this one
+      long long a = 0, b = i - 1;
+      while (a < b) {
+        const long long mid = (a + b) >> 1;
+        if (keys[mid] < key) a = mid + 1;
+        else b = mid;
+      }
+      lo = a;
+    }
+    if (hi < M && keys[hi] == key) {  // first position > i whose key differs
+      long long a = hi + 1, b = M;
+      while (a < b) {
+        const long long mid = (a + b) >> 1;
+        if (keys[mid] == key) a = mid + 1;
+        else b = mid;
+      }
+      hi = a;
+    }
+    const long long off = key > kZeroKey ? s.nz : 0;
+    const int c = __ldg(cluster + pays[i]);
+    atomicAdd(&s_tr[c], (unsigned long long)(lo + hi + 2 * off + 1));
+    atomicAdd(&s_nnz[c], 1u);
+  }
+  wmu_tie_groups(keys, s, N, reinterpret_cast<double*>(s.cur ? k0 : k1), sm, s_out,
+                 [](long long, long long, long long) {});
+  for (int c = tid; c < n_clusters; c += kWmuThreads) {
+    const long long nc = cluster_size[c];
+    WmuGeneOut o = s_out;
+    o.two_r1 = s_tr[c] + (unsigned long long)(nc - s_nnz[c]) * (unsigned long long)(2 * s.n_neg + s.nz + 1);
+    int single;
+    out_z[(size_t)c * n_genes + g] = wmu_z(o, nc, N - nc, &single);
+    if (c == 0) out_single[g] = single;
+  }
+  __syncthreads();
+}
+
 __global__ void __launch_bounds__(kWmuThreads, 2)
 wmu_markers_rank_kernel(const double* __restrict__ mat, long long n_genes, long long n_cells,
                         const int* __restrict__ cluster, const long long* __restrict__ cluster_size, int n_clusters,
@@ -442,7 +516,6 @@ wmu_markers_rank_kernel(const double* __restrict__ mat, long long n_genes, long 
 
   const long long N = n_cells;
   const int tid = threadIdx.x;
-  const unsigned long long kZeroKey = 0x8000000000000000ull;  // wmu_key(0.0)
   unsigned long long* const k0 = scratch_keys + (size_t)blockIdx.x * 2 * N;
   unsigned long long* const k1 = k0 + N;
   unsigned* const p0 = scratch_pay + (size_t)blockIdx.x * (3 * N + 2);
@@ -453,47 +526,47 @@ wmu_markers_rank_kernel(const double* __restrict__ mat, long long n_genes, long 
       s_tr[c] = 0;
       s_nnz[c] = 0;
     }
-    const WmuSorted s = wmu_load_sort(mat, mat, n_genes, g, N, N, k0, k1, p0, p1, sm);
-    const long long M = s.M;
-    const unsigned long long* keys = s.cur ? k1 : k0;
-    const unsigned* pays = s.cur ? p1 : p0;
-    for (long long i = tid; i < M; i += kWmuThreads) {
-      const unsigned long long key = keys[i];
-      long long lo = i, hi = i + 1;
-      if (i > 0 && keys[i - 1] == key) {  // first position whose key equals this one
-        long long a = 0, b = i - 1;
-        while (a < b) {
-          const long long mid = (a + b) >> 1;
-          if (keys[mid] < key) a = mid + 1;
-          else b = mid;
-        }
-        lo = a;
-      }
-      if (hi < M && keys[hi] == key) {  // first position > i whose key differs
-        long long a = hi + 1, b = M;
-        while (a < b) {
-          const long long mid = (a + b) >> 1;
-          if (keys[mid] == key) a = mid + 1;
-          else b = mid;
-        }
-        hi = a;
-      }
-      const long long off = key > kZeroKey ? s.nz : 0;
-      const int c = __ldg(cluster + pays[i]);
-      atomicAdd(&s_tr[c], (unsigned long long)(lo + hi + 2 * off + 1));
-      atomicAdd(&s_nnz[c], 1u);
-    }
-    wmu_tie_groups(keys, s, N, reinterpret_cast<double*>(s.cur ? k0 : k1), sm, s_out,
-                   [](long long, long long, long long) {});
+    const WmuSorted s = wmu_load_dense(mat, mat, n_genes, g, N, N, k0, p0, sm);
+    wmu_markers_gene(s, g, n_genes, N, cluster, cluster_size, n_clusters, k0, k1, p0, p1, s_tr, s_nnz, sm, s_out,
+                     out_z, out_single);
+  }
+}
+
+// The same for a gene-major sparse matrix (wmu_csc_to_genes below): gene g's stored values are
+// ent_x[gene_ptr[g] .. gene_ptr[g + 1]) at cells ent_cell[...], cells ascending; every other cell is 0.
+// Only the stored values are read.  Scratch per CTA: keys[2][cap] | pay[2][cap], cap >= the largest
+// number of stored values of a gene.
+__global__ void __launch_bounds__(kWmuThreads, 2)
+wmu_markers_csr_rank_kernel(const double* __restrict__ ent_x, const unsigned* __restrict__ ent_cell,
+                            const long long* __restrict__ gene_ptr, long long n_genes, long long n_cells,
+                            const int* __restrict__ cluster, const long long* __restrict__ cluster_size,
+                            int n_clusters, long long cap, unsigned long long* __restrict__ scratch_keys,
+                            unsigned* __restrict__ scratch_pay, double* __restrict__ out_z,
+                            int* __restrict__ out_single) {
+  __shared__ WmuSortSmem sm;
+  __shared__ WmuGeneOut s_out;
+  GFICF_DYNAMIC_SMEM_T(unsigned long long, wmu_cluster_acc);
+  unsigned long long* const s_tr = wmu_cluster_acc;
+  unsigned* const s_nnz = reinterpret_cast<unsigned*>(wmu_cluster_acc + n_clusters);
+
+  const int tid = threadIdx.x;
+  unsigned long long* const k0 = scratch_keys + (size_t)blockIdx.x * 2 * cap;
+  unsigned long long* const k1 = k0 + cap;
+  unsigned* const p0 = scratch_pay + (size_t)blockIdx.x * 2 * cap;
+  unsigned* const p1 = p0 + cap;
+
+  for (long long g = blockIdx.x; g < n_genes; g += gridDim.x) {
     for (int c = tid; c < n_clusters; c += kWmuThreads) {
-      const long long nc = cluster_size[c];
-      WmuGeneOut o = s_out;
-      o.two_r1 = s_tr[c] + (unsigned long long)(nc - s_nnz[c]) * (unsigned long long)(2 * s.n_neg + s.nz + 1);
-      int single;
-      out_z[(size_t)c * n_genes + g] = wmu_z(o, nc, N - nc, &single);
-      if (c == 0) out_single[g] = single;
+      s_tr[c] = 0;
+      s_nnz[c] = 0;
     }
-    __syncthreads();
+    const long long lo = gene_ptr[g];
+    const WmuSorted s = wmu_load(gene_ptr[g + 1] - lo, 0, n_cells, k0, p0, sm, [&](long long i, unsigned* p) {
+      *p = __ldg(ent_cell + lo + i);
+      return __ldg(ent_x + lo + i);
+    });
+    wmu_markers_gene(s, g, n_genes, n_cells, cluster, cluster_size, n_clusters, k0, k1, p0, p1, s_tr, s_nnz, sm,
+                     s_out, out_z, out_single);
   }
 }
 
@@ -619,6 +692,141 @@ wmu_markers_means_kernel(const double* __restrict__ mat, long long n_genes, long
     out_ratio[(size_t)c * n_genes + g0 + lane] =
         __ddiv_rn(__ddiv_rn(s_in, (double)nc), __ddiv_rn(s_out, (double)(n_cells - nc)));
   }
+}
+
+// ---------------------------------------------------------------------------
+// Sparse input: a genes x cells matrix in compressed-column form (R's dgCMatrix: colptr = p, row = i,
+// x), turned gene-major on the device, then the two markers kernels read only the stored values.
+// ---------------------------------------------------------------------------
+constexpr unsigned kFlagCscRow = 1u;  // a row id outside [0, n_genes), or row ids not strictly increasing in a column
+
+// Transpose, step 1 (warp per column): checks every row id before anything indexes with it, and writes
+// the radix-sort input key = gene, payload = entry index, the entry's cell, and the per-gene counts.
+// A bad entry raises kFlagCscRow and gets key 0 (the sort stays in bounds; the call then fails).
+__global__ void __launch_bounds__(256)
+wmu_csc_keys_kernel(const int* __restrict__ colptr, const int* __restrict__ row, long long n_cells, long long n_genes,
+                    unsigned* __restrict__ col_of, unsigned long long* __restrict__ keys, unsigned* __restrict__ vals,
+                    int* __restrict__ gene_cnt, unsigned* __restrict__ flags) {
+  const int lane = threadIdx.x & 31;
+  const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
+  bool bad = false;
+  for (long long c = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); c < n_cells; c += nwarps) {
+    const long long lo = colptr[c], hi = colptr[c + 1];
+    for (long long e = lo + lane; e < hi; e += 32) {
+      const int r = row[e];
+      col_of[e] = (unsigned)c;
+      vals[e] = (unsigned)e;
+      if (r >= 0 && r < n_genes && (e == lo || row[e - 1] < r)) {
+        keys[e] = (unsigned long long)r;
+        atomicAdd(gene_cnt + r, 1);
+      } else {
+        keys[e] = 0;
+        bad = true;
+      }
+    }
+  }
+  if (bad) atomicOr(flags, kFlagCscRow);
+}
+
+// Transpose, step 3 (after the stable sort by gene): sorted position q holds entry vals[q]; the entries of a
+// gene keep their column order, so its cells are ascending.
+__global__ void __launch_bounds__(256)
+wmu_csc_gather_kernel(const unsigned* __restrict__ vals, const unsigned* __restrict__ col_of,
+                      const double* __restrict__ x, long long nnz, unsigned* __restrict__ ent_cell,
+                      double* __restrict__ ent_x) {
+  for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < nnz; q += (long long)gridDim.x * blockDim.x) {
+    const unsigned e = vals[q];
+    ent_cell[q] = col_of[e];
+    ent_x[q] = x[e];
+  }
+}
+
+// s + 1.0 + 1.0 + ... (m additions, each rounded), replayed in O(binades) steps.  While ulp(s) <= 1, adding
+// an integer is exact as long as the result stays within s's binade or reaches its upper end 2^(e+1)
+// (s >= 0), or does not pass 0 (s < 0): those steps are taken in one addition.  The step that leaves that
+// range is a real addition (where rounding happens).  Above 2^53, s + 1 rounds back to s after at most one
+// step (ties to even), and the run stops there.  Bit-identical to the loop, sign of zero included.
+__device__ __forceinline__ double wmu_ones_run(double s, long long m) {
+  while (m > 0) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(s);
+    const int ef = (int)((b >> 52) & 0x7ffu);
+    long long t = 0;
+    if (ef <= 1023 + 52) {  // ulp(s) <= 1
+      t = (b >> 63) ? (long long)(-s)
+                    : (long long)__dadd_rn(__longlong_as_double((long long)((unsigned long long)(ef + 1) << 52)), -s);
+      if (t > m) t = m;
+    }
+    if (t > 0) {
+      s = __dadd_rn(s, (double)t);
+      m -= t;
+      continue;
+    }
+    const double n = __dadd_rn(s, 1.0);
+    --m;
+    if (n == s || n != n) break;  // a fixed point (or NaN): every further step gives the same
+    s = n;
+  }
+  return s;
+}
+
+// Fold-change means from the gene-major sparse matrix: for each (gene, cluster c) the same two sequential
+// chains as wmu_markers_means_kernel -- sum(v + 1) over c's cells and over all other cells, in cell order --
+// walking only the gene's stored values.  The zeros between two stored values of a chain are a run of
+// additions of 1.0, replayed by wmu_ones_run.  Run lengths: in-chain, the difference of the cells' ranks
+// inside c (crank[cell], the cell's rank inside its own cluster); out-chain, the difference of the cells'
+// positions among the non-c cells, cell - #{c cells below it}, with the count found in c's ascending cell
+// list (members[cptr[c] ..]) by a galloping search that only moves forward.
+// Thread = cluster blockIdx.y * blockDim.x + threadIdx.x of gene blockIdx.x.
+// out_ratio[c * n_genes + g] = avg_in / avg_out.
+__global__ void __launch_bounds__(128)
+wmu_markers_csr_means_kernel(const double* __restrict__ ent_x, const unsigned* __restrict__ ent_cell,
+                             const long long* __restrict__ gene_ptr, long long n_genes, long long n_cells,
+                             const int* __restrict__ cluster, const int* __restrict__ crank,
+                             const int* __restrict__ members, const long long* __restrict__ cptr, int n_clusters,
+                             double* __restrict__ out_ratio) {
+  const long long g = blockIdx.x;
+  const int c = (int)(blockIdx.y * blockDim.x + threadIdx.x);
+  if (c >= n_clusters) return;
+  const long long lo = gene_ptr[g], hi = gene_ptr[g + 1];
+  const int* const L = members + cptr[c];
+  const long long nc = cptr[c + 1] - cptr[c];
+  double s_in = 0.0, s_out = 0.0;
+  long long in_next = 0, out_next = 0;  // chain positions of the next value of each chain
+  long long p = 0;                      // c cells below the current cell: L[0, p) < cell
+  long long next_c = nc > 0 ? L[0] : n_cells;  // L[p]
+  for (long long q = lo; q < hi; ++q) {
+    const long long cell = __ldg(ent_cell + q);
+    const double v1 = __dadd_rn(__ldg(ent_x + q), 1.0);
+    if (__ldg(cluster + cell) == c) {
+      const long long r = __ldg(crank + cell);
+      s_in = __dadd_rn(wmu_ones_run(s_in, r - in_next), v1);
+      in_next = r + 1;
+      p = r + 1;
+      next_c = p < nc ? __ldg(L + p) : n_cells;
+    } else {
+      if (next_c < cell) {  // first index >= p whose cell is above `cell`
+        long long a = p + 1, step = 1;  // L[0, a) < cell
+        while (a + step <= nc && __ldg(L + a + step - 1) < cell) {
+          a += step;
+          step <<= 1;
+        }
+        long long b = a + step - 1 < nc ? a + step - 1 : nc;
+        while (a < b) {
+          const long long mid = (a + b) >> 1;
+          if (__ldg(L + mid) < cell) a = mid + 1;
+          else b = mid;
+        }
+        p = a;
+        next_c = p < nc ? __ldg(L + p) : n_cells;
+      }
+      const long long r = cell - p;
+      s_out = __dadd_rn(wmu_ones_run(s_out, r - out_next), v1);
+      out_next = r + 1;
+    }
+  }
+  s_in = wmu_ones_run(s_in, nc - in_next);
+  s_out = wmu_ones_run(s_out, (n_cells - nc) - out_next);
+  out_ratio[(size_t)c * n_genes + g] = __ddiv_rn(__ddiv_rn(s_in, (double)nc), __ddiv_rn(s_out, (double)(n_cells - nc)));
 }
 
 }  // namespace gficf

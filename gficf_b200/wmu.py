@@ -43,6 +43,19 @@ def rcpp_parallel_WMU_test(matX, matY, printOutput: bool = False) -> np.ndarray:
     return out
 
 
+def _cluster_ids(cluster, n_cells):
+    """The markers calls' cluster ids as contiguous int32 and n_clusters = max id + 1."""
+    cl = np.asarray(cluster)
+    if cl.ndim != 1 or cl.shape[0] != n_cells:
+        raise ValueError("cluster must hold one id per column (cell) of mat")
+    if cl.size and not np.issubdtype(cl.dtype, np.integer):
+        raise TypeError("cluster ids must be integers")
+    if cl.size and (cl.min() < 0 or cl.max() >= 2 ** 31 - 1):
+        raise ValueError("cluster ids must be 0-based and below 2^31 - 1")
+    ids = np.ascontiguousarray(cl, dtype=np.int32)
+    return ids, (int(ids.max()) + 1 if ids.size else 0)
+
+
 def rcpp_parallel_WMU_markers(mat, cluster, printOutput: bool = False) -> np.ndarray:
     """Every cluster's one-vs-rest test in one call: a genes x cells matrix and one 0-based cluster id
     per cell -> (n_genes, 2, n_clusters) float64 (Fortran order).  out[:, :, c] equals, bit for bit,
@@ -51,21 +64,51 @@ def rcpp_parallel_WMU_markers(mat, cluster, printOutput: bool = False) -> np.nda
     m = np.asfortranarray(np.asarray(mat), dtype=np.float64)
     if m.ndim != 2:
         raise TypeError("a numeric matrix (2-D) is required")
-    cl = np.asarray(cluster)
-    if cl.ndim != 1 or cl.shape[0] != m.shape[1]:
-        raise ValueError("cluster must hold one id per column (cell) of mat")
-    if cl.size and not np.issubdtype(cl.dtype, np.integer):
-        raise TypeError("cluster ids must be integers")
-    if cl.size and (cl.min() < 0 or cl.max() >= 2 ** 31 - 1):
-        raise ValueError("cluster ids must be 0-based and below 2^31 - 1")
-    ids = np.ascontiguousarray(cl, dtype=np.int32)
-    k = int(ids.max()) + 1 if ids.size else 0
+    ids, k = _cluster_ids(cluster, m.shape[1])
     if printOutput:
         sys.stdout.write(_BANNER)
     g = m.shape[0]
     out = np.empty((g, 2, k), dtype=np.float64, order="F")
     err = C.create_string_buffer(512)
     rc = _lib.lib().gficf_cuda_wmu_markers(m.ctypes.data, g, m.shape[1], ids.ctypes.data, k, out.ctypes.data, err, 512)
+    _lib.check(rc, err)
+    if printOutput:
+        sys.stdout.write(_BANNER_DONE)
+    return out
+
+
+def _int32_index(a, what):
+    a = np.asarray(a)
+    if not np.issubdtype(a.dtype, np.integer):
+        raise TypeError("%s must be an integer array" % what)
+    if a.dtype != np.int32 and a.size and (a.min() < -2 ** 31 or a.max() >= 2 ** 31):
+        raise ValueError("%s does not fit in int32 (the dgCMatrix slots are R integers)" % what)
+    return np.ascontiguousarray(a, dtype=np.int32)
+
+
+def rcpp_parallel_WMU_markers_sparse(mat, cluster, printOutput: bool = False) -> np.ndarray:
+    """rcpp_parallel_WMU_markers for a scipy.sparse CSC matrix or array (genes x cells; R's dgCMatrix has
+    the same slots).  Only the stored values are uploaded and read; the result equals, bit for bit,
+    rcpp_parallel_WMU_markers(mat.toarray(), cluster).  Stored zeros are zeros.  Other sparse formats and
+    dense arrays raise TypeError (convert with .tocsc() first); index arrays that do not fit in int32 raise
+    ValueError."""
+    import scipy.sparse as sp
+
+    if not sp.issparse(mat) or mat.format != "csc":
+        raise TypeError("a scipy.sparse CSC matrix (genes x cells) is required")
+    g, n = mat.shape
+    colptr = _int32_index(mat.indptr, "indptr")
+    row = _int32_index(mat.indices, "indices")
+    x = np.ascontiguousarray(mat.data, dtype=np.float64)
+    if colptr.size != n + 1 or row.size < colptr[-1] or x.size < colptr[-1]:
+        raise ValueError("indptr / indices / data do not describe a %d x %d matrix" % (g, n))
+    ids, k = _cluster_ids(cluster, n)
+    if printOutput:
+        sys.stdout.write(_BANNER)
+    out = np.empty((g, 2, k), dtype=np.float64, order="F")
+    err = C.create_string_buffer(512)
+    rc = _lib.lib().gficf_cuda_wmu_markers_csc(colptr.ctypes.data, row.ctypes.data, x.ctypes.data, g, n,
+                                               ids.ctypes.data, k, out.ctypes.data, err, 512)
     _lib.check(rc, err)
     if printOutput:
         sys.stdout.write(_BANNER_DONE)

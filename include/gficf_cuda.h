@@ -337,6 +337,24 @@ int gficf_cuda_wmu_test(const double* mat_x, const double* mat_y, int64_t n_gene
 int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, const int32_t* cluster,
                            int32_t n_clusters, double* out, char* err, size_t errlen);
 
+/* gficf_cuda_wmu_markers on a sparse matrix: genes x cells in compressed-column form, the slots of R's
+ * dgCMatrix as they are -- colptr = p (n_cells + 1 entries, colptr[0] = 0, never decreasing), row = i
+ * (0-based gene of each stored value, strictly increasing inside a column), x = the stored values;
+ * nnz = colptr[n_cells].  cluster, n_clusters, out and the timings as for gficf_cuda_wmu_markers, and out
+ * equals, bit for bit, what gficf_cuda_wmu_markers returns for the densified matrix.  Stored zeros (and
+ * -0.0) are zeros.  Only the stored values cross PCIe (12 bytes each, plus 4 per cell for colptr); the device
+ * turns them gene-major (stable radix sort by gene), and the rank and means kernels read only them.
+ * Device memory: 41.5 bytes per stored value (12 of input, 29.5 of transpose scratch that also holds the
+ * gene-major copy), 12 per cell and 12 per gene, the n_genes x n_clusters results (16 bytes each), and the
+ * rank kernel's sort scratch of 24 bytes x the largest number of stored values of a gene, per resident CTA.
+ * GFICF_E_ARG: as gficf_cuda_wmu_markers, and a malformed matrix -- colptr[0] != 0 or colptr decreasing
+ * (checked on the host before any upload), a row id outside [0, n_genes) or row ids not strictly increasing
+ * in a column (checked on the device before any kernel indexes with them).  GFICF_E_LIMIT: as
+ * gficf_cuda_wmu_markers, and n_genes >= 2^31 - 1.  One device. */
+int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const double* x, int64_t n_genes,
+                               int64_t n_cells, const int32_t* cluster, int32_t n_clusters, double* out, char* err,
+                               size_t errlen);
+
 /* ---- the data-parallel pieces of the community detection that reads the graph (SURVEY 8f row 3;
  * reference src/ModularityOptimizer.cpp).  The sequential, RNG-ordered local moving loop (:484-583)
  * stays on the host; these are the steps around it that touch every edge:
