@@ -46,6 +46,9 @@
 #ifndef GFICF_SMALL_MINB
 #define GFICF_SMALL_MINB 4       // resident CTAs per SM the k<=32 kernel is compiled for
 #endif
+#ifndef GFICF_MAX_TRIES
+#define GFICF_MAX_TRIES 256      // multipliers the k<=128 kernels try before raising kFlagHashFail (1: tests of that path)
+#endif
 #include <stdint.h>
 
 namespace gficf {
@@ -53,7 +56,7 @@ namespace gficf {
 constexpr int kPadId = -2;              // pad entries of an index row (never equals an id or kEmpty)
 constexpr unsigned kEmpty = 0xFFFFFFFFu;  // empty hash slot
 constexpr unsigned kFlagBadId = 1u, kFlagDupId = 2u, kFlagHashFail = 4u;
-constexpr int kMaxTries = 256;
+constexpr int kMaxTries = GFICF_MAX_TRIES;
 constexpr unsigned kMult0 = 0x9E3779B1u;  // odd; successive multipliers come from an LCG
 
 __device__ __forceinline__ unsigned next_mult(unsigned m) { return (m * 0x2C1B3C6Du + 0x297A2D39u) | 1u; }

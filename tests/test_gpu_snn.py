@@ -93,6 +93,28 @@ def test_host_buffer_entry(cuda, oracle):
     assert e.value.code == 5
 
 
+def test_self_ids_in_the_graph_build(cuda, oracle):
+    """Duplicate cells keep themselves in their neighbour list after neigh[, -1]: rows that list their
+    own cell (a self loop with u = k) next to rows that do not, device and host-buffer entries."""
+    from gficf_b200 import snn
+    from tests.test_jaccard_slabs_emu import self_ids
+
+    n, k = 6_000, 30
+    rng = np.random.default_rng(6)
+    a = np.ascontiguousarray(self_ids(rng, k, n) - 1, dtype=np.int32)
+    for i in np.flatnonzero(rng.random(n) < 0.5):  # half the rows drop their self id again
+        j = int(np.flatnonzero(a[i] == i)[0])
+        a[i, j] = rng.choice(np.setdiff1d(np.arange(n), np.append(a[i], i)))
+    idx0 = torch.from_numpy(a)
+    r = synth.to_r_matrix(idx0)
+    names, cols, rows_ref, data_ref = louvain.lower_triangle_edges(oracle.parallel(r))
+    colptr, rows, w, vcell, flags = _gpu_triangle(n, k, idx0)
+    assert flags & ~16 == 0
+    _same_graph(names.astype(np.int64), cols, rows_ref, data_ref, colptr, rows, w, vcell)
+    g = snn.snn_graph(r)
+    _same_graph(names.astype(np.int64), cols, rows_ref, data_ref, g["colptr"], g["row"], g["weight"], g["vertex_cell"])
+
+
 @pytest.mark.skipif(not os.path.exists(MODOPT_BIN), reason="oracle/_ref/modopt not shipped")
 def test_labels_from_device_graph(cuda, oracle):
     n, k = 50_000, 30

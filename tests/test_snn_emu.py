@@ -42,12 +42,13 @@ def counts_with_mutual_bit(idx):
     return um
 
 
-def emu_lower(L, idx, grid_w=3, grid_t=2):
+def emu_lower(L, idx, grid_w=3, grid_t=2, um=None):
     n, k = idx.shape
     kp = int(gficf_b200.lib().gficf_cuda_row_stride(k))
     padded = np.full((n, kp), -2, np.int32)
     padded[:, :k] = idx
-    um = counts_with_mutual_bit(idx)
+    if um is None:
+        um = counts_with_mutual_bit(idx)
     colptr = np.zeros(n + 1, np.int64)
     row, w, vcell = np.zeros(n * k, np.int32), np.zeros(n * k), np.zeros(n, np.int32)
     nv, nnz = C.c_longlong(0), C.c_longlong(0)
@@ -57,10 +58,10 @@ def emu_lower(L, idx, grid_w=3, grid_t=2):
     return colptr[:nv.value + 1], row[:nnz.value], w[:nnz.value], vcell[:nv.value], flags
 
 
-def check(L, oracle, idx0):
+def check(L, oracle, idx0, um=None):
     idx = idx0.numpy() if hasattr(idx0, "numpy") else idx0
     names, cols, rows_ref, data_ref = louvain.lower_triangle_edges(oracle.parallel(synth.to_r_matrix(idx0)))
-    colptr, rows, w, vcell, flags = emu_lower(L, idx)
+    colptr, rows, w, vcell, flags = emu_lower(L, idx, um=um)
     assert flags & ~16 == 0
     assert np.array_equal(vcell, names.astype(np.int64))  # igraph's vertex numbering
     assert np.array_equal(np.repeat(np.arange(names.size), np.diff(colptr)), cols)
@@ -95,3 +96,34 @@ def test_emulated_hub_columns_take_the_big_sorts(emu, oracle):
         pytest.skip("the construction produced a repeated id")
     _, colptr = check(emu, oracle, torch.from_numpy(idx))
     assert np.diff(colptr).max() > 512
+
+
+@pytest.fixture(scope="module")
+def jaccard_emu(tmp_path_factory):
+    from tests.test_jaccard_slabs_emu import _build
+
+    return _build(str(tmp_path_factory.mktemp("emu") / "libjaccard_emu.so"), [])
+
+
+@pytest.mark.parametrize("n,k", [(300, 7), (400, 30), (200, 64)])
+def test_emulated_graph_with_self_ids_from_the_count_kernel(emu, jaccard_emu, oracle, n, k):
+    """Duplicate cells are common in real data, so a cell can be in its own list after neigh[, -1]: rows
+    that list themselves (a self loop with u = k) mixed with rows that do not.  The
+    mutual-bit counts come from the emulated count kernel (mode 4), as on the device."""
+    from tests.test_jaccard_slabs_emu import run_slab, self_ids
+
+    rng = np.random.default_rng(n + k)
+    r = self_ids(rng, k, n)
+    keep = rng.random(n) < 0.5  # half the rows drop their self id again
+    a = (r - 1).astype(np.int64)
+    for i in np.flatnonzero(keep):
+        j = int(np.flatnonzero(a[i] == i)[0])
+        free = np.setdiff1d(np.arange(n), np.append(a[i], i))
+        a[i, j] = rng.choice(free)
+    idx = a.astype(np.int32)
+    _, um, _, flags = run_slab(jaccard_emu, idx + 1.0, 4, 0, n, grid=3)
+    assert flags == 0
+    assert np.array_equal(um, counts_with_mutual_bit(idx))
+    import torch
+
+    check(emu, oracle, torch.from_numpy(idx), um=um.astype(np.uint8))
