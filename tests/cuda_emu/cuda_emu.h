@@ -12,8 +12,14 @@
 // than the hardware is intended:
 //   * a collective with a partial mask, or one that not all 32 lanes of the warp reach, aborts;
 //   * a __syncthreads() that some live thread of the CTA never reaches aborts (deadlock report);
-//   * atomics are plain read-modify-writes (fibres never run concurrently), so results that
-//     depend on the ORDER of atomics show up as differences against the GPU, not here.
+//   * atomics are plain read-modify-writes (fibres never run concurrently): their order is the
+//     order in which the fibres run, which the schedule below decides.
+// Schedule (emu_set_schedule): in every round the runnable fibres run in ascending threadIdx.x
+// (the default), descending, or a permutation drawn afresh each round from a seeded xorshift; the
+// CTAs of a launch, over x and y, run in the same kind of order.  A missing barrier where a lower
+// thread writes and a higher one reads, an atomic cursor whose order leaks into the output, or a
+// CTA that reads what a lower-numbered CTA of the same launch wrote passes in ascending order only.
+// Dynamic shared memory is filled with 0xA5 at the start of every CTA.
 #pragma once
 #include <ucontext.h>
 
@@ -68,6 +74,32 @@ struct CtaState {
 
 inline CtaState* g_cta = nullptr;
 inline long long g_launches = 0;
+
+// the order in which runnable fibres (and the CTAs of a launch) are visited
+enum Schedule : int { kAscending = 0, kDescending = 1, kRandom = 2 };
+inline int g_schedule = kAscending;
+inline unsigned long long g_rng = 1;  // xorshift64 state, never 0
+
+inline unsigned long long next_random() {
+  g_rng ^= g_rng << 13;
+  g_rng ^= g_rng >> 7;
+  g_rng ^= g_rng << 17;
+  return g_rng;
+}
+
+// order[0..n) := the visiting order of n items under the current schedule
+inline void schedule_order(std::vector<unsigned>& order, unsigned n) {
+  order.resize(n);
+  for (unsigned i = 0; i < n; ++i) order[i] = g_schedule == kDescending ? n - 1 - i : i;
+  if (g_schedule == kRandom)
+    for (unsigned i = n; i > 1; --i) {  // Fisher-Yates
+      const unsigned j = (unsigned)(next_random() % i);
+      const unsigned t = order[i - 1];
+      order[i - 1] = order[j];
+      order[j] = t;
+    }
+}
+
 // the launch's dynamic shared memory (CTAs run one at a time); static so that it lies inside the 32-bit
 // window of emulated shared-memory addresses (smem_base below), like the kernels' static __shared__ arrays
 constexpr size_t kMaxDynamicSmem = 232 * 1024;
@@ -119,6 +151,9 @@ inline void warp_barrier() {
 inline void fibre_entry() {
   CtaState* c = g_cta;
   c->body();
+  // lanes of this warp already wait in a collective that it will never reach (in ascending order the
+  // next lane to arrive reports it; in other orders every other lane may have arrived already)
+  if (c->warps[c->cur->tid >> 5].arrived) die("warp collective reached while lanes of the warp have exited");
   c->cur->st = St::Done;
   --c->live;
   // a thread that exits while others wait at __syncthreads: the hardware lets the rest proceed
@@ -132,6 +167,16 @@ inline void fibre_entry() {
 
 }  // namespace cuda_emu
 
+// mode 0 ascending, 1 descending, 2 random(seed): the schedule of every later launch.  Exported from
+// every harness library for ctypes (`used` emits the inline definition even where nothing calls it).
+extern "C" inline __attribute__((used, visibility("default"))) void emu_set_schedule(int mode,
+                                                                                     unsigned long long seed) {
+  if (mode < cuda_emu::kAscending || mode > cuda_emu::kRandom) cuda_emu::die("unknown schedule");
+  cuda_emu::g_schedule = mode;
+  cuda_emu::g_rng = seed * 0x9E3779B97F4A7C15ull + 0x2545F4914F6CDD1Dull;  // any seed, 0 included
+  if (cuda_emu::g_rng == 0) cuda_emu::g_rng = 1;
+}
+
 inline cuda_emu::Idx3 threadIdx, blockIdx;
 inline cuda_emu::Dim3 blockDim, gridDim;
 
@@ -143,7 +188,6 @@ constexpr size_t kStackBytes = 64 * 1024;
 template <class F>
 void launch(unsigned grid, unsigned block, F&& body, size_t dynamic_smem_bytes = 0, unsigned grid_y = 1) {
   if (dynamic_smem_bytes > kMaxDynamicSmem) die("more dynamic shared memory than an SM has");
-  memset(g_dyn_smem, 0xA5, dynamic_smem_bytes);
   if (block == 0 || block % 32 != 0 || block > 1024) die("block size must be a multiple of 32, at most 1024");
   ++g_launches;
   gridDim = Dim3{grid, grid_y, 1};
@@ -156,9 +200,12 @@ void launch(unsigned grid, unsigned block, F&& body, size_t dynamic_smem_bytes =
   while (stack_pool.size() < block) stack_pool.emplace_back(new char[kStackBytes]);
   cta.warps.resize(block / 32);
   g_cta = &cta;
-  for (unsigned by = 0; by < grid_y; ++by)
-  for (unsigned b = 0; b < grid; ++b) {
-    blockIdx = Idx3{b, by, 0};
+  std::vector<unsigned> ctas, order;
+  if ((unsigned long long)grid * grid_y > 0xFFFFFFFFull) die("more CTAs than the emulation numbers");
+  schedule_order(ctas, grid * grid_y);  // y-major, like the nested loops of the ascending order
+  for (const unsigned c : ctas) {
+    blockIdx = Idx3{c % grid, c / grid, 0};
+    memset(g_dyn_smem, 0xA5, dynamic_smem_bytes);  // every CTA starts from poison, not its predecessor's data
     cta.live = block;
     cta.cta_arrived = 0;
     for (auto& w : cta.warps) w.arrived = 0;
@@ -174,7 +221,8 @@ void launch(unsigned grid, unsigned block, F&& body, size_t dynamic_smem_bytes =
     }
     while (cta.live) {
       bool ran = false;
-      for (unsigned t = 0; t < block; ++t) {
+      schedule_order(order, block);
+      for (const unsigned t : order) {
         Fibre& f = cta.fibres[t];
         if (f.st != St::Runnable) continue;
         ran = true;
