@@ -1087,6 +1087,11 @@ int default_devices() {
 
 }  // namespace
 
+// the launch plans shared with the CPU emulation (they use CU_TRY)
+#include "network_plan.h"
+#include "snn_plan.h"
+#include "wmu_csc_plan.h"
+
 // ============================================================================
 // C ABI
 // ============================================================================
@@ -1229,6 +1234,49 @@ int gficf_cuda_last_launch(int32_t* grid, int32_t* block, int32_t* smem_bytes, i
 }  // extern "C"
 
 namespace {
+// The caller's current device, made current again when a host-level call ends, whichever way it ends.
+struct DeviceRestore {
+  int dev = -1;
+  DeviceRestore() {
+    if (cudaGetDevice(&dev) != cudaSuccess) {
+      cudaGetLastError();
+      dev = -1;
+    }
+  }
+  ~DeviceRestore() {
+    if (dev >= 0) cudaSetDevice(dev);
+  }
+};
+
+float event_ms(cudaEvent_t a, cudaEvent_t b) {
+  float ms = 0;
+  CU_TRY(cudaEventElapsedTime(&ms, a, b));
+  return ms;
+}
+
+// One single-device host-buffer call: a device must be visible; the call holds g_call_mu and runs on device 0
+// with its workspace ready, and the caller's device is current again when it ends.
+struct SingleDeviceCall {
+  std::unique_lock<std::mutex> lk;
+  DeviceRestore restore;
+  DeviceWs& ws = g_ws[0];
+  std::chrono::steady_clock::time_point t0;
+  SingleDeviceCall() {
+    if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
+    lk = std::unique_lock<std::mutex>(g_call_mu);
+    t0 = std::chrono::steady_clock::now();
+    CU_TRY(cudaSetDevice(0));
+    ws.ensure(0);
+    g_active_devices.store(1);
+  }
+  // gficf_cuda_last_timings: the four phase times, the wall time of the call, launches and bytes copied back
+  void timings(double h2d_ms, double k0_ms, double k1_ms, double d2h_ms, double launches, double d2h_bytes) {
+    const double wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    const double tm[8] = {h2d_ms, k0_ms, k1_ms, d2h_ms, wall, 0, launches, d2h_bytes};
+    memcpy(tl_timings, tm, sizeof tm);
+  }
+};
+
 int jaccard_host_call(const void* idx, int elem, int64_t n, int32_t k, double* out, int32_t n_devices,
                       int32_t mode, int64_t* n_written, char* err, size_t errlen) {
   API_BEGIN
@@ -1253,8 +1301,7 @@ int jaccard_host_call(const void* idx, int elem, int64_t n, int32_t k, double* o
   if ((long long)ndev > n) ndev = 1;
 
   std::lock_guard<std::mutex> lk(g_call_mu);
-  int prev_dev = 0;
-  cudaGetDevice(&prev_dev);
+  DeviceRestore restore;
   const auto t0 = std::chrono::steady_clock::now();
   const long long rows_per = (n + ndev - 1) / ndev;
   g_active_devices.store(ndev);
@@ -1303,7 +1350,6 @@ int jaccard_host_call(const void* idx, int elem, int64_t n, int32_t k, double* o
       }
     }
   }
-  cudaSetDevice(prev_dev);
   const auto t1 = std::chrono::steady_clock::now();
   unsigned flags = 0;
   double tm[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -1397,6 +1443,7 @@ int gficf_cuda_jaccard_rank(const double* idx, int64_t n, int32_t k, double* out
     throw Err{GFICF_E_LIMIT, "n*k must stay below 2^31 (the reference's int row index)"};
   if (k > 65535) throw Err{GFICF_E_LIMIT, "k above 65535 is not supported"};
   std::lock_guard<std::mutex> lk(g_call_mu);
+  DeviceRestore restore;
   const auto t0 = std::chrono::steady_clock::now();
   const int nr = g_mp.nranks;
   const long long rows_per = (n + nr - 1) / nr;
@@ -1687,41 +1734,6 @@ int gficf_cuda_jaccard_counts_mutual_dev(const int32_t* d_idx_i32, int64_t n, in
   DEV_END
 }
 
-// scratch layout of gficf_cuda_snn_lower_dev (all pieces 256-byte aligned)
-struct SnnScratch {
-  int *act, *vid, *cnt_b, *cnt, *cursor, *big_cols, *n_big;
-  unsigned* first;
-  long long *off_a, *off_b, *block_sums, *total, *nv;
-  gficf::SnnEntry* entries;
-  size_t bytes;
-};
-static SnnScratch snn_scratch_layout(char* base, int64_t n, int64_t cap) {
-  SnnScratch s;
-  size_t off = 0;
-  auto take = [&](size_t b) {
-    char* p = base + off;
-    off += (b + 255) / 256 * 256;
-    return p;
-  };
-  const size_t nb = (size_t)((n + gficf::kScanBlock - 1) / gficf::kScanBlock + 2);
-  s.act = (int*)take((size_t)n * 4);
-  s.vid = (int*)take((size_t)n * 4);
-  s.first = (unsigned*)take((size_t)n * 4);
-  s.cnt_b = (int*)take((size_t)n * 4);
-  s.cnt = (int*)take((size_t)n * 4);
-  s.cursor = (int*)take((size_t)n * 4);
-  s.big_cols = (int*)take((size_t)(cap / gficf::kSnnWarpRankMax + 2) * 4);
-  s.n_big = (int*)take(4);
-  s.off_a = (long long*)take((size_t)(n + 1) * 8);
-  s.off_b = (long long*)take((size_t)(n + 1) * 8);
-  s.block_sums = (long long*)take(nb * 8);
-  s.total = (long long*)take(8);
-  s.nv = (long long*)take(8);
-  s.entries = (gficf::SnnEntry*)take((size_t)cap * sizeof(gficf::SnnEntry));
-  s.bytes = off;
-  return s;
-}
-
 size_t gficf_cuda_snn_scratch_bytes(int64_t n, int64_t cap) {
   if (n < 0 || cap < 0) return 0;
   return snn_scratch_layout(nullptr, n, cap).bytes;
@@ -1736,51 +1748,17 @@ int gficf_cuda_snn_lower_dev(const int32_t* d_idx_i32, int64_t n, int32_t k, con
     return GFICF_E_ARG;
   if (k > 127 || n >= 0x7fffffffLL || n * (long long)k >= 0xffffffffLL) return GFICF_E_LIMIT;
   if (cap < n * (int64_t)k) return GFICF_E_ARG;
-  cudaStream_t st = (cudaStream_t)stream;
-  const int kp = row_stride(k);
-  const long long nb = (n + kScanBlock - 1) / kScanBlock;
-  const SnnScratch sc = snn_scratch_layout((char*)d_scratch, n, cap);
-  long long* d_nv = d_n_vertices ? (long long*)d_n_vertices : sc.nv;
-  auto scan = [&](const int* cnt, long long* out) {  // exclusive scan, out[n] = total
-    scan_block_sums_kernel<<<(int)nb, kScanBlock, 0, st>>>(cnt, n, sc.block_sums);
-    compact_scan_kernel<<<1, 1024, 0, st>>>(sc.block_sums, nb, sc.total);
-    scan_finish_kernel<<<(int)nb, kScanBlock, 0, st>>>(cnt, n, sc.block_sums, sc.total, out);
-  };
-  const int grid_w = grid_1d(n * 32, 256, 8);  // warp per row / column
-  const int grid_t = grid_1d(n, 256, 8);
-  // cnt_b, cnt, cursor, big_cols, n_big are contiguous in the layout: one memset
-  CU_TRY(cudaMemsetAsync(sc.cnt_b, 0, (size_t)((char*)sc.off_a - (char*)sc.cnt_b), st));
-  CU_TRY(cudaMemsetAsync(sc.first, 0xff, (size_t)n * 4, st));
-  // 1. igraph's vertex numbering (first appearance in c(from, to) of the kept rows)
-  snn_active_kernel<<<grid_w, 256, 0, st>>>(d_um, n, k, sc.act, d_flags);
-  scan(sc.act, sc.off_a);
-  snn_vertex_ids_kernel<<<grid_t, 256, 0, st>>>(n, sc.act, sc.off_a, sc.off_b, sc.vid, 0, nullptr, d_nv);
-  snn_targets_kernel<0><<<grid_w, 256, 0, st>>>(d_idx_i32, d_um, n, k, kp, sc.act, sc.off_a, sc.first, sc.cnt_b,
-                                               sc.off_b, sc.vid);
-  snn_targets_kernel<1><<<grid_w, 256, 0, st>>>(d_idx_i32, d_um, n, k, kp, sc.act, sc.off_a, sc.first, sc.cnt_b,
-                                               sc.off_b, sc.vid);
-  scan(sc.cnt_b, sc.off_b);
-  snn_targets_kernel<2><<<grid_w, 256, 0, st>>>(d_idx_i32, d_um, n, k, kp, sc.act, sc.off_a, sc.first, sc.cnt_b,
-                                               sc.off_b, sc.vid);
-  snn_vertex_ids_kernel<<<grid_t, 256, 0, st>>>(n, sc.act, sc.off_a, sc.off_b, sc.vid, 1,
-                                                (int*)d_vertex_cell, d_nv);
-  // 2. entries per column, column pointers, scatter, rows ascending inside a column
-  snn_edges_kernel<false><<<grid_w, 256, 0, st>>>(d_idx_i32, d_um, n, k, kp, sc.vid, sc.cnt, nullptr, nullptr);
-  scan(sc.cnt, (long long*)d_colptr);
-  snn_edges_kernel<true><<<grid_w, 256, 0, st>>>(d_idx_i32, d_um, n, k, kp, sc.vid, sc.cursor,
-                                                (const long long*)d_colptr, sc.entries);
-  snn_sort_columns_kernel<<<grid_w, 256, 0, st>>>((const long long*)d_colptr, d_nv, sc.entries, d_row, d_w,
-                                                  sc.big_cols, sc.n_big);
   static thread_local bool attr_set[64] = {};
   int dev = 0;
   CU_TRY(cudaGetDevice(&dev));
-  const int big_smem = kSnnSmemSortMax * 12;
   if (!attr_set[dev & 63]) {
-    CU_TRY(cudaFuncSetAttribute(snn_sort_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, big_smem));
+    CU_TRY(cudaFuncSetAttribute(snn_sort_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                kSnnSmemSortMax * 12));
     attr_set[dev & 63] = true;
   }
-  snn_sort_big_kernel<<<sm_count() * 2, 256, big_smem, st>>>((const long long*)d_colptr, sc.entries, d_row, d_w,
-                                                           sc.big_cols, sc.n_big);
+  snn_lower((cudaStream_t)stream, snn_scratch_layout((char*)d_scratch, n, cap), sm_count() * 8, sm_count() * 2,
+            d_idx_i32, n, k, row_stride(k), d_um, (long long*)d_colptr, d_row, d_w, d_vertex_cell,
+            (long long*)d_n_vertices, d_flags);
   CU_TRY(cudaGetLastError());
   return GFICF_OK;
   DEV_END
@@ -1799,15 +1777,8 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   if (k > 127) throw Err{GFICF_E_LIMIT, "the graph build carries the mutual flag in bit 7 of the count byte: k <= 127"};
   if (n >= 0x7fffffffLL - 2 || (long double)n * k >= 2147483647.0L)
     throw Err{GFICF_E_LIMIT, "n*k must stay below 2^31 (the reference's int row index)"};
-  if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
-  std::lock_guard<std::mutex> lk(g_call_mu);
-  int prev_dev = 0;
-  cudaGetDevice(&prev_dev);
-  const auto t0 = std::chrono::steady_clock::now();
-  DeviceWs& ws = g_ws[0];
-  CU_TRY(cudaSetDevice(0));
-  ws.ensure(0);
-  g_active_devices.store(1);
+  SingleDeviceCall call;
+  DeviceWs& ws = call.ws;
   const long long E = (long long)n * k;
   const int kp = row_stride(k);
   ws.in_raw.need((size_t)E * elem_bytes);
@@ -1815,12 +1786,21 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   ws.counts.need((size_t)E);
   ws.scratch.need(gficf_cuda_snn_scratch_bytes(n, E));
   // results on the device: colptr | w | row | vertex map
-  const size_t o_w = ((size_t)(n + 1) * 8 + 255) / 256 * 256, o_row = o_w + (size_t)E * 8,
-               o_vc = o_row + ((size_t)E * 4 + 255) / 256 * 256;
-  ws.out.need(o_vc + (size_t)n * 4);
-  char* d_res = (char*)ws.out.p;
+  int64_t* d_colptr;
+  double* d_w;
+  int *d_row, *d_vc;
+  auto results = [&](char* base) {
+    ScratchCarver c{base};
+    d_colptr = c.take<int64_t>(n + 1);
+    d_w = c.take<double>(E);
+    d_row = c.take<int>(E);
+    d_vc = c.take<int>(n);
+    return c.bytes;
+  };
+  ws.out.need(results(nullptr));
+  results((char*)ws.out.p);
   unsigned* d_flags = (unsigned*)ws.small.p;
-  long long* d_nv = (long long*)((char*)ws.small.p + 16);
+  int64_t* d_nv = (int64_t*)((char*)ws.small.p + 16);
   CU_TRY(cudaMemsetAsync(ws.small.p, 0, 64, ws.s_comp));
   CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
   const size_t dev_elem = h2d_block(ws, idx_colmajor, n, ws.in_raw.p, n, k, (size_t)elem_bytes, ws.s_comp);
@@ -1832,18 +1812,16 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
   if (!launch_fast<2>((const int*)ws.idx.p, k, 0, n, nullptr, nullptr, nullptr, ws.counts.p, d_flags, ws.s_comp))
     throw Err{GFICF_E_LIMIT, "k outside the range of the mutual-bit count kernel"};
-  const int rc = gficf_cuda_snn_lower_dev((const int32_t*)ws.idx.p, n, k, (const uint8_t*)ws.counts.p,
-                                          (int64_t*)d_res, (int32_t*)(d_res + o_row), (double*)(d_res + o_w), E,
-                                          (int32_t*)(d_res + o_vc), (int64_t*)d_nv, ws.scratch.p, d_flags, ws.s_comp);
+  const int rc = gficf_cuda_snn_lower_dev((const int32_t*)ws.idx.p, n, k, (const uint8_t*)ws.counts.p, d_colptr, d_row,
+                                          d_w, E, d_vc, d_nv, ws.scratch.p, d_flags, ws.s_comp);
   if (rc != GFICF_OK) throw Err{rc, "graph kernels could not be launched"};
   CU_TRY(cudaEventRecord(ws.ev[3], ws.s_comp));
   // flags, vertex count and entry count decide what is copied back
   CU_TRY(cudaMemcpyAsync(ws.h_small, ws.small.p, 32, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaMemcpyAsync((char*)ws.h_small + 32, d_res + (size_t)n * 8, 8, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaMemcpyAsync((char*)ws.h_small + 32, d_colptr + n, 8, cudaMemcpyDeviceToHost, ws.s_comp));
   CU_TRY(cudaStreamSynchronize(ws.s_comp));
   const unsigned flags = ws.h_small[0];
   const long long nv = *(long long*)((char*)ws.h_small + 16), total = *(long long*)((char*)ws.h_small + 32);
-  cudaSetDevice(prev_dev);
   if (flags & kFlagBadId)
     throw Err{GFICF_E_RANGE,
               "neighbour ids must be integers in [1, nrow] (NaN, fractional or out-of-range id found)"};
@@ -1852,94 +1830,20 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   if (nnz) *nnz = total;
   if (n_vertices) *n_vertices = nv;
   if (total > cap) throw Err{GFICF_E_ARG, fmt("row / w capacity %lld is below the %lld entries of the graph", (long long)cap, total)};
-  CU_TRY(cudaSetDevice(0));
   std::vector<Seg> segs;
-  segs.push_back({(char*)colptr, d_res, (size_t)(n + 1) * 8, nullptr});
+  segs.push_back({(char*)colptr, (char*)d_colptr, (size_t)(n + 1) * 8, nullptr});
   if (total) {
-    segs.push_back({(char*)row, d_res + o_row, (size_t)total * 4, nullptr});
-    segs.push_back({(char*)w, d_res + o_w, (size_t)total * 8, nullptr});
+    segs.push_back({(char*)row, (char*)d_row, (size_t)total * 4, nullptr});
+    segs.push_back({(char*)w, (char*)d_w, (size_t)total * 8, nullptr});
   }
-  if (vertex_cell && nv) segs.push_back({(char*)vertex_cell, d_res + o_vc, (size_t)nv * 4, nullptr});
+  if (vertex_cell && nv) segs.push_back({(char*)vertex_cell, (char*)d_vc, (size_t)nv * 4, nullptr});
   CU_TRY(cudaEventRecord(ws.ev[4], ws.s_copy));
   d2h_segs(ws, segs, ws.s_copy);
   CU_TRY(cudaEventRecord(ws.ev[5], ws.s_copy));
   CU_TRY(cudaStreamSynchronize(ws.s_copy));
-  float ms[4] = {0, 0, 0, 0};
-  CU_TRY(cudaEventElapsedTime(&ms[0], ws.ev[0], ws.ev[1]));
-  CU_TRY(cudaEventElapsedTime(&ms[1], ws.ev[1], ws.ev[2]));
-  CU_TRY(cudaEventElapsedTime(&ms[2], ws.ev[2], ws.ev[3]));
-  CU_TRY(cudaEventElapsedTime(&ms[3], ws.ev[4], ws.ev[5]));
-  cudaSetDevice(prev_dev);
-  double tm[8] = {ms[0], ms[1], ms[2], ms[3],
-                  std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(), 0, 22,
-                  (double)(n + 1) * 8 + (double)total * 12 + (vertex_cell ? (double)nv * 4 : 0.0)};
-  memcpy(tl_timings, tm, sizeof tm);
-  return GFICF_OK;
-  API_END
-}
-
-// ---------------------------------------------------------------- Mann-Whitney U per gene (next row 4)
-int gficf_cuda_wmu_test(const double* mat_x, const double* mat_y, int64_t n_genes, int64_t n1, int64_t n2,
-                        double* out, char* err, size_t errlen) {
-  API_BEGIN
-  if (err && errlen) err[0] = 0;
-  if (n_genes < 0 || n1 < 0 || n2 < 0) throw Err{GFICF_E_ARG, "negative matrix dimension"};
-  if (n_genes == 0) return GFICF_OK;
-  if (!mat_x || !mat_y || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
-  if (n1 < 1 || n2 < 1) throw Err{GFICF_E_ARG, "both groups need at least one cell"};
-  if (n1 + n2 >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 cells per gene"};
-  if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
-  std::lock_guard<std::mutex> lk(g_call_mu);
-  int prev_dev = 0;
-  cudaGetDevice(&prev_dev);
-  const auto t0 = std::chrono::steady_clock::now();
-  DeviceWs& ws = g_ws[0];
-  CU_TRY(cudaSetDevice(0));
-  ws.ensure(0);
-  g_active_devices.store(1);
-  const long long N = n1 + n2;
-  int per_sm = 0;
-  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_rank_kernel, kWmuThreads, 0));
-  const int grid = (int)std::min<long long>(n_genes, (long long)std::max(1, per_sm) * sm_count());
-  // device buffers: X | Y in in_raw; per-CTA sort scratch in scratch (keys) and counts (payload);
-  // z, ratio, single flags in out
-  const size_t bx = (size_t)n_genes * n1 * 8, by = (size_t)n_genes * n2 * 8;
-  ws.in_raw.need(bx + by);
-  ws.scratch.need((size_t)grid * 2 * N * sizeof(unsigned long long));
-  ws.counts.need((size_t)grid * (3 * N + 2) * sizeof(unsigned));
-  ws.out.need((size_t)n_genes * (8 + 8 + 4) + 64);
-  double* d_x = (double*)ws.in_raw.p;
-  double* d_y = (double*)((char*)ws.in_raw.p + bx);
-  double* d_z = (double*)ws.out.p;
-  double* d_ratio = d_z + n_genes;
-  int* d_single = (int*)(d_ratio + n_genes);
-  CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
-  h2d_block(ws, mat_x, n_genes * n1, d_x, n_genes * n1, 1, 8, ws.s_comp, /*ids=*/false);
-  h2d_block(ws, mat_y, n_genes * n2, d_y, n_genes * n2, 1, 8, ws.s_comp, /*ids=*/false);
-  CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
-  wmu_rank_kernel<<<grid, kWmuThreads, 0, ws.s_comp>>>(d_x, d_y, n_genes, n1, n2, (unsigned long long*)ws.scratch.p,
-                                                       (unsigned*)ws.counts.p, d_z, d_single);
-  wmu_means_kernel<<<(int)((n_genes + kMeanGenes - 1) / kMeanGenes), kMeanThreads, 0, ws.s_comp>>>(d_x, d_y, n_genes, n1, n2,
-                                                                                                   d_ratio);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
-  std::vector<double> h((size_t)n_genes * 2);
-  std::vector<int> hs((size_t)n_genes);
-  CU_TRY(cudaMemcpyAsync(h.data(), d_z, (size_t)n_genes * 16, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaStreamSynchronize(ws.s_comp));
-  // the two transcendental steps, one per gene: getPvalue (mann_whitney.cpp:101-110) and log2 (:100)
-  for (int64_t g = 0; g < n_genes; ++g) {
-    out[g] = hs[(size_t)g] ? 1.0 : gficf_host::wmu_pvalue(h[(size_t)g]);
-    out[n_genes + g] = log2(h[(size_t)(n_genes + g)]);
-  }
-  float ms0 = 0, ms1 = 0;
-  CU_TRY(cudaEventElapsedTime(&ms0, ws.ev[0], ws.ev[1]));
-  CU_TRY(cudaEventElapsedTime(&ms1, ws.ev[1], ws.ev[2]));
-  cudaSetDevice(prev_dev);
-  double tm[8] = {ms0, 0, ms1, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
-                  0, 2, (double)n_genes * 20};
-  memcpy(tl_timings, tm, sizeof tm);
+  call.timings(event_ms(ws.ev[0], ws.ev[1]), event_ms(ws.ev[1], ws.ev[2]), event_ms(ws.ev[2], ws.ev[3]),
+               event_ms(ws.ev[4], ws.ev[5]), 22,
+               (double)(n + 1) * 8 + (double)total * 12 + (vertex_cell ? (double)nv * 4 : 0.0));
   return GFICF_OK;
   API_END
 }
@@ -1970,38 +1874,63 @@ std::vector<long long> markers_cluster_sizes(const int32_t* cluster, int64_t n_c
   return size;
 }
 
-// Host finish of both markers entries: the two transcendental steps per (gene, cluster), as in
-// gficf_cuda_wmu_test.  h = z | ratio, each n_clusters blocks of n_genes; block c of out is cluster c's
-// n_genes x 2 result.  Clusters are spread over host threads when there are many values.
-void markers_finish(const std::vector<double>& h, const std::vector<int>& hs, int64_t n_genes, int32_t n_clusters,
-                    double* out) {
-  const long long C = n_clusters;
-  const size_t zc = (size_t)n_genes * C;
-  auto finish = [&](long long c_lo, long long c_hi) {
-    for (long long c = c_lo; c < c_hi; ++c) {
-      const double* z = h.data() + (size_t)c * n_genes;
-      const double* ratio = h.data() + zc + (size_t)c * n_genes;
-      double* o = out + (size_t)c * 2 * n_genes;
-      for (int64_t g = 0; g < n_genes; ++g) {
-        o[g] = hs[(size_t)g] ? 1.0 : gficf_host::wmu_pvalue(z[g]);
-        o[n_genes + g] = log2(ratio[g]);
-      }
-    }
-  };
-  const long long nthreads =
-      std::min<long long>({C, (long long)std::max(1u, std::thread::hardware_concurrency()), 16LL,
-                           std::max(1LL, (long long)zc / 16384)});
-  if (nthreads <= 1) {
-    finish(0, C);
-  } else {
-    std::vector<std::thread> th;
-    for (long long t = 0; t < nthreads; ++t) th.emplace_back(finish, C * t / nthreads, C * (t + 1) / nthreads);
-    for (auto& x : th) x.join();
-  }
+// The end shared by the Mann-Whitney entries: launches checked, ev[2] recorded, z | ratio (n_clusters blocks of
+// n_genes) and the per-gene single flags read back and finished into out (wmu_finish).
+void wmu_read_and_finish(DeviceWs& ws, const double* d_z, const int* d_single, int64_t n_genes, int32_t n_clusters,
+                         double* out) {
+  CU_TRY(cudaGetLastError());
+  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
+  const size_t zc = (size_t)n_genes * n_clusters;
+  std::vector<double> h(zc * 2);
+  std::vector<int> hs((size_t)n_genes);
+  CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
+  CU_TRY(cudaStreamSynchronize(ws.s_comp));
+  wmu_finish(h.data(), hs.data(), n_genes, n_clusters, out);
 }
 }  // namespace
 
 extern "C" {
+
+// ---------------------------------------------------------------- Mann-Whitney U per gene (next row 4)
+int gficf_cuda_wmu_test(const double* mat_x, const double* mat_y, int64_t n_genes, int64_t n1, int64_t n2,
+                        double* out, char* err, size_t errlen) {
+  API_BEGIN
+  if (err && errlen) err[0] = 0;
+  if (n_genes < 0 || n1 < 0 || n2 < 0) throw Err{GFICF_E_ARG, "negative matrix dimension"};
+  if (n_genes == 0) return GFICF_OK;
+  if (!mat_x || !mat_y || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  if (n1 < 1 || n2 < 1) throw Err{GFICF_E_ARG, "both groups need at least one cell"};
+  if (n1 + n2 >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 cells per gene"};
+  SingleDeviceCall call;
+  DeviceWs& ws = call.ws;
+  const long long N = n1 + n2;
+  int per_sm = 0;
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_rank_kernel, kWmuThreads, 0));
+  const int grid = (int)std::min<long long>(n_genes, (long long)std::max(1, per_sm) * sm_count());
+  // device buffers: X | Y in in_raw; per-CTA sort scratch in scratch (keys) and counts (payload);
+  // z, ratio, single flags in out
+  const size_t bx = (size_t)n_genes * n1 * 8, by = (size_t)n_genes * n2 * 8;
+  ws.in_raw.need(bx + by);
+  ws.scratch.need((size_t)grid * 2 * N * sizeof(unsigned long long));
+  ws.counts.need((size_t)grid * (3 * N + 2) * sizeof(unsigned));
+  ws.out.need((size_t)n_genes * (8 + 8 + 4) + 64);
+  double* d_x = (double*)ws.in_raw.p;
+  double* d_y = (double*)((char*)ws.in_raw.p + bx);
+  double* d_z = (double*)ws.out.p;
+  double* d_ratio = d_z + n_genes;
+  int* d_single = (int*)(d_ratio + n_genes);
+  CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
+  h2d_block(ws, mat_x, n_genes * n1, d_x, n_genes * n1, 1, 8, ws.s_comp, /*ids=*/false);
+  h2d_block(ws, mat_y, n_genes * n2, d_y, n_genes * n2, 1, 8, ws.s_comp, /*ids=*/false);
+  CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
+  wmu_test_launch(ws.s_comp, grid, d_x, d_y, n_genes, n1, n2, (unsigned long long*)ws.scratch.p, (unsigned*)ws.counts.p,
+                  d_z, d_ratio, d_single);
+  wmu_read_and_finish(ws, d_z, d_single, n_genes, 1, out);
+  call.timings(event_ms(ws.ev[0], ws.ev[1]), 0, event_ms(ws.ev[1], ws.ev[2]), 0, 2, (double)n_genes * 20);
+  return GFICF_OK;
+  API_END
+}
 
 // One-vs-rest Mann-Whitney U for every cluster in one call: one upload, one sort per gene
 int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, const int32_t* cluster,
@@ -2012,34 +1941,34 @@ int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, 
   if (n_genes == 0) return GFICF_OK;
   if (!mat || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
   const std::vector<long long> size = markers_cluster_sizes(cluster, n_cells, n_clusters);
-  if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
-  std::lock_guard<std::mutex> lk(g_call_mu);
-  int prev_dev = 0;
-  cudaGetDevice(&prev_dev);
-  const auto t0 = std::chrono::steady_clock::now();
-  DeviceWs& ws = g_ws[0];
-  CU_TRY(cudaSetDevice(0));
-  ws.ensure(0);
-  g_active_devices.store(1);
+  SingleDeviceCall call;
+  DeviceWs& ws = call.ws;
   const long long N = n_cells, C = n_clusters;
-  const size_t acc_smem = (size_t)C * kWmuClusterSmemBytes;
   CU_TRY(cudaFuncSetAttribute(wmu_markers_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                               kWmuMaxClusters * kWmuClusterSmemBytes));
   int per_sm = 0;
-  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_rank_kernel, kWmuThreads, acc_smem));
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_rank_kernel, kWmuThreads,
+                                                       (size_t)C * kWmuClusterSmemBytes));
   const int grid = (int)std::min<long long>(n_genes, (long long)std::max(1, per_sm) * sm_count());
   // device buffers: the matrix in in_raw; cluster ids | cluster sizes in idx; per-CTA sort scratch in
   // scratch (keys) and counts (payload); z | ratio per (gene, cluster) and the per-gene single flags in out
-  const size_t bm = (size_t)n_genes * N * 8, bid = ((size_t)N * 4 + 255) / 256 * 256;
+  const size_t bm = (size_t)n_genes * N * 8;
+  int* d_cl;
+  long long* d_size;
+  auto ids = [&](char* base) {
+    ScratchCarver c{base};
+    d_cl = c.take<int>(N);
+    d_size = c.take<long long>(C);
+    return c.bytes;
+  };
   ws.in_raw.need(bm);
-  ws.idx.need(bid + (size_t)C * 8);
+  ws.idx.need(ids(nullptr));
+  ids((char*)ws.idx.p);
   ws.scratch.need((size_t)grid * 2 * N * sizeof(unsigned long long));
   ws.counts.need((size_t)grid * (3 * N + 2) * sizeof(unsigned));
   const size_t zc = (size_t)n_genes * C;
   ws.out.need(zc * 16 + (size_t)n_genes * 4 + 64);
   double* d_mat = (double*)ws.in_raw.p;
-  int* d_cl = (int*)ws.idx.p;
-  long long* d_size = (long long*)((char*)ws.idx.p + bid);
   double* d_z = (double*)ws.out.p;
   double* d_ratio = d_z + zc;
   int* d_single = (int*)(d_ratio + zc);
@@ -2048,26 +1977,10 @@ int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, 
   h2d_block(ws, cluster, N, d_cl, N, 1, 4, ws.s_comp, /*ids=*/false);
   h2d_block(ws, size.data(), C, d_size, C, 1, 8, ws.s_comp, /*ids=*/false);
   CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
-  wmu_markers_rank_kernel<<<grid, kWmuThreads, acc_smem, ws.s_comp>>>(
-      d_mat, n_genes, N, d_cl, d_size, n_clusters, (unsigned long long*)ws.scratch.p, (unsigned*)ws.counts.p, d_z,
-      d_single);
-  const dim3 mgrid((unsigned)((n_genes + kMeanGenes - 1) / kMeanGenes), (unsigned)((C + kMarkClusters - 1) / kMarkClusters));
-  wmu_markers_means_kernel<<<mgrid, kMarkThreads, 0, ws.s_comp>>>(d_mat, n_genes, N, d_cl, d_size, n_clusters, d_ratio);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
-  std::vector<double> h(zc * 2);
-  std::vector<int> hs((size_t)n_genes);
-  CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaStreamSynchronize(ws.s_comp));
-  markers_finish(h, hs, n_genes, n_clusters, out);
-  float ms0 = 0, ms1 = 0;
-  CU_TRY(cudaEventElapsedTime(&ms0, ws.ev[0], ws.ev[1]));
-  CU_TRY(cudaEventElapsedTime(&ms1, ws.ev[1], ws.ev[2]));
-  cudaSetDevice(prev_dev);
-  double tm[8] = {ms0, 0, ms1, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
-                  0, 2, (double)zc * 16 + (double)n_genes * 4};
-  memcpy(tl_timings, tm, sizeof tm);
+  wmu_markers_launch(ws.s_comp, grid, d_mat, n_genes, N, d_cl, d_size, n_clusters, (unsigned long long*)ws.scratch.p,
+                     (unsigned*)ws.counts.p, d_z, d_ratio, d_single);
+  wmu_read_and_finish(ws, d_z, d_single, n_genes, n_clusters, out);
+  call.timings(event_ms(ws.ev[0], ws.ev[1]), 0, event_ms(ws.ev[1], ws.ev[2]), 0, 2, (double)zc * 16 + (double)n_genes * 4);
   return GFICF_OK;
   API_END
 }
@@ -2075,7 +1988,6 @@ int gficf_cuda_wmu_markers(const double* mat, int64_t n_genes, int64_t n_cells, 
 }  // extern "C"
 
 // ---------------------------------------------------------------- network pieces of the community detection (next row 3)
-#include "network_plan.h"
 
 extern "C" {
 
@@ -2124,7 +2036,6 @@ int gficf_cuda_network_reduce_dev(const int64_t* d_first, const int32_t* d_neigh
 }  // extern "C"
 
 // ---------------------------------------------------------------- Mann-Whitney markers from a sparse matrix
-#include "wmu_csc_plan.h"
 
 extern "C" {
 
@@ -2146,37 +2057,40 @@ int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const 
   const long long nnz = colptr[n_cells];
   if (nnz > 0 && (!row || !x)) throw Err{GFICF_E_ARG, "null matrix pointer"};
   const std::vector<long long> size = markers_cluster_sizes(cluster, n_cells, n_clusters);
-  if (visible_devices() < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
-  std::lock_guard<std::mutex> lk(g_call_mu);
-  int prev_dev = 0;
-  cudaGetDevice(&prev_dev);
-  const auto t0 = std::chrono::steady_clock::now();
-  DeviceWs& ws = g_ws[0];
-  CU_TRY(cudaSetDevice(0));
-  ws.ensure(0);
-  g_active_devices.store(1);
+  SingleDeviceCall call;
+  DeviceWs& ws = call.ws;
   const long long N = n_cells, C = n_clusters;
   const WmuClusterLists cl = wmu_cluster_lists(cluster, N, n_clusters);
   // device buffers: colptr | row | x in in_raw; cluster ids | crank | members | cluster sizes | cptr in idx;
   // the transpose's scratch in scratch (the gene-major values end up there); per-CTA sort scratch of the
   // rank kernel in counts; z | ratio per (gene, cluster) and the per-gene single flags in out
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  const size_t b_cp = al((size_t)(N + 1) * 4), b_row = al((size_t)nnz * 4), b_x = (size_t)nnz * 8;
-  ws.in_raw.need(b_cp + b_row + b_x + 8);
-  const size_t b_cell = al((size_t)N * 4), b_size = al((size_t)C * 8);
-  ws.idx.need(3 * b_cell + b_size + (size_t)(C + 1) * 8);
+  int *d_colptr, *d_row, *d_cl, *d_crank, *d_members;
+  double* d_x;
+  long long *d_size, *d_cptr;
+  auto matrix = [&](char* base) {
+    ScratchCarver c{base};
+    d_colptr = c.take<int>(N + 1);
+    d_row = c.take<int>(nnz);
+    d_x = c.take<double>(nnz + 1);
+    return c.bytes;
+  };
+  auto lists = [&](char* base) {
+    ScratchCarver c{base};
+    d_cl = c.take<int>(N);
+    d_crank = c.take<int>(N);
+    d_members = c.take<int>(N);
+    d_size = c.take<long long>(C);
+    d_cptr = c.take<long long>(C + 1);
+    return c.bytes;
+  };
+  ws.in_raw.need(matrix(nullptr));
+  matrix((char*)ws.in_raw.p);
+  ws.idx.need(lists(nullptr));
+  lists((char*)ws.idx.p);
   ws.scratch.need(wmu_csc_layout(nullptr, n_genes, nnz).bytes);
   const WmuCscScratch sc = wmu_csc_layout((char*)ws.scratch.p, n_genes, nnz);
   const size_t zc = (size_t)n_genes * C;
   ws.out.need(zc * 16 + (size_t)n_genes * 4 + 64);
-  int* d_colptr = (int*)ws.in_raw.p;
-  int* d_row = (int*)((char*)ws.in_raw.p + b_cp);
-  double* d_x = (double*)((char*)ws.in_raw.p + b_cp + b_row);
-  int* d_cl = (int*)ws.idx.p;
-  int* d_crank = (int*)((char*)ws.idx.p + b_cell);
-  int* d_members = (int*)((char*)ws.idx.p + 2 * b_cell);
-  long long* d_size = (long long*)((char*)ws.idx.p + 3 * b_cell);
-  long long* d_cptr = (long long*)((char*)ws.idx.p + 3 * b_cell + b_size);
   double* d_z = (double*)ws.out.p;
   double* d_ratio = d_z + zc;
   int* d_single = (int*)(d_ratio + zc);
@@ -2200,38 +2114,22 @@ int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const 
   CU_TRY(cudaStreamSynchronize(ws.s_comp));
   if (flags & kFlagCscRow)
     throw Err{GFICF_E_ARG, "a row id is outside [0, n_genes) or row ids are not strictly increasing in a column"};
-  long long cap = 1;
-  for (int64_t g = 0; g < n_genes; ++g) cap = std::max(cap, gptr[(size_t)g + 1] - gptr[(size_t)g]);
-  const size_t acc_smem = (size_t)C * kWmuClusterSmemBytes;
+  const long long cap = wmu_gene_cap(gptr.data(), n_genes);
   CU_TRY(cudaFuncSetAttribute(wmu_markers_csr_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                               kWmuMaxClusters * kWmuClusterSmemBytes));
   int per_sm = 0;
-  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_csr_rank_kernel, kWmuThreads, acc_smem));
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_csr_rank_kernel, kWmuThreads,
+                                                       (size_t)C * kWmuClusterSmemBytes));
   const int grid = (int)std::min<long long>(n_genes, (long long)std::max(1, per_sm) * sm_count());
   ws.counts.need((size_t)grid * 2 * cap * (sizeof(unsigned long long) + sizeof(unsigned)));
   unsigned long long* d_keys = (unsigned long long*)ws.counts.p;
   unsigned* d_pay = (unsigned*)(d_keys + (size_t)grid * 2 * cap);
-  wmu_markers_csr_rank_kernel<<<grid, kWmuThreads, acc_smem, ws.s_comp>>>(
-      gm.ent_x, gm.ent_cell, sc.gene_ptr, n_genes, N, d_cl, d_size, n_clusters, cap, d_keys, d_pay, d_z, d_single);
-  const int mthreads = wmu_csr_means_threads(n_clusters);
-  const dim3 mgrid((unsigned)n_genes, (unsigned)((C + mthreads - 1) / mthreads));
-  wmu_markers_csr_means_kernel<<<mgrid, mthreads, 0, ws.s_comp>>>(gm.ent_x, gm.ent_cell, sc.gene_ptr, n_genes, N, d_cl,
-                                                                  d_crank, d_members, d_cptr, n_clusters, d_ratio);
-  CU_TRY(cudaGetLastError());
-  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
-  std::vector<double> h(zc * 2);
-  std::vector<int> hs((size_t)n_genes);
-  CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)n_genes * 4, cudaMemcpyDeviceToHost, ws.s_comp));
-  CU_TRY(cudaStreamSynchronize(ws.s_comp));
-  markers_finish(h, hs, n_genes, n_clusters, out);
-  float ms0 = 0, ms1 = 0;
-  CU_TRY(cudaEventElapsedTime(&ms0, ws.ev[0], ws.ev[1]));
-  CU_TRY(cudaEventElapsedTime(&ms1, ws.ev[1], ws.ev[2]));
-  cudaSetDevice(prev_dev);
-  double tm[8] = {ms0, 0, ms1, 0, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(),
-                  0, (double)(7 + 5 * ((bits_for(n_genes - 1) + 7) / 8)), (double)zc * 16 + (double)n_genes * 4 + 4 + (double)gptr.size() * 8};
-  memcpy(tl_timings, tm, sizeof tm);
+  wmu_markers_csc_launch(ws.s_comp, grid, gm, sc.gene_ptr, n_genes, N, d_cl, d_crank, d_members, d_size, d_cptr,
+                         n_clusters, cap, d_keys, d_pay, d_z, d_ratio, d_single);
+  wmu_read_and_finish(ws, d_z, d_single, n_genes, n_clusters, out);
+  call.timings(event_ms(ws.ev[0], ws.ev[1]), 0, event_ms(ws.ev[1], ws.ev[2]), 0,
+               (double)(7 + 5 * ((bits_for(n_genes - 1) + 7) / 8)),
+               (double)zc * 16 + (double)n_genes * 4 + 4 + (double)gptr.size() * 8);
   return GFICF_OK;
   API_END
 }

@@ -3,45 +3,9 @@
 // tests/cuda_emu/network_emu.cpp with GFICF_CUDA_EMU defined, so the SAME sequence of launches is
 // what the CPU test suite runs against the oracle and what runs on the B200.
 #pragma once
-#include <stddef.h>
-#include <string.h>
-
 #include "gficf_cuda.h"
 #include "network_kernels.cuh"
-
-#ifdef GFICF_CUDA_EMU
-typedef int net_stream_t;
-#define GFICF_LAUNCH(st, kernel, grid, block, ...) \
-  cuda_emu::launch((unsigned)(grid), (unsigned)(block), [=] { kernel(__VA_ARGS__); })
-inline void net_zero(net_stream_t, void* p, size_t bytes) { memset(p, 0, bytes); }
-inline void net_copy(net_stream_t, void* dst, const void* src, size_t bytes) { memcpy(dst, src, bytes); }
-inline void net_read(net_stream_t, void* host, const void* dev, size_t bytes) { memcpy(host, dev, bytes); }
-inline void net_check_launches() {}
-#else
-typedef cudaStream_t net_stream_t;
-#define GFICF_LAUNCH(st, kernel, grid, block, ...) kernel<<<(unsigned)(grid), (unsigned)(block), 0, (st)>>>(__VA_ARGS__)
-inline void net_zero(net_stream_t st, void* p, size_t bytes) { CU_TRY(cudaMemsetAsync(p, 0, bytes, st)); }
-inline void net_copy(net_stream_t st, void* dst, const void* src, size_t bytes) {
-  CU_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st));
-}
-// the few scalars the host needs to size the next launches (entry counts): one small synchronous read
-inline void net_read(net_stream_t st, void* host, const void* dev, size_t bytes) {
-  CU_TRY(cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, st));
-  CU_TRY(cudaStreamSynchronize(st));
-}
-inline void net_check_launches() { CU_TRY(cudaGetLastError()); }
-#endif
-
-// Test builds only (tests/cuda_emu, AddressSanitizer): every scratch piece is followed by a red zone and
-// only the pieces themselves are addressable, so a kernel that runs past its piece is reported.
-#ifdef GFICF_NET_ASAN
-#include <sanitizer/asan_interface.h>
-#define GFICF_NET_REDZONE 256
-#define GFICF_NET_PIECE(p, b) do { if (base) __asan_unpoison_memory_region((p), (b)); } while (0)
-#else
-#define GFICF_NET_REDZONE 0
-#define GFICF_NET_PIECE(p, b) do { } while (0)
-#endif
+#include "plan_common.h"
 
 namespace gficf {
 
@@ -84,39 +48,33 @@ struct NetScratch {
 
 inline NetScratch net_scratch_layout(char* base, long long nn, long long cap) {
   NetScratch s;
-  size_t off = 0;
-  auto take = [&](size_t b) {
-    char* p = base + off;
-    off += (b + GFICF_NET_REDZONE + 255) / 256 * 256;
-    GFICF_NET_PIECE(p, b);
-    return p;
-  };
+  ScratchCarver c{base};
   if (cap < nn) cap = nn;
   const long long n_tiles = (cap + kRadixTile - 1) / kRadixTile + 1;
   const long long scan_len = (256 * n_tiles > cap ? 256 * n_tiles : cap) + 1;
-  for (int b = 0; b < 2; ++b) s.keys[b] = (unsigned long long*)take((size_t)cap * 8);
-  for (int b = 0; b < 2; ++b) s.vals[b] = (unsigned*)take((size_t)cap * 4);
-  s.aux = (unsigned*)take((size_t)cap * 4);
-  s.perm = (unsigned*)take((size_t)nn * 4);
-  s.head = (int*)take((size_t)cap * 4);
-  s.seg_start = (unsigned*)take((size_t)cap * 4);
-  s.seg_id = (long long*)take((size_t)(cap + 1) * 8);
-  s.seg_key = (unsigned long long*)take((size_t)cap * 8);
-  s.seg_w = (double*)take((size_t)cap * 8);
-  s.hist = (int*)take((size_t)(256 * n_tiles) * 4);
-  s.offsets = (long long*)take((size_t)(256 * n_tiles + 1) * 8);
-  s.block_sums = (long long*)take((size_t)(scan_len / kScanBlock + 2) * 8);
-  s.total = (long long*)take(8);
-  s.cnt = (int*)take((size_t)(nn + 1) * 4);
-  s.ptr_a = (long long*)take((size_t)(nn + 1) * 8);
-  s.ptr_b = (long long*)take((size_t)(nn + 1) * 8);
-  s.dbl_b = (double*)take((size_t)(nn + 1) * 8);
-  s.seq_state = (SeqState*)take(sizeof(SeqState));
-  s.seq_fn = (SeqFn*)take((size_t)kSeqMaxBlocks * sizeof(SeqFn));
-  s.sums = (double*)take(64);
-  s.ptr_c = (long long*)take((size_t)(nn + 1) * 8);
-  s.cnt_b = (int*)take((size_t)(nn + 1) * 4);
-  s.bytes = off;
+  for (int b = 0; b < 2; ++b) s.keys[b] = c.take<unsigned long long>(cap);
+  for (int b = 0; b < 2; ++b) s.vals[b] = c.take<unsigned>(cap);
+  s.aux = c.take<unsigned>(cap);
+  s.perm = c.take<unsigned>(nn);
+  s.head = c.take<int>(cap);
+  s.seg_start = c.take<unsigned>(cap);
+  s.seg_id = c.take<long long>(cap + 1);
+  s.seg_key = c.take<unsigned long long>(cap);
+  s.seg_w = c.take<double>(cap);
+  s.hist = c.take<int>(256 * n_tiles);
+  s.offsets = c.take<long long>(256 * n_tiles + 1);
+  s.block_sums = c.take<long long>(scan_len / kScanBlock + 2);
+  s.total = c.take<long long>(1);
+  s.cnt = c.take<int>(nn + 1);
+  s.ptr_a = c.take<long long>(nn + 1);
+  s.ptr_b = c.take<long long>(nn + 1);
+  s.dbl_b = c.take<double>(nn + 1);
+  s.seq_state = c.take<SeqState>(1);
+  s.seq_fn = c.take<SeqFn>(kSeqMaxBlocks);
+  s.sums = c.take<double>(8);
+  s.ptr_c = c.take<long long>(nn + 1);
+  s.cnt_b = c.take<int>(nn + 1);
+  s.bytes = c.bytes;
   return s;
 }
 

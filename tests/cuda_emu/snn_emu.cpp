@@ -1,72 +1,25 @@
-// snn_emu.cpp -- the graph-build kernels (gficf_b200/csrc/snn_kernels.cuh) compiled as plain C++ against
-// the CUDA emulation.  TEST INFRASTRUCTURE.  The launch sequence below restates the one of
-// gficf_cuda_snn_lower_dev (gficf_b200/csrc/gficf_cuda.cu), with small grids so that the grid-stride
-// loops are exercised; built and loaded by tests/test_snn_emu.py:
-//   g++ -O1 -std=c++17 -ffp-contract=off -DGFICF_CUDA_EMU -Itests/cuda_emu -Igficf_b200/csrc -shared -fPIC
+// snn_emu.cpp -- the graph build of gficf_cuda_snn_lower_dev through its own launch sequence
+// (gficf_b200/csrc/snn_plan.h) on the CUDA emulation.  TEST INFRASTRUCTURE; built and loaded by
+// tests/test_snn_emu.py:
+//   g++ -O1 -std=c++17 -ffp-contract=off -DGFICF_CUDA_EMU -Itests/cuda_emu -Igficf_b200/csrc -Iinclude -shared -fPIC
 #include <vector>
 
-#include "snn_kernels.cuh"
+#include "snn_plan.h"
 
 using namespace gficf;
 
-#define LAUNCH(kernel, grid, block, ...) cuda_emu::launch((unsigned)(grid), (unsigned)(block), [=] { kernel(__VA_ARGS__); })
-
-namespace {
-void scan(const int* cnt, long long n, long long* out, long long* block_sums, long long* total) {
-  const long long nb = (n + kScanBlock - 1) / kScanBlock;
-  LAUNCH(scan_block_sums_kernel, nb, kScanBlock, cnt, n, block_sums);
-  LAUNCH(compact_scan_kernel, 1, 1024, block_sums, nb, total);
-  LAUNCH(scan_finish_kernel, nb, kScanBlock, cnt, n, (const long long*)block_sums, (const long long*)total, out);
-}
-}  // namespace
-
 // idx: n x kp int32 (0-based, padded rows), um: n*k bytes (count | mutual << 7).  Outputs sized by the
 // caller: colptr[n+1], row / w [n*k], vertex_cell[n].  Returns the flags; *n_vertices, *nnz are set.
+// max_ctas caps the grid-stride launches, sort_ctas is the grid of the shared-memory column sort.
 extern "C" unsigned emu_snn_lower(const int* idx, long long n, int k, int kp, const unsigned char* um,
                                   long long* colptr, int* row, double* w, int* vertex_cell,
-                                  long long* n_vertices, long long* nnz, int grid_w, int grid_t) {
-  const long long cap = n * k;
-  const long long nb = (n + kScanBlock - 1) / kScanBlock;
-  std::vector<int> act(n, -7), vid(n, -7), cnt_b(n, 0), cnt(n, 0), cursor(n, 0), big_cols(cap / kSnnWarpRankMax + 2, -7);
-  std::vector<unsigned> first(n, 0xFFFFFFFFu);
-  std::vector<long long> off_a(n + 1, -7), off_b(n + 1, -7), block_sums(nb + 2, -7);
-  std::vector<SnnEntry> entries(cap);
-  long long total = 0, nv = 0;
-  int n_big = 0;
+                                  long long* n_vertices, long long* nnz, int max_ctas, int sort_ctas) {
+  // scratch is never assumed initialised: every 32-bit word starts as 1, non-zero (a missing zero fill shows)
+  // and below every edge number (so does a missing 0xFF fill of the first-appearance minima)
+  std::vector<unsigned> scratch(snn_scratch_layout(nullptr, n, n * k).bytes / 4, 1u);
   unsigned flags = 0;
-  int *d_act = act.data(), *d_vid = vid.data(), *d_cnt_b = cnt_b.data(), *d_cnt = cnt.data(), *d_cursor = cursor.data(),
-      *d_big = big_cols.data(), *d_nbig = &n_big;
-  unsigned *d_first = first.data(), *d_flags = &flags;
-  long long *d_off_a = off_a.data(), *d_off_b = off_b.data(), *d_bs = block_sums.data(), *d_total = &total, *d_nv = &nv;
-  SnnEntry* d_entries = entries.data();
-
-  LAUNCH(snn_active_kernel, grid_w, 256, um, n, k, d_act, d_flags);
-  scan(d_act, n, d_off_a, d_bs, d_total);
-  LAUNCH(snn_vertex_ids_kernel, grid_t, 256, n, (const int*)d_act, (const long long*)d_off_a, (const long long*)d_off_b,
-         d_vid, 0, (int*)nullptr, d_nv);
-  LAUNCH(snn_targets_kernel<0>, grid_w, 256, idx, um, n, k, kp, (const int*)d_act, (const long long*)d_off_a, d_first,
-         d_cnt_b, (const long long*)d_off_b, d_vid);
-  LAUNCH(snn_targets_kernel<1>, grid_w, 256, idx, um, n, k, kp, (const int*)d_act, (const long long*)d_off_a, d_first,
-         d_cnt_b, (const long long*)d_off_b, d_vid);
-  scan(d_cnt_b, n, d_off_b, d_bs, d_total);
-  LAUNCH(snn_targets_kernel<2>, grid_w, 256, idx, um, n, k, kp, (const int*)d_act, (const long long*)d_off_a, d_first,
-         d_cnt_b, (const long long*)d_off_b, d_vid);
-  LAUNCH(snn_vertex_ids_kernel, grid_t, 256, n, (const int*)d_act, (const long long*)d_off_a, (const long long*)d_off_b,
-         d_vid, 1, vertex_cell, d_nv);
-  LAUNCH(snn_edges_kernel<false>, grid_w, 256, idx, um, n, k, kp, (const int*)d_vid, d_cnt, (const long long*)nullptr,
-         (SnnEntry*)nullptr);
-  scan(d_cnt, n, colptr, d_bs, d_total);
-  LAUNCH(snn_edges_kernel<true>, grid_w, 256, idx, um, n, k, kp, (const int*)d_vid, d_cursor, (const long long*)colptr,
-         d_entries);
-  LAUNCH(snn_sort_columns_kernel, grid_w, 256, (const long long*)colptr, (const long long*)d_nv,
-         (const SnnEntry*)d_entries, row, w, d_big, d_nbig);
-  cuda_emu::launch(2, 256,
-                   [=] {
-                     snn_sort_big_kernel((const long long*)colptr, (const SnnEntry*)d_entries, row, w, (const int*)d_big,
-                                         (const int*)d_nbig);
-                   },
-                   (size_t)kSnnSmemSortMax * 12);
-  *n_vertices = nv;
-  *nnz = colptr[nv];
+  snn_lower(0, snn_scratch_layout((char*)scratch.data(), n, n * k), max_ctas, sort_ctas, idx, n, k, kp, um, colptr,
+            row, w, vertex_cell, n_vertices, &flags);
+  *nnz = colptr[*n_vertices];
   return flags;
 }

@@ -1,14 +1,10 @@
-// wmu_emu.cpp -- the Mann-Whitney kernels (gficf_b200/csrc/wmu_kernels.cuh) compiled as plain C++
-// against the CUDA emulation, followed by the host half of gficf_cuda_wmu_test (host_stats.cpp: normal
-// cdf, log2).  TEST INFRASTRUCTURE; built and loaded by tests/test_wmu_emu.py:
-//   g++ -O1 -std=c++17 -ffp-contract=off -DGFICF_CUDA_EMU -Itests/cuda_emu -Igficf_b200/csrc -shared -fPIC
+// wmu_emu.cpp -- gficf_cuda_wmu_test's launches and host finish (gficf_b200/csrc/wmu_csc_plan.h) on the CUDA
+// emulation.  TEST INFRASTRUCTURE; built and loaded by tests/test_wmu_emu.py:
+//   g++ -O1 -std=c++17 -ffp-contract=off -DGFICF_CUDA_EMU -Itests/cuda_emu -Igficf_b200/csrc -Iinclude -shared -fPIC
 //   tests/cuda_emu/wmu_emu.cpp gficf_b200/csrc/host_stats.cpp
-#include <math.h>
-
 #include <vector>
 
-#include "host_stats.h"
-#include "wmu_kernels.cuh"
+#include "wmu_csc_plan.h"
 
 using namespace gficf;
 
@@ -18,18 +14,9 @@ extern "C" void emu_wmu_test(const double* mat_x, const double* mat_y, long long
   if (grid > n_genes) grid = (int)n_genes;
   std::vector<unsigned long long> keys((size_t)grid * 2 * N, 0xA5A5A5A5A5A5A5A5ull);
   std::vector<unsigned> pay((size_t)grid * (3 * N + 2), 0xA5A5A5A5u);
-  std::vector<double> z(n_genes), ratio(n_genes);
+  std::vector<double> z_ratio((size_t)n_genes * 2);
   std::vector<int> single(n_genes);
-  unsigned long long* d_keys = keys.data();
-  unsigned* d_pay = pay.data();
-  double *d_z = z.data(), *d_ratio = ratio.data();
-  int* d_single = single.data();
-  cuda_emu::launch((unsigned)grid, kWmuThreads,
-                   [=] { wmu_rank_kernel(mat_x, mat_y, n_genes, n1, n2, d_keys, d_pay, d_z, d_single); });
-  cuda_emu::launch((unsigned)((n_genes + kMeanGenes - 1) / kMeanGenes), kMeanThreads,
-                   [=] { wmu_means_kernel(mat_x, mat_y, n_genes, n1, n2, d_ratio); });
-  for (long long g = 0; g < n_genes; ++g) {  // as in gficf_cuda_wmu_test
-    out[g] = single[g] ? 1.0 : gficf_host::wmu_pvalue(z[g]);
-    out[n_genes + g] = log2(ratio[g]);
-  }
+  wmu_test_launch(0, grid, mat_x, mat_y, n_genes, n1, n2, keys.data(), pay.data(), z_ratio.data(),
+                  z_ratio.data() + n_genes, single.data());
+  wmu_finish(z_ratio.data(), single.data(), n_genes, 1, out);
 }

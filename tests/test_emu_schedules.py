@@ -556,8 +556,8 @@ def test_a_removed_barrier_fails_only_under_permuted_schedules(libs, tmp_path):
     assert n == 1, "the barrier is gone from wmu_kernels.cuh: pick another"
     (csrc / "wmu_kernels.cuh").write_text(mutant)
     so = str(tmp_path / "libwmu_emu_mutant.so")
-    cmd = ["g++", "-O1", "-std=c++17", "-ffp-contract=off", "-DGFICF_CUDA_EMU", "-I" + EMU, "-I" + str(csrc), "-shared",
-           "-fPIC", "-Wall", "-Wno-unknown-pragmas", "-Werror", os.path.join(EMU, "wmu_emu.cpp"),
+    cmd = ["g++", "-O1", "-std=c++17", "-ffp-contract=off", "-DGFICF_CUDA_EMU", "-I" + EMU, "-I" + str(csrc),
+           "-I" + os.path.join(ROOT, "include"), "-shared", "-fPIC", "-Wall", "-Wno-unknown-pragmas", "-Werror", os.path.join(EMU, "wmu_emu.cpp"),
            str(csrc / "host_stats.cpp"), "-o", so]
     out = subprocess.run(cmd, capture_output=True, text=True)
     assert out.returncode == 0, out.stderr

@@ -54,6 +54,40 @@ def test_set_devices_default(cuda, oracle):
     assert np.array_equal(got, oracle.parallel(r))
 
 
+def test_single_device_calls_leave_the_callers_device_current(cuda):
+    """The host-buffer graph-build and Mann-Whitney calls run on device 0; the caller's current device is
+    current again when they return, also when they fail (a malformed row id is found on the device)."""
+    if _ndev(cuda) < 2:
+        pytest.skip("needs >= 2 GPUs")
+    import scipy.sparse as sp
+    import torch
+
+    from gficf_b200 import snn
+    from tests.test_wmu_markers_sparse_emu import malformed_cases
+
+    torch.cuda.set_device(1)
+    try:
+        _, colptr, row = malformed_cases()[1]
+        bad = sp.csc_matrix((5, 4))
+        bad.indptr, bad.indices, bad.data = colptr, row, np.arange(1.0, row.size + 1.0)
+        with pytest.raises(cuda.GficfCudaError) as e:
+            cuda.rcpp_parallel_WMU_markers_sparse(bad, np.array([0, 1, 0, 1], dtype=np.int32))
+        assert e.value.code == 1 and "row id" in e.value.message
+        assert torch.cuda.current_device() == 1
+        rng = np.random.default_rng(5)
+        m = np.asfortranarray(np.floor(rng.gamma(1.0, 2.0, size=(20, 300))))
+        cl = (np.arange(300) % 4).astype(np.int32)
+        calls = (lambda: cuda.rcpp_parallel_WMU_test(m[:, :100], m[:, 100:]),
+                 lambda: cuda.rcpp_parallel_WMU_markers(m, cl),
+                 lambda: cuda.rcpp_parallel_WMU_markers_sparse(sp.csc_matrix(m), cl),
+                 lambda: snn.snn_graph(synth.to_r_matrix(synth.knn_index(3_000, 10, scramble=True))))
+        for i, call in enumerate(calls):
+            call()
+            assert torch.cuda.current_device() == 1, i
+    finally:
+        torch.cuda.set_device(0)
+
+
 _WORKER = r"""
 import os, sys, numpy as np, torch, torch.distributed as dist
 sys.path.insert(0, %(root)r)

@@ -21,7 +21,7 @@ _ll, _ip, _dp, _bp = C.POINTER(C.c_longlong), C.POINTER(C.c_int), C.POINTER(C.c_
 def emu(tmp_path_factory):
     so = str(tmp_path_factory.mktemp("emu") / "libsnn_emu.so")
     cmd = ["g++", "-O1", "-std=c++17", "-ffp-contract=off", "-DGFICF_CUDA_EMU", "-I" + os.path.join(ROOT, "tests", "cuda_emu"),
-           "-I" + os.path.join(ROOT, "gficf_b200", "csrc"), "-shared", "-fPIC", "-Wall", "-Wno-unknown-pragmas", "-Werror",
+           "-I" + os.path.join(ROOT, "gficf_b200", "csrc"), "-I" + os.path.join(ROOT, "include"), "-shared", "-fPIC", "-Wall", "-Wno-unknown-pragmas", "-Werror",
            os.path.join(ROOT, "tests", "cuda_emu", "snn_emu.cpp"), "-o", so]
     out = subprocess.run(cmd, capture_output=True, text=True)
     assert out.returncode == 0, out.stderr
@@ -42,7 +42,7 @@ def counts_with_mutual_bit(idx):
     return um
 
 
-def emu_lower(L, idx, grid_w=3, grid_t=2, um=None):
+def emu_lower(L, idx, max_ctas=2, sort_ctas=2, um=None):
     n, k = idx.shape
     kp = int(gficf_b200.lib().gficf_cuda_row_stride(k))
     padded = np.full((n, kp), -2, np.int32)
@@ -54,7 +54,7 @@ def emu_lower(L, idx, grid_w=3, grid_t=2, um=None):
     nv, nnz = C.c_longlong(0), C.c_longlong(0)
     p = lambda a, t: a.ctypes.data_as(t)  # noqa: E731
     flags = L.emu_snn_lower(p(padded, _ip), n, k, kp, p(um, _bp), p(colptr, _ll), p(row, _ip), p(w, _dp), p(vcell, _ip),
-                            C.byref(nv), C.byref(nnz), grid_w, grid_t)
+                            C.byref(nv), C.byref(nnz), max_ctas, sort_ctas)
     return colptr[:nv.value + 1], row[:nnz.value], w[:nnz.value], vcell[:nv.value], flags
 
 

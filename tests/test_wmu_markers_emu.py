@@ -22,7 +22,7 @@ _ip = C.POINTER(C.c_int32)
 def emu(tmp_path_factory):
     so = str(tmp_path_factory.mktemp("emu") / "libwmu_markers_emu.so")
     cmd = ["g++", "-O1", "-std=c++17", "-ffp-contract=off", "-DGFICF_CUDA_EMU", "-I" + os.path.join(ROOT, "tests", "cuda_emu"),
-           "-I" + os.path.join(ROOT, "gficf_b200", "csrc"), "-shared", "-fPIC", "-Wall", "-Wno-unknown-pragmas", "-Werror",
+           "-I" + os.path.join(ROOT, "gficf_b200", "csrc"), "-I" + os.path.join(ROOT, "include"), "-shared", "-fPIC", "-Wall", "-Wno-unknown-pragmas", "-Werror",
            os.path.join(ROOT, "tests", "cuda_emu", "wmu_markers_emu.cpp"),
            os.path.join(ROOT, "gficf_b200", "csrc", "host_stats.cpp"), "-o", so]
     out = subprocess.run(cmd, capture_output=True, text=True)
