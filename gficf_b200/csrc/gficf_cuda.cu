@@ -74,11 +74,29 @@ std::string fmt(const char* f, ...) {
     }                                                                                    \
   } while (0)
 
+// cudaFuncAttributeMaxDynamicSharedMemorySize of a kernel, set once per device and host thread
+void set_max_dynamic_smem(const void* kernel, size_t bytes) {
+  static thread_local std::vector<std::pair<const void*, int>> done;
+  int dev = 0;
+  CU_TRY(cudaGetDevice(&dev));
+  const std::pair<const void*, int> key(kernel, dev);
+  if (std::find(done.begin(), done.end(), key) != done.end()) return;
+  CU_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  done.push_back(key);
+}
+
+}  // namespace
+
+// the launch plans shared with the CPU emulation (they use CU_TRY, Err and set_max_dynamic_smem)
+#include "jaccard_plan.h"
+#include "network_plan.h"
+#include "snn_plan.h"
+#include "wmu_csc_plan.h"
+
+namespace {
+
 // ------------------------------------------------------------------ launch bookkeeping
-struct LaunchInfo {
-  int grid = 0, block = 0, smem = 0, variant = 0;
-};
-thread_local LaunchInfo tl_launch;
+thread_local LaunchInfo tl_launch;  // the last count kernel of this thread (gficf_cuda_last_launch)
 thread_local double tl_timings[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 struct OutputInfo {
   int mode = 1;           // OutMode of the last host-buffer call
@@ -105,147 +123,9 @@ int sm_count() {
   return sms;
 }
 
-// k > 32: rows are padded to a multiple of GFICF_WIDE_ROW_INTS ints.  16 (64 bytes): a row never
-// straddles an extra 64-byte DRAM burst; 8 (32 bytes, whole sectors): k = 100 fetches 416 instead of
-// 448 bytes per gathered row (A/B in profiles/r02_wide_k.md).
-#ifndef GFICF_WIDE_ROW_INTS
-#define GFICF_WIDE_ROW_INTS 16
-#endif
-int32_t row_stride(int32_t k) {
-  if (k <= 4) return 4;
-  if (k <= 8) return 8;
-  if (k <= 16) return 16;
-  if (k <= 32) return 32;
-  return (k + GFICF_WIDE_ROW_INTS - 1) / GFICF_WIDE_ROW_INTS * GFICF_WIDE_ROW_INTS;
-}
-
-// Table slots per warp-group.  A multiplier is collision free with probability ~exp(-k^2/2/slots)
-// (0.37 at slots = k^2/2, 0.14 at k=128 in 4096 slots); a failed try costs warp 0 ~150 cycles of a
-// ~20k-cycle row, so the smaller table (more resident warp-groups) wins.
-#ifndef GFICF_WIDE_MAX_LOG_TS
-#define GFICF_WIDE_MAX_LOG_TS 12
-#endif
-int wide_log_ts(int k) {
-  const int want = k <= 45 ? 10 : (k <= 64 ? 11 : (k <= 90 ? 12 : 13));
-  return want < GFICF_WIDE_MAX_LOG_TS ? want : GFICF_WIDE_MAX_LOG_TS;
-}
-
-size_t wide_smem_bytes(int log_ts) { return (size_t)wide_smem_words(log_ts) * 4 + 129 * sizeof(double); }
-
-// persistent grid: resident CTAs per SM x SM count, capped by the work.  tl_cta_cap (> 0) lowers the
-// CTAs per SM so that two persistent kernels on different streams can be resident side by side
-// (gficf_cuda_set_launch_ctas_per_sm).
+// tl_cta_cap (> 0) lowers the resident CTAs per SM of the persistent kernels so that two of them on
+// different streams can be resident side by side (gficf_cuda_set_launch_ctas_per_sm)
 thread_local int tl_cta_cap = 0;
-template <typename K>
-int persistent_grid(K kernel, int block, size_t smem, long long work_ctas) {
-  int per_sm = 0;
-  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, block, smem));
-  if (per_sm < 1) per_sm = 1;
-  if (tl_cta_cap > 0 && per_sm > tl_cta_cap) per_sm = tl_cta_cap;
-  long long g = (long long)per_sm * sm_count();
-  if (g > work_ctas) g = work_ctas;
-  if (g < 1) g = 1;
-  return (int)g;
-}
-
-template <int KP, int CO, bool SKIP>
-void launch_small_t(const int* idx, int k, long long lo, long long hi, double* f, double* t, double* w,
-                    uint8_t* u, unsigned* flags, cudaStream_t st, unsigned tag) {
-  auto kern = jaccard_small_k_kernel<KP, CO, SKIP>;
-  const int block = kSmallWarps * 32;
-  const int grid = persistent_grid(kern, block, 0, (hi - lo + kSmallWarps - 1) / kSmallWarps);
-  const int lg_group = CO == 3 ? 3 : 0;  // CO == 3: groups of 8 rows (8k bytes: whole 8- or 16-byte vectors)
-  const long long work = CO == 3 ? (((hi - lo) >> lg_group) + 1 + kSmallWarps - 1) / kSmallWarps
-                                 : (hi - lo + kSmallWarps - 1) / kSmallWarps;
-  const int grid3 = CO == 3 ? persistent_grid(kern, block, 0, work) : grid;
-  kern<<<grid3, block, 0, st>>>(idx, k, lo, hi, f, t, w, u, flags, tag, lg_group);
-  tl_launch = {grid3, block, (int)(sizeof(unsigned) * kSmallWarps * SmallK<KP>::TS + 33 * 8), KP};
-}
-
-// the pad-skipping variant costs registers, so it is used only when a whole 16-byte piece of every
-// row is padding (k <= KP-4, e.g. k=25..28 in 32-int rows); k=30 keeps the lean variant
-template <int KP, int CO>
-void launch_small(const int* idx, int k, long long lo, long long hi, double* f, double* t, double* w,
-                  uint8_t* u, unsigned* flags, cudaStream_t st, unsigned tag) {
-  if (KP > 4 && k <= KP - 4) launch_small_t<KP, CO, true>(idx, k, lo, hi, f, t, w, u, flags, st, tag);
-  else launch_small_t<KP, CO, false>(idx, k, lo, hi, f, t, w, u, flags, st, tag);
-}
-
-template <int LOG_TS, int CO>
-void launch_wide(const int* idx, int k, int kp, long long lo, long long hi, double* f, double* t,
-                 double* w, uint8_t* u, unsigned* flags, cudaStream_t st, unsigned tag) {
-  auto kern = jaccard_wide_k_kernel<LOG_TS, CO>;
-  const size_t smem = wide_smem_bytes(LOG_TS);
-  static thread_local bool attr_set[64] = {};
-  int dev = 0;
-  CU_TRY(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63]) {
-    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set[dev & 63] = true;
-  }
-  const int block = kWideWarps * 32;
-  const int grid = persistent_grid(kern, block, smem, hi - lo);
-  kern<<<grid, block, smem, st>>>(idx, k, kp, lo, hi, f, t, w, u, flags, tag);
-  tl_launch = {grid, block, (int)smem, 1000 + LOG_TS};
-}
-
-template <bool CO>
-void launch_large(const int* idx, int k, int kp, long long lo, long long hi, double* f, double* t,
-                  double* w, void* u, unsigned* flags, cudaStream_t st) {
-  const size_t smem = large_smem_bytes();
-  const int block = kLargeWarps * 32;
-  int dev = 0;
-  CU_TRY(cudaGetDevice(&dev));
-  static thread_local bool attr_set[64][2] = {};
-  auto k8 = jaccard_large_k_kernel<uint8_t, CO>;
-  auto k16 = jaccard_large_k_kernel<uint16_t, CO>;
-  if (!attr_set[dev & 63][CO]) {
-    CU_TRY(cudaFuncSetAttribute(k8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CU_TRY(cudaFuncSetAttribute(k16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set[dev & 63][CO] = true;
-  }
-  if (k <= 255) {
-    const int grid = persistent_grid(k8, block, smem, hi - lo);
-    k8<<<grid, block, smem, st>>>(idx, k, kp, lo, hi, f, t, w, (uint8_t*)u, flags);
-    tl_launch = {grid, block, (int)smem, 2000};
-  } else {
-    const int grid = persistent_grid(k16, block, smem, hi - lo);
-    k16<<<grid, block, smem, st>>>(idx, k, kp, lo, hi, f, t, w, (uint16_t*)u, flags);
-    tl_launch = {grid, block, (int)smem, 2001};
-  }
-}
-
-// fast kernels; returns false when k is outside their range.  CO: 0 = (from,to,w) doubles,
-// 1 = counts, 2 = counts with the mutual-neighbour bit (k <= 127)
-template <int CO>
-bool launch_fast(const int* idx, int k, long long lo, long long hi, double* f, double* t, double* w,
-                 void* u_any, unsigned* flags, cudaStream_t st, unsigned tag = 0) {
-  uint8_t* u = (uint8_t*)u_any;  // one byte per edge for k <= 255, two above
-  if (CO == 2 && k > 127) return false;  // bit 7 of the count byte carries the mutual flag
-  if (tag && ((CO != 1 && CO != 3) || k > 127)) return false;  // ... or the epoch bit of the streaming gather
-  if (CO == 3 && k > 32) return false;                           // grouped vector stores: the k <= 32 kernel only
-  if (hi <= lo) return true;
-  const int kp = row_stride(k);
-  if (k <= 4) launch_small<4, CO>(idx, k, lo, hi, f, t, w, u, flags, st, tag);
-  else if (k <= 8) launch_small<8, CO>(idx, k, lo, hi, f, t, w, u, flags, st, tag);
-  else if (k <= 16) launch_small<16, CO>(idx, k, lo, hi, f, t, w, u, flags, st, tag);
-  else if (k <= 32) launch_small<32, CO>(idx, k, lo, hi, f, t, w, u, flags, st, tag);
-  else if (k <= 128) {
-    switch (wide_log_ts(k)) {
-      case 10: launch_wide<10, CO>(idx, k, kp, lo, hi, f, t, w, u, flags, st, tag); break;
-      case 11: launch_wide<11, CO>(idx, k, kp, lo, hi, f, t, w, u, flags, st, tag); break;
-      case 12: launch_wide<12, CO>(idx, k, kp, lo, hi, f, t, w, u, flags, st, tag); break;
-      default: launch_wide<13, CO>(idx, k, kp, lo, hi, f, t, w, u, flags, st, tag); break;
-    }
-  } else if (k <= kLargeMaxK) {
-    if (CO == 2) return false;
-    launch_large<(CO != 0)>(idx, k, kp, lo, hi, f, t, w, u_any, flags, st);
-  } else {
-    return false;
-  }
-  CU_TRY(cudaGetLastError());
-  return true;
-}
 
 // bounded spins of the peer-memory kernels: GFICF_CUDA_PEER_TIMEOUT_MS (default 20 s) in SM clocks.
 // The clock rate is queried once per device: cudaDevAttrClockRate is one of the attributes the
@@ -273,78 +153,8 @@ long long peer_spin_clocks(long long timeout_ms) {
   return timeout_ms * (long long)khz;
 }
 
-int grid_1d(long long total, int block, int cap_per_sm = 8) {
-  long long g = (total + block - 1) / block;
-  long long cap = (long long)sm_count() * cap_per_sm;
-  if (g > cap) g = cap;
-  if (g < 1) g = 1;
-  return (int)g;
-}
-
-template <typename T>
-void launch_layout(const T* src, long long ld_rows, long long ld_row0, long long n, int k,
-                   long long lo, long long hi, int* dst, unsigned* flags, cudaStream_t st) {
-  if (hi <= lo) return;
-  const int kp = row_stride(k);
-  int tile_r = kLayoutTileR;
-  while (tile_r > 1 && (size_t)tile_r * (kp + 1) * sizeof(int) > 48 * 1024) tile_r /= 2;
-  const size_t smem = (size_t)tile_r * (kp + 1) * sizeof(int);
-  if (smem > 48 * 1024) throw Err{GFICF_E_LIMIT, "k too large for the layout pre-pass (k <= 12000)"};
-  const long long ntiles = (hi - lo + tile_r - 1) / tile_r;
-  long long g = std::min<long long>(ntiles, (long long)sm_count() * 8);
-  layout_colmajor_kernel<T><<<(int)g, kLayoutThreads, smem, st>>>(src, ld_rows, ld_row0, n, k, kp, lo, hi,
-                                                                  dst, flags, tile_r);
-  CU_TRY(cudaGetLastError());
-}
-
-void launch_exact(const int* idx, int k, long long lo, long long hi, int set_sem, void* d_u,
-                  cudaStream_t st) {
-  if (hi <= lo) return;
-  const int kp = row_stride(k);
-  const long long total = (hi - lo) * (long long)k;
-  const int grid = grid_1d(total, 128, 16);
-  if (k <= 255)
-    jaccard_exact_kernel<uint8_t><<<grid, 128, 0, st>>>(idx, k, kp, lo, hi, set_sem, (uint8_t*)d_u);
-  else
-    jaccard_exact_kernel<uint16_t><<<grid, 128, 0, st>>>(idx, k, kp, lo, hi, set_sem, (uint16_t*)d_u);
-  CU_TRY(cudaGetLastError());
-}
-
-size_t expand_scratch_bytes(long long slab_e) {
-  const long long nchunks = (slab_e + kCompactChunk - 1) / kCompactChunk;
-  return (size_t)(nchunks + 1) * sizeof(long long);
-}
-
-template <typename CT>
-void launch_expand_t(const int* idx, int k, long long lo, long long hi, const CT* d_u, int mode,
-                     double* f, double* t, double* w, void* scratch, long long* d_nw,
-                     cudaStream_t st) {
-  const int kp = row_stride(k);
-  const long long total = (hi - lo) * (long long)k;
-  if (total <= 0) return;
-  if (mode == GFICF_MODE_PARALLEL) {
-    expand_fixed_kernel<CT><<<grid_1d(total, kExpandThreads, 8), kExpandThreads, 0, st>>>(
-        idx, k, kp, lo, hi, d_u, f, t, w);
-  } else {
-    long long* chunk = (long long*)scratch;
-    const long long nchunks = (total + kCompactChunk - 1) / kCompactChunk;
-    if (nchunks > 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "slab too large for compaction"};
-    compact_count_kernel<CT><<<(int)nchunks, kCompactThreads, 0, st>>>(d_u, total, chunk);
-    compact_scan_kernel<<<1, 1024, 0, st>>>(chunk, nchunks, d_nw);
-    compact_scatter_kernel<CT><<<(int)nchunks, kCompactThreads, 0, st>>>(idx, k, kp, lo, d_u, total,
-                                                                        chunk, f, t, w);
-    zero_tail_kernel<<<grid_1d(total, 256, 8), 256, 0, st>>>(d_nw, total, f, t, w);
-  }
-  CU_TRY(cudaGetLastError());
-}
-
-void launch_expand(const int* idx, int k, long long lo, long long hi, const void* d_u, int mode,
-                   double* f, double* t, double* w, void* scratch, long long* d_nw, cudaStream_t st) {
-  if (k <= 255)
-    launch_expand_t<uint8_t>(idx, k, lo, hi, (const uint8_t*)d_u, mode, f, t, w, scratch, d_nw, st);
-  else
-    launch_expand_t<uint16_t>(idx, k, lo, hi, (const uint16_t*)d_u, mode, f, t, w, scratch, d_nw, st);
-}
+// the Jaccard plan on the current device and stream
+JacCtx jac_ctx(cudaStream_t st) { return JacCtx{st, sm_count(), tl_cta_cap, &tl_launch}; }
 
 // ------------------------------------------------------------------ per-device workspace
 struct Buf {
@@ -883,11 +693,11 @@ void device_phase0(Slab s, SlabResult* res) {
     res->h2d_bytes = (double)s.rows * k * dev_elem;
     CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
     if (dev_elem == 8)
-      launch_layout((const double*)ws.in_raw.p, s.rows, s.lo, s.n, k, s.lo, s.hi, (int*)ws.idx.p, d_flags,
-                    ws.s_comp);
+      launch_layout(jac_ctx(ws.s_comp), (const double*)ws.in_raw.p, s.rows, s.lo, s.n, k, s.lo, s.hi,
+                    (int*)ws.idx.p, d_flags);
     else
-      launch_layout((const int*)ws.in_raw.p, s.rows, s.lo, s.n, k, s.lo, s.hi, (int*)ws.idx.p, d_flags,
-                    ws.s_comp);
+      launch_layout(jac_ctx(ws.s_comp), (const int*)ws.in_raw.p, s.rows, s.lo, s.n, k, s.lo, s.hi, (int*)ws.idx.p,
+                    d_flags);
     res->launches += s.rows > 0;
     CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
   } catch (const Err& e) {
@@ -928,7 +738,7 @@ void device_phase1(Slab s, SlabResult* res) {
         if (clo >= chi) break;
         const long long eo = (clo - s.lo) * k;
         CU_TRY(cudaEventRecord(ws.ev_k0[c], ws.s_comp));
-        launch_fast<1>(d_idx, k, clo, chi, nullptr, nullptr, nullptr, d_cnt + eo, d_flags, ws.s_comp);
+        launch_fast<1>(jac_ctx(ws.s_comp), d_idx, k, clo, chi, nullptr, nullptr, nullptr, d_cnt + eo, d_flags);
         CU_TRY(cudaEventRecord(ws.ev_k1[c], ws.s_comp));
         CU_TRY(cudaEventRecord(ws.ev_chunk[c], ws.s_comp));
         CU_TRY(cudaStreamWaitEvent(ws.s_copy, ws.ev_chunk[c], 0));
@@ -940,8 +750,7 @@ void device_phase1(Slab s, SlabResult* res) {
       CU_TRY(cudaEventRecord(ws.ev_cnt_done, ws.s_copy));
       res->d2h_bytes += (double)s.slab_e;
       if (use_dma) {
-        launch_expand(d_idx, k, s.lo, s.hi, d_cnt, GFICF_MODE_PARALLEL, d_from, d_to, d_w, nullptr, nullptr,
-                      ws.s_comp);
+        launch_expand(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, d_cnt, false, d_from, d_to, d_w, nullptr, nullptr);
         res->launches++;
       }
       CU_TRY(cudaEventRecord(ws.ev_exp, ws.s_comp));
@@ -971,8 +780,7 @@ void device_phase1(Slab s, SlabResult* res) {
         if (clo >= chi) break;
         const long long eo = (clo - s.lo) * k;
         CU_TRY(cudaEventRecord(ws.ev_k0[c], ws.s_comp));
-        launch_fast<0>(d_idx, k, clo, chi, d_from + eo, d_to + eo, d_w + eo, nullptr, d_flags,
-                           ws.s_comp);
+        launch_fast<0>(jac_ctx(ws.s_comp), d_idx, k, clo, chi, d_from + eo, d_to + eo, d_w + eo, nullptr, d_flags);
         CU_TRY(cudaEventRecord(ws.ev_k1[c], ws.s_comp));
         CU_TRY(cudaEventRecord(ws.ev_chunk[c], ws.s_comp));
         res->launches++;
@@ -995,8 +803,7 @@ void device_phase1(Slab s, SlabResult* res) {
     } else if (fast_ok && s.slab_e > 0) {
       ws.counts.need(std::max<size_t>(16, (size_t)s.slab_e * cbytes));
       CU_TRY(cudaEventRecord(ws.ev_k0[0], ws.s_comp));
-      launch_fast<1>(d_idx, k, s.lo, s.hi, nullptr, nullptr, nullptr, ws.counts.p, d_flags,
-                        ws.s_comp);
+      launch_fast<1>(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, nullptr, nullptr, nullptr, ws.counts.p, d_flags);
       CU_TRY(cudaEventRecord(ws.ev_k1[0], ws.s_comp));
       res->launches++;
       res->counts_ready = true;
@@ -1037,11 +844,11 @@ void device_phase2(Slab s, bool exact, SlabResult* res) {
     ws.scratch.need(expand_scratch_bytes(s.slab_e));
     CU_TRY(cudaEventRecord(ws.ev[6], ws.s_comp));
     if (exact || !res->counts_ready) {
-      launch_exact(d_idx, k, s.lo, s.hi, s.mode == GFICF_MODE_SERIAL ? 1 : 0, ws.counts.p, ws.s_comp);
+      launch_exact(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, s.mode == GFICF_MODE_SERIAL ? 1 : 0, ws.counts.p);
       res->launches++;
     }
-    launch_expand(d_idx, k, s.lo, s.hi, ws.counts.p, s.mode, d_from, d_to, d_w, ws.scratch.p, d_nw,
-                  ws.s_comp);
+    launch_expand(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, ws.counts.p, s.mode == GFICF_MODE_SERIAL, d_from, d_to,
+                  d_w, ws.scratch.p, d_nw);
     res->launches += s.mode == GFICF_MODE_SERIAL ? 4 : 1;
     CU_TRY(cudaEventRecord(ws.ev[7], ws.s_comp));
     read_small(ws, res);
@@ -1086,11 +893,6 @@ int default_devices() {
 }
 
 }  // namespace
-
-// the launch plans shared with the CPU emulation (they use CU_TRY)
-#include "network_plan.h"
-#include "snn_plan.h"
-#include "wmu_csc_plan.h"
 
 // ============================================================================
 // C ABI
@@ -1585,8 +1387,7 @@ int gficf_cuda_layout_dev(const double* d_idx_f64, int64_t ld_rows, int64_t ld_r
                           uint32_t* d_flags, void* stream) {
   DEV_BEGIN
   if (!d_idx_f64 || !d_idx_i32 || !d_flags || k < 1 || row_lo < 0 || row_hi > n) return GFICF_E_ARG;
-  launch_layout(d_idx_f64, ld_rows, ld_row0, n, k, row_lo, row_hi, d_idx_i32, d_flags,
-                (cudaStream_t)stream);
+  launch_layout(jac_ctx((cudaStream_t)stream), d_idx_f64, ld_rows, ld_row0, n, k, row_lo, row_hi, d_idx_i32, d_flags);
   return GFICF_OK;
   DEV_END
 }
@@ -1595,12 +1396,7 @@ int gficf_cuda_pad_dev(const int32_t* d_idx_dense, int64_t n, int32_t k, int64_t
                        int64_t row_hi, int32_t* d_idx_i32, uint32_t* d_flags, void* stream) {
   DEV_BEGIN
   if (!d_idx_dense || !d_idx_i32 || !d_flags || k < 1 || row_lo < 0 || row_hi > n) return GFICF_E_ARG;
-  if (row_hi <= row_lo) return GFICF_OK;
-  const int kp = row_stride(k);
-  const long long total = (row_hi - row_lo) * (long long)kp;
-  pad_i32_kernel<<<grid_1d(total, 256, 8), 256, 0, (cudaStream_t)stream>>>(
-      d_idx_dense, n, k, kp, row_lo, row_hi, d_idx_i32, d_flags);
-  CU_TRY(cudaGetLastError());
+  launch_pad(jac_ctx((cudaStream_t)stream), d_idx_dense, n, k, row_lo, row_hi, d_idx_i32, d_flags);
   return GFICF_OK;
   DEV_END
 }
@@ -1611,8 +1407,8 @@ int gficf_cuda_jaccard_dev(const int32_t* d_idx_i32, int64_t n, int32_t k, int64
   DEV_BEGIN
   if (!d_idx_i32 || !d_from || !d_to || !d_w || !d_flags || k < 1 || row_lo < 0 || row_hi > n)
     return GFICF_E_ARG;
-  if (!launch_fast<0>(d_idx_i32, k, row_lo, row_hi, d_from, d_to, d_w, nullptr, d_flags,
-                          (cudaStream_t)stream))
+  if (!launch_fast<0>(jac_ctx((cudaStream_t)stream), d_idx_i32, k, row_lo, row_hi, d_from, d_to, d_w, nullptr,
+                      d_flags))
     return GFICF_E_LIMIT;
   return GFICF_OK;
   DEV_END
@@ -1622,8 +1418,8 @@ int gficf_cuda_jaccard_counts_dev(const int32_t* d_idx_i32, int64_t n, int32_t k
                                   int64_t row_hi, uint8_t* d_u, uint32_t* d_flags, void* stream) {
   DEV_BEGIN
   if (!d_idx_i32 || !d_u || !d_flags || k < 1 || row_lo < 0 || row_hi > n) return GFICF_E_ARG;
-  if (!launch_fast<1>(d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr, (void*)d_u, d_flags,
-                         (cudaStream_t)stream))
+  if (!launch_fast<1>(jac_ctx((cudaStream_t)stream), d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr,
+                      (void*)d_u, d_flags))
     return GFICF_E_LIMIT;
   return GFICF_OK;
   DEV_END
@@ -1639,10 +1435,11 @@ int gficf_cuda_jaccard_counts_tagged_dev(const int32_t* d_idx_i32, int64_t n, in
   tag &= 0x80u;
   // k <= 32: grouped rows, 16-byte vector stores (d_u is typically a peer GPU's memory)
   const bool grouped = k <= 32 && !by_rows;
-  const bool ok = grouped ? launch_fast<3>(d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr, (void*)d_u,
-                                           d_flags, (cudaStream_t)stream, tag)
-                          : launch_fast<1>(d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr, (void*)d_u,
-                                           d_flags, (cudaStream_t)stream, tag);
+  const JacCtx cx = jac_ctx((cudaStream_t)stream);
+  const bool ok = grouped ? launch_fast<3>(cx, d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr, (void*)d_u,
+                                           d_flags, tag)
+                          : launch_fast<1>(cx, d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr, (void*)d_u,
+                                           d_flags, tag);
   if (!ok) return GFICF_E_LIMIT;
   return GFICF_OK;
   DEV_END
@@ -1655,42 +1452,9 @@ int gficf_cuda_expand_stream_dev(const int32_t* d_idx_i32, int32_t k, const int6
   DEV_BEGIN
   if (!d_idx_i32 || !d_u || !d_from || !d_to || !d_w || !d_flags || !seg_lo || !seg_hi) return GFICF_E_ARG;
   if (k < 1 || k > 127 || (tag & ~0x80u) || n_seg < 0 || n_seg > kMaxStreamSegs) return GFICF_E_LIMIT;
-  StreamSegs segs;
-  int ns = 0;
-  long long longest = 0;
-  for (int i = 0; i < n_seg; ++i) {
-    if (seg_lo[i] < 0 || seg_hi[i] < seg_lo[i]) return GFICF_E_ARG;
-    if (seg_hi[i] == seg_lo[i]) continue;
-    segs.lo[ns] = seg_lo[i];
-    segs.hi[ns] = seg_hi[i];
-    longest = std::max<long long>(longest, (seg_hi[i] - seg_lo[i]) * (long long)k);
-    ++ns;
-  }
-  if (!ns) return GFICF_OK;
-  // the resident CTAs are shared evenly by the segments: every sub-grid then advances
-  // through its segment at the same rate as the ranks that produce the segments
-  // two adjacent edges per thread (16-byte stores) when every output column is 16-byte aligned and every
-  // segment starts on an even edge; GFICF_CUDA_STREAM_WIDTH=1 forces the one-edge form (A/B switch)
-  bool pair = (((uintptr_t)d_from | (uintptr_t)d_to | (uintptr_t)d_w) & 15) == 0 && ((uintptr_t)d_u & 1) == 0;
-  for (int i = 0; i < ns; ++i) pair = pair && ((segs.lo[i] * (long long)k) & 1) == 0;
-  const char* we = getenv("GFICF_CUDA_STREAM_WIDTH");
-  if (we && we[0] == '1') pair = false;
-  const int w = pair ? 2 : 1;
-  int per_sm = 0;
-  if (pair) CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, expand_stream_kernel<2>, kExpandThreads, 0));
-  else CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, expand_stream_kernel<1>, kExpandThreads, 0));
-  if (tl_cta_cap > 0 && per_sm > tl_cta_cap) per_sm = tl_cta_cap;  // leave room for a kernel on another stream
-  long long gx = std::max<long long>(1, (long long)sm_count() * std::max(1, per_sm) / ns);
-  gx = std::min<long long>(gx, (longest / w + kExpandThreads - 1) / kExpandThreads);
-  gx = std::max<long long>(gx, 1);
-  const dim3 grid((unsigned)gx, (unsigned)ns);
-  if (pair)
-    expand_stream_kernel<2><<<grid, kExpandThreads, 0, (cudaStream_t)stream>>>(
-        d_idx_i32, k, row_stride(k), segs, d_u, d_from, d_to, d_w, tag, peer_spin_clocks(timeout_ms), d_flags);
-  else
-    expand_stream_kernel<1><<<grid, kExpandThreads, 0, (cudaStream_t)stream>>>(
-        d_idx_i32, k, row_stride(k), segs, d_u, d_from, d_to, d_w, tag, peer_spin_clocks(timeout_ms), d_flags);
-  CU_TRY(cudaGetLastError());
+  if (!launch_expand_stream(jac_ctx((cudaStream_t)stream), d_idx_i32, k, seg_lo, seg_hi, n_seg, d_u, d_from, d_to,
+                            d_w, tag, peer_spin_clocks(timeout_ms), d_flags))
+    return GFICF_E_ARG;
   return GFICF_OK;
   DEV_END
 }
@@ -1699,7 +1463,7 @@ int gficf_cuda_jaccard_exact_dev(const int32_t* d_idx_i32, int64_t n, int32_t k,
                                  int64_t row_hi, int32_t set_semantics, void* d_u, void* stream) {
   DEV_BEGIN
   if (!d_idx_i32 || !d_u || k < 1 || k > 65535 || row_lo < 0 || row_hi > n) return GFICF_E_ARG;
-  launch_exact(d_idx_i32, k, row_lo, row_hi, set_semantics, d_u, (cudaStream_t)stream);
+  launch_exact(jac_ctx((cudaStream_t)stream), d_idx_i32, k, row_lo, row_hi, set_semantics, d_u);
   return GFICF_OK;
   DEV_END
 }
@@ -1716,8 +1480,8 @@ int gficf_cuda_expand_dev(const int32_t* d_idx_i32, int32_t k, int64_t row_lo, i
     return GFICF_E_ARG;
   if (mode == GFICF_MODE_SERIAL && (!d_scratch || !d_n_written)) return GFICF_E_ARG;
   if (mode != GFICF_MODE_SERIAL && mode != GFICF_MODE_PARALLEL) return GFICF_E_ARG;
-  launch_expand(d_idx_i32, k, row_lo, row_hi, d_u, mode, d_from, d_to, d_w, d_scratch,
-                (long long*)d_n_written, (cudaStream_t)stream);
+  launch_expand(jac_ctx((cudaStream_t)stream), d_idx_i32, k, row_lo, row_hi, d_u, mode == GFICF_MODE_SERIAL, d_from,
+                d_to, d_w, d_scratch, (long long*)d_n_written);
   return GFICF_OK;
   DEV_END
 }
@@ -1727,8 +1491,8 @@ int gficf_cuda_jaccard_counts_mutual_dev(const int32_t* d_idx_i32, int64_t n, in
                                          int64_t row_hi, uint8_t* d_um, uint32_t* d_flags, void* stream) {
   DEV_BEGIN
   if (!d_idx_i32 || !d_um || !d_flags || k < 1 || row_lo < 0 || row_hi > n) return GFICF_E_ARG;
-  if (!launch_fast<2>(d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr, (void*)d_um, d_flags,
-                      (cudaStream_t)stream))
+  if (!launch_fast<2>(jac_ctx((cudaStream_t)stream), d_idx_i32, k, row_lo, row_hi, nullptr, nullptr, nullptr,
+                      (void*)d_um, d_flags))
     return GFICF_E_LIMIT;
   return GFICF_OK;
   DEV_END
@@ -1748,14 +1512,7 @@ int gficf_cuda_snn_lower_dev(const int32_t* d_idx_i32, int64_t n, int32_t k, con
     return GFICF_E_ARG;
   if (k > 127 || n >= 0x7fffffffLL || n * (long long)k >= 0xffffffffLL) return GFICF_E_LIMIT;
   if (cap < n * (int64_t)k) return GFICF_E_ARG;
-  static thread_local bool attr_set[64] = {};
-  int dev = 0;
-  CU_TRY(cudaGetDevice(&dev));
-  if (!attr_set[dev & 63]) {
-    CU_TRY(cudaFuncSetAttribute(snn_sort_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                kSnnSmemSortMax * 12));
-    attr_set[dev & 63] = true;
-  }
+  net_max_dynamic_smem(snn_sort_big_kernel, kSnnSmemSortMax * 12);
   snn_lower((cudaStream_t)stream, snn_scratch_layout((char*)d_scratch, n, cap), sm_count() * 8, sm_count() * 2,
             d_idx_i32, n, k, row_stride(k), d_um, (long long*)d_colptr, d_row, d_w, d_vertex_cell,
             (long long*)d_n_vertices, d_flags);
@@ -1806,11 +1563,12 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   const size_t dev_elem = h2d_block(ws, idx_colmajor, n, ws.in_raw.p, n, k, (size_t)elem_bytes, ws.s_comp);
   CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
   if (dev_elem == 8)
-    launch_layout((const double*)ws.in_raw.p, n, 0, n, k, 0, n, (int*)ws.idx.p, d_flags, ws.s_comp);
+    launch_layout(jac_ctx(ws.s_comp), (const double*)ws.in_raw.p, n, 0, n, k, 0, n, (int*)ws.idx.p, d_flags);
   else
-    launch_layout((const int*)ws.in_raw.p, n, 0, n, k, 0, n, (int*)ws.idx.p, d_flags, ws.s_comp);
+    launch_layout(jac_ctx(ws.s_comp), (const int*)ws.in_raw.p, n, 0, n, k, 0, n, (int*)ws.idx.p, d_flags);
   CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
-  if (!launch_fast<2>((const int*)ws.idx.p, k, 0, n, nullptr, nullptr, nullptr, ws.counts.p, d_flags, ws.s_comp))
+  if (!launch_fast<2>(jac_ctx(ws.s_comp), (const int*)ws.idx.p, k, 0, n, nullptr, nullptr, nullptr, ws.counts.p,
+                      d_flags))
     throw Err{GFICF_E_LIMIT, "k outside the range of the mutual-bit count kernel"};
   const int rc = gficf_cuda_snn_lower_dev((const int32_t*)ws.idx.p, n, k, (const uint8_t*)ws.counts.p, d_colptr, d_row,
                                           d_w, E, d_vc, d_nv, ws.scratch.p, d_flags, ws.s_comp);

@@ -260,7 +260,7 @@ def test_jaccard_exact_kernel_and_compaction(libs, oracle, k):
 @pytest.mark.parametrize("k,mode", [(30, 7), (30, 6), (64, 6)])
 def test_jaccard_streaming_expand(libs, oracle, k, mode):
     """Tagged counts (row stores or 8-row groups), then expand_stream_kernel over three segments on a 2 x 3
-    grid: the 2-D CTA order is permuted too."""
+    grid (6 emulated SMs shared by the 3 segments): the 2-D CTA order is permuted too."""
     from tests.conftest import random_knn
     from tests.test_jaccard_slabs_emu import u_of
 
@@ -268,7 +268,7 @@ def test_jaccard_streaming_expand(libs, oracle, k, mode):
     idx = random_knn(rng, k + 40, k)
     lo, hi = 7, k + 40
     par = oracle.parallel_rows(idx, lo, hi)
-    out, cnt, _, flags = _jaccard(libs, idx, mode, lo, hi)
+    out, cnt, _, flags = _jaccard(libs, idx, mode, lo, hi, grid=6)
     assert flags == 0 and np.array_equal(cnt, u_of(par, k) | 0x80) and np.array_equal(out, par)
 
 

@@ -3,9 +3,8 @@ the last output chunk of the host ABI sees; and the hash-failure fallback end to
 
 * Every k in 1..160 and the large-k edges: the fused kernel and counts + expand write rows
   [row_lo, row_hi) into sentinel-filled buffers with guard zones, and the kernel each k is dispatched
-  to (gficf_cuda_last_launch) is the one the CPU emulation's restated dispatch picks
-  (tests/cuda_emu/jaccard_emu.cpp, emu_jaccard_variant): the CPU tests run the kernels through that
-  dispatch, so it must stay the product's.
+  to (gficf_cuda_last_launch) is the one the CPU emulation reports (tests/cuda_emu/jaccard_emu.cpp,
+  emu_jaccard_variant): both run the dispatch of gficf_b200/csrc/jaccard_plan.h.
 * The host ABI cuts a device's rows into chunks whose output leaves while the next chunk is counted;
   a repeated id in the last row must still send the whole call down the exact path.
 * A build with GFICF_MAX_TRIES=1 makes every row whose ids collide under the first multiplier raise

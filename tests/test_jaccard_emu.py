@@ -87,7 +87,7 @@ def test_emulated_fast_kernels_match_oracle(emu, oracle, n, k):
         assert flags == 0 and np.array_equal(ut, u | 0x80)
     if k <= 127:  # both halves of the streaming gather: tagged counts, then the expand that reads (polls) them
         for mode in (6, 7) if k <= 32 else (6,):
-            out, ut, _, flags = run(emu, idx, mode)
+            out, ut, _, flags = run(emu, idx, mode, grid=6)  # 6 emulated SMs: 2 CTAs per segment
             assert flags == 0 and np.array_equal(ut, u | 0x80) and np.array_equal(out, want), mode
 
 

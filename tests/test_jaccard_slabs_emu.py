@@ -174,8 +174,8 @@ def slab_of(rng, n, which, max_rows=None):
 @pytest.mark.parametrize("k", range(1, 129))
 def test_every_k_on_slabs(emu, oracle, k):
     """Counts + expand (mode 1) at every k <= 128, the mutual bit (mode 4) for k <= 127, the fused kernel
-    (mode 0) for k <= 32 and every third k above; input family, slab start, slab end and grid vary with k
-    (one CTA, a few, and more warps than rows)."""
+    (mode 0) for k <= 32 and every third k above; input family, slab start, slab end and the emulated SM
+    count vary with k (one SM, a few, and more SMs than the slab gives the persistent kernels work for)."""
     rng = np.random.default_rng(1000 + k)
     fam = FAMILIES[k % len(FAMILIES)]
     idx = fam(rng, k, 24)
@@ -257,7 +257,7 @@ def test_streaming_gather_on_slabs(emu, oracle, k, mode):
     n = idx.shape[0]
     for lo, hi in ((7, n), (9, n - 5), (17, n - 2)):
         par = oracle.parallel_rows(idx, lo, hi)
-        out, cnt, _, flags = run_slab(emu, idx, mode, lo, hi, offset=lo % 2)
+        out, cnt, _, flags = run_slab(emu, idx, mode, lo, hi, grid=6, offset=lo % 2)  # 2 CTAs per segment
         assert flags == 0 and np.array_equal(cnt, u_of(par, k) | 0x80) and np.array_equal(out, par), (lo, hi)
 
 
