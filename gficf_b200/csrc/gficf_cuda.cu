@@ -203,7 +203,6 @@ struct DeviceWs {
   bool init = false;
   cudaStream_t s_comp = nullptr, s_copy = nullptr;
   cudaEvent_t ev[8] = {};
-  cudaEvent_t ev_chunk[kMaxChunks] = {};
   cudaEvent_t ev_k0[kMaxChunks] = {}, ev_k1[kMaxChunks] = {};
   // in_raw: device copy of the caller's rows (f64 or int32, column-major); small: flags + n_written
   Buf in_raw, idx, out, counts, scratch, small;
@@ -220,7 +219,6 @@ struct DeviceWs {
     CU_TRY(cudaStreamCreateWithFlags(&s_comp, cudaStreamNonBlocking));
     CU_TRY(cudaStreamCreateWithFlags(&s_copy, cudaStreamNonBlocking));
     for (auto& e : ev) CU_TRY(cudaEventCreate(&e));
-    for (auto& e : ev_chunk) CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     for (auto& e : ev_k0) CU_TRY(cudaEventCreate(&e));
     for (auto& e : ev_k1) CU_TRY(cudaEventCreate(&e));
     for (auto& e : ev_slot) CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -247,7 +245,6 @@ struct DeviceWs {
     if (h_small) cudaFreeHost(h_small);
     h_small = nullptr;
     for (auto& e : ev) cudaEventDestroy(e);
-    for (auto& e : ev_chunk) cudaEventDestroy(e);
     for (auto& e : ev_k0) cudaEventDestroy(e);
     for (auto& e : ev_k1) cudaEventDestroy(e);
     for (auto& e : ev_slot) cudaEventDestroy(e);
@@ -371,19 +368,12 @@ OutMode out_mode_env() {
   return kOutAuto;
 }
 
-struct Piece {
-  char* host;
-  char* dev;
-  size_t bytes;
-  cudaEvent_t wait_before;
-};
-
 // narrow (host -> device only): the source holds ids as doubles; the workers convert every piece to
 // int32 inside its pinned slot (gficf_host::f64_to_i32) and the copy engine moves HALF the bytes;
-// Seg.bytes / Piece.bytes count SOURCE bytes, Seg.dev addresses the int32 destination.
+// Seg.bytes counts SOURCE bytes, Seg.dev addresses the int32 destination.
 void staged_copy(DeviceWs& ws, const std::vector<Seg>& segs, bool to_device, cudaStream_t st,
                  bool narrow = false) {
-  std::vector<Piece> pieces;
+  std::vector<Seg> pieces;
   for (const Seg& g : segs) {
     bool first = true;
     for (size_t off = 0; off < g.bytes; off += kStageChunk) {
@@ -413,7 +403,7 @@ void staged_copy(DeviceWs& ws, const std::vector<Seg>& segs, bool to_device, cud
     for (;;) {
       const int j = next.fetch_add(1);
       if (j >= np || failed.load()) return;
-      const Piece& pc = pieces[j];
+      const Seg& pc = pieces[j];
       char* slot = ring + (size_t)(j % kStageSlots) * kStageChunk;
       if (to_device) {
         // the slot is free once the DMA of piece j - kStageSlots has completed
@@ -442,7 +432,7 @@ void staged_copy(DeviceWs& ws, const std::vector<Seg>& segs, bool to_device, cud
   for (int t = 0; t < nthreads; ++t) pool.emplace_back(worker);
   cudaError_t err = cudaSuccess;
   for (int j = 0; j < np && err == cudaSuccess; ++j) {
-    const Piece& pc = pieces[j];
+    const Seg& pc = pieces[j];
     char* slot = ring + (size_t)(j % kStageSlots) * kStageChunk;
     if (pc.wait_before) err = cudaStreamWaitEvent(st, pc.wait_before, 0);
     // a worker that failed stops marking pieces: never wait for it (failed ends the loop below)
@@ -550,20 +540,34 @@ struct Slab {
   ncclComm_t comm = nullptr;  // communicator of this rank when ndev > 1
   long long n, rows_per, lo, hi, rows, E, slab_e;
   const void* h_idx;
-  int elem = 8;  // bytes per element of the caller's matrix: 8 = double, 4 = int32
-  int out_mode = kOutDma;  // resolved OutMode of this call (never kOutAuto)
+  int elem;      // bytes per element of the caller's matrix: 8 = double, 4 = int32
+  int out_mode;  // resolved OutMode of this call (never kOutAuto)
   double* h_out;
-  Slab(int rank_, int ndev_, const void* h_idx_, long long n_, int k_, long long rows_per_,
-       double* h_out_, int mode_)
+  Slab(int rank_, int ndev_, const void* h_idx_, int elem_, long long n_, int k_, long long rows_per_,
+       double* h_out_, int mode_, int out_mode_)
       : rank(rank_), ndev(ndev_), k(k_), kp(row_stride(k_)), mode(mode_), dev(rank_), n(n_),
-        rows_per(rows_per_), h_idx(h_idx_), h_out(h_out_) {
+        rows_per(rows_per_), h_idx(h_idx_), elem(elem_), out_mode(out_mode_), h_out(h_out_) {
     lo = std::min<long long>(n, rank * rows_per);
     hi = std::min<long long>(n, lo + rows_per);
     rows = hi - lo;
     E = n * (long long)k;
     slab_e = rows * (long long)k;
   }
+  // output column c (0 from, 1 to, 2 weight) of this slab: in the caller's matrix, and in ws.out
+  double* h_col(int c) const { return h_out + c * E + lo * k; }
+  double* d_col(const DeviceWs& ws, int c) const { return (double*)ws.out.p + c * slab_e; }
+  int count_bytes() const { return k <= 255 ? 1 : 2; }  // per edge in ws.counts
+  void need_counts(DeviceWs& ws) const {  // counts and compaction scratch of the exact / expand kernels
+    ws.counts.need(std::max<size_t>(16, (size_t)slab_e * count_bytes()));
+    ws.scratch.need(expand_scratch_bytes(slab_e));
+  }
 };
+
+float event_ms(cudaEvent_t a, cudaEvent_t b) {
+  float ms = 0;
+  CU_TRY(cudaEventElapsedTime(&ms, a, b));
+  return ms;
+}
 
 void read_small(DeviceWs& ws, SlabResult* res) {
   CU_TRY(cudaMemcpyAsync(ws.h_small, ws.small.p, 16, cudaMemcpyDeviceToHost, ws.s_comp));
@@ -572,21 +576,14 @@ void read_small(DeviceWs& ws, SlabResult* res) {
 }
 
 void d2h_slab(DeviceWs& ws, const Slab& s, SlabResult* res) {
-  double* d_from = (double*)ws.out.p;
-  double* d_to = d_from + s.slab_e;
-  double* d_w = d_to + s.slab_e;
   CU_TRY(cudaEventRecord(ws.ev[4], ws.s_copy));
-  const size_t bytes = (size_t)s.slab_e * sizeof(double);
-  d2h_segs(ws,
-           {{(char*)(s.h_out + s.lo * s.k), (char*)d_from, bytes, nullptr},
-            {(char*)(s.h_out + s.E + s.lo * s.k), (char*)d_to, bytes, nullptr},
-            {(char*)(s.h_out + 2 * s.E + s.lo * s.k), (char*)d_w, bytes, nullptr}},
-           ws.s_copy);
+  std::vector<Seg> segs;
+  for (int c = 0; c < 3; ++c)
+    segs.push_back({(char*)s.h_col(c), (char*)s.d_col(ws, c), (size_t)s.slab_e * sizeof(double), nullptr});
+  d2h_segs(ws, segs, ws.s_copy);
   CU_TRY(cudaEventRecord(ws.ev[5], ws.s_copy));
   CU_TRY(cudaStreamSynchronize(ws.s_copy));
-  float ms = 0;
-  CU_TRY(cudaEventElapsedTime(&ms, ws.ev[4], ws.ev[5]));
-  res->ms_d2h += ms;
+  res->ms_d2h += event_ms(ws.ev[4], ws.ev[5]);
 }
 
 // Counts-over-PCIe output of the parallel export (modes host / hybrid, see OutMode).
@@ -636,7 +633,6 @@ void counts_output_phase(DeviceWs& ws, const Slab& s, SlabResult* res, bool use_
   cudaError_t err = cudaSuccess;
   long long dma_items = 0;
   if (use_dma) {
-    const double* d_out = (const double*)ws.out.p;
     err = cudaStreamWaitEvent(ws.s_copy, ws.ev_exp, 0);
     long long it;
     // at most 3 copies queued: the copy engine never idles, and it never claims far ahead of what it moves
@@ -646,9 +642,8 @@ void counts_output_phase(DeviceWs& ws, const Slab& s, SlabResult* res, bool use_
       const size_t bytes = (size_t)(b - a) * k * sizeof(double);
       if (dma_items >= 3) err = cudaEventSynchronize(ws.ev_dma[(dma_items - 3) & 3]);
       if (err == cudaSuccess)
-        err = cudaMemcpyAsync(s.h_out + (size_t)col * s.E + (size_t)(s.lo + a) * k,
-                              d_out + (size_t)col * s.slab_e + (size_t)a * k, bytes, cudaMemcpyDeviceToHost,
-                              ws.s_copy);
+        err = cudaMemcpyAsync(s.h_col(col) + (size_t)a * k, s.d_col(ws, col) + (size_t)a * k, bytes,
+                              cudaMemcpyDeviceToHost, ws.s_copy);
       if (err == cudaSuccess) err = cudaEventRecord(ws.ev_dma[dma_items & 3], ws.s_copy);
       res->d2h_bytes += (double)bytes;
       ++dma_items;
@@ -661,11 +656,25 @@ void counts_output_phase(DeviceWs& ws, const Slab& s, SlabResult* res, bool use_
   res->host_items = (double)cpu_items.load() / (double)std::max<long long>(1, nitems);
 }
 
-// Phase 1 of one device's share (rows [lo,hi) of n): H2D of its rows, layout pre-pass, exchange
-// of the int32 index slabs (in-place NCCL all-gather when ndev>1), then the fast kernel:
-//   parallel export, k<=128: fused kernel in row chunks, the D2H of chunk c overlapping the
-//     kernel of chunk c+1 (the result stands unless some device raises a dup/hash flag);
-//   serial export, k<=128:   fast count kernel (the compaction happens in phase 2).
+// Flags cleared, then rows [lo,hi) of the caller's n x k column-major ids (elem bytes each) uploaded into
+// ws.in_raw (ev[0]..ev[1]) and laid out as padded int32 rows in ws.idx (ev[1]..ev[2]).  Returns the bytes
+// copied host -> device.  Phase 0 of the Jaccard call and of the graph build.
+double upload_rows(DeviceWs& ws, const void* h_idx, int elem, long long n, int k, long long lo, long long hi) {
+  const long long rows = hi - lo;
+  unsigned* d_flags = (unsigned*)ws.small.p;
+  CU_TRY(cudaMemsetAsync(ws.small.p, 0, 64, ws.s_comp));
+  CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
+  const size_t dev_elem =
+      h2d_block(ws, (const char*)h_idx + (size_t)lo * elem, n, ws.in_raw.p, rows, k, (size_t)elem, ws.s_comp);
+  CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
+  if (dev_elem == 8)
+    launch_layout(jac_ctx(ws.s_comp), (const double*)ws.in_raw.p, rows, lo, n, k, lo, hi, (int*)ws.idx.p, d_flags);
+  else
+    launch_layout(jac_ctx(ws.s_comp), (const int*)ws.in_raw.p, rows, lo, n, k, lo, hi, (int*)ws.idx.p, d_flags);
+  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
+  return (double)rows * k * dev_elem;
+}
+
 // Phase 0: everything that can fail locally -- workspaces, H2D of the device's rows, layout
 // pre-pass.  No collective in here: if any device fails, the call ends before anybody enters the
 // all-gather (a collective that one participant never joins would hang the others' GPUs).
@@ -674,43 +683,31 @@ void device_phase0(Slab s, SlabResult* res) {
     DeviceWs& ws = g_ws[s.dev];
     CU_TRY(cudaSetDevice(s.dev));
     ws.ensure(s.dev);
-    const int k = s.k;
-    const int cbytes = k <= 255 ? 1 : 2;
-    ws.in_raw.need(std::max<size_t>(16, (size_t)s.rows * k * s.elem));
+    ws.in_raw.need(std::max<size_t>(16, (size_t)s.rows * s.k * s.elem));
     ws.idx.need(std::max<size_t>(16, (size_t)s.rows_per * s.ndev * s.kp * sizeof(int)));
     if (s.out_mode != kOutHost) ws.out.need(std::max<size_t>(16, (size_t)s.slab_e * 3 * sizeof(double)));
-    if (s.mode == GFICF_MODE_SERIAL || k > kLargeMaxK || s.out_mode != kOutDma) {
-      ws.counts.need(std::max<size_t>(16, (size_t)s.slab_e * cbytes));
-      ws.scratch.need(expand_scratch_bytes(s.slab_e));
-    }
+    if (s.mode == GFICF_MODE_SERIAL || s.k > kLargeMaxK || s.out_mode != kOutDma) s.need_counts(ws);
     if (s.out_mode != kOutDma) ws.h_counts.need(std::max<size_t>(16, (size_t)s.slab_e));
     if (s.out_mode == kOutHost) ws.out.need(16);  // grown on demand should the exact path be needed
-    unsigned* d_flags = (unsigned*)ws.small.p;
-    CU_TRY(cudaMemsetAsync(ws.small.p, 0, 64, ws.s_comp));
-    CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
-    const size_t dev_elem = h2d_block(ws, (const char*)s.h_idx + (size_t)s.lo * s.elem, s.n, ws.in_raw.p,
-                                      s.rows, k, s.elem, ws.s_comp);
-    res->h2d_bytes = (double)s.rows * k * dev_elem;
-    CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
-    if (dev_elem == 8)
-      launch_layout(jac_ctx(ws.s_comp), (const double*)ws.in_raw.p, s.rows, s.lo, s.n, k, s.lo, s.hi,
-                    (int*)ws.idx.p, d_flags);
-    else
-      launch_layout(jac_ctx(ws.s_comp), (const int*)ws.in_raw.p, s.rows, s.lo, s.n, k, s.lo, s.hi, (int*)ws.idx.p,
-                    d_flags);
+    res->h2d_bytes = upload_rows(ws, s.h_idx, s.elem, s.n, s.k, s.lo, s.hi);
     res->launches += s.rows > 0;
-    CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
   } catch (const Err& e) {
     res->err = e;
   }
 }
 
+// Phase 1: exchange of the int32 index slabs (in-place NCCL all-gather when ndev>1), then the fast kernel:
+//   parallel export, k<=128, counts over PCIe (out_mode host / hybrid): count kernel in row chunks, the D2H
+//     of chunk c's counts overlapping the kernel of chunk c+1, then the output phase;
+//   parallel export, k<=128, dma: fused kernel in row chunks, the D2H of chunk c overlapping the
+//     kernel of chunk c+1 (the result stands unless some device raises a dup/hash flag);
+//   serial export, k<=128:   fast count kernel (the compaction happens in phase 2).
+// Chunk c of the kernel runs between ev_k0[c] and ev_k1[c]; the copy of its output waits for ev_k1[c].
 void device_phase1(Slab s, SlabResult* res) {
   try {
     DeviceWs& ws = g_ws[s.dev];
     CU_TRY(cudaSetDevice(s.dev));
     const int k = s.k;
-    const int cbytes = k <= 255 ? 1 : 2;
     unsigned* d_flags = (unsigned*)ws.small.p;
     if (s.ndev > 1) {
       const size_t cnt = (size_t)s.rows_per * s.kp;
@@ -721,10 +718,8 @@ void device_phase1(Slab s, SlabResult* res) {
 
     const int* d_idx = (const int*)ws.idx.p;
     const bool fast_ok = k <= kLargeMaxK;
-    double* d_from = (double*)ws.out.p;
-    double* d_to = d_from + s.slab_e;
-    double* d_w = d_to + s.slab_e;
-    int used = 0;
+    int used = 0;           // kernel chunks timed by ev_k0 / ev_k1
+    bool d2h_timed = false;  // ev[4]..ev[5] enclose the D2H of the fused kernel's output
     if (fast_ok && s.mode == GFICF_MODE_PARALLEL && s.out_mode != kOutDma && s.slab_e > 0) {
       // counts-over-PCIe: count kernel in row chunks, the D2H of chunk c's counts overlapping the
       // kernel of chunk c+1; then the output phase (host threads [+ copy engine])
@@ -740,8 +735,7 @@ void device_phase1(Slab s, SlabResult* res) {
         CU_TRY(cudaEventRecord(ws.ev_k0[c], ws.s_comp));
         launch_fast<1>(jac_ctx(ws.s_comp), d_idx, k, clo, chi, nullptr, nullptr, nullptr, d_cnt + eo, d_flags);
         CU_TRY(cudaEventRecord(ws.ev_k1[c], ws.s_comp));
-        CU_TRY(cudaEventRecord(ws.ev_chunk[c], ws.s_comp));
-        CU_TRY(cudaStreamWaitEvent(ws.s_copy, ws.ev_chunk[c], 0));
+        CU_TRY(cudaStreamWaitEvent(ws.s_copy, ws.ev_k1[c], 0));
         CU_TRY(cudaMemcpyAsync((char*)ws.h_counts.p + eo, d_cnt + eo, (size_t)(chi - clo) * k,
                                cudaMemcpyDeviceToHost, ws.s_copy));
         res->launches++;
@@ -750,7 +744,8 @@ void device_phase1(Slab s, SlabResult* res) {
       CU_TRY(cudaEventRecord(ws.ev_cnt_done, ws.s_copy));
       res->d2h_bytes += (double)s.slab_e;
       if (use_dma) {
-        launch_expand(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, d_cnt, false, d_from, d_to, d_w, nullptr, nullptr);
+        launch_expand(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, d_cnt, false, s.d_col(ws, 0), s.d_col(ws, 1),
+                      s.d_col(ws, 2), nullptr, nullptr);
         res->launches++;
       }
       CU_TRY(cudaEventRecord(ws.ev_exp, ws.s_comp));
@@ -760,65 +755,48 @@ void device_phase1(Slab s, SlabResult* res) {
       if (!(res->flags & (kFlagBadId | kFlagDupId | kFlagHashFail)))
         counts_output_phase(ws, s, res, use_dma);  // else: the exact path rewrites everything
       res->ms_d2h = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_out0).count();
-      CU_TRY(cudaStreamSynchronize(ws.s_copy));
-      CU_TRY(cudaEventElapsedTime(&res->ms_h2d, ws.ev[0], ws.ev[1]));
-      CU_TRY(cudaEventElapsedTime(&res->ms_k0, ws.ev[1], ws.ev[2]));
-      CU_TRY(cudaEventElapsedTime(&res->ms_gather, ws.ev[2], ws.ev[3]));
-      for (int c = 0; c < used; ++c) {
-        float ms = 0;
-        CU_TRY(cudaEventElapsedTime(&ms, ws.ev_k0[c], ws.ev_k1[c]));
-        res->ms_k1 += ms;
-      }
-      return;
-    }
-    if (fast_ok && s.mode == GFICF_MODE_PARALLEL) {
-      const int nch =
-          (int)std::min<long long>(kMaxChunks, std::max<long long>(1, s.slab_e * 24 / (48ll << 20)));
-      const long long rpc = (s.rows + nch - 1) / nch;
-      for (int c = 0; c < nch; ++c) {
-        const long long clo = s.lo + c * rpc, chi = std::min(s.hi, clo + rpc);
-        if (clo >= chi) break;
-        const long long eo = (clo - s.lo) * k;
-        CU_TRY(cudaEventRecord(ws.ev_k0[c], ws.s_comp));
-        launch_fast<0>(jac_ctx(ws.s_comp), d_idx, k, clo, chi, d_from + eo, d_to + eo, d_w + eo, nullptr, d_flags);
-        CU_TRY(cudaEventRecord(ws.ev_k1[c], ws.s_comp));
-        CU_TRY(cudaEventRecord(ws.ev_chunk[c], ws.s_comp));
+    } else {
+      if (fast_ok && s.mode == GFICF_MODE_PARALLEL) {
+        const int nch =
+            (int)std::min<long long>(kMaxChunks, std::max<long long>(1, s.slab_e * 24 / (48ll << 20)));
+        const long long rpc = (s.rows + nch - 1) / nch;
+        std::vector<Seg> segs;
+        for (int c = 0; c < nch; ++c) {
+          const long long clo = s.lo + c * rpc, chi = std::min(s.hi, clo + rpc);
+          if (clo >= chi) break;
+          const long long eo = (clo - s.lo) * k;
+          CU_TRY(cudaEventRecord(ws.ev_k0[c], ws.s_comp));
+          launch_fast<0>(jac_ctx(ws.s_comp), d_idx, k, clo, chi, s.d_col(ws, 0) + eo, s.d_col(ws, 1) + eo,
+                         s.d_col(ws, 2) + eo, nullptr, d_flags);
+          CU_TRY(cudaEventRecord(ws.ev_k1[c], ws.s_comp));
+          for (int col = 0; col < 3; ++col)
+            segs.push_back({(char*)(s.h_col(col) + eo), (char*)(s.d_col(ws, col) + eo),
+                            (size_t)(chi - clo) * k * sizeof(double), col == 0 ? ws.ev_k1[c] : nullptr});
+          res->launches++;
+          used = c + 1;
+        }
+        CU_TRY(cudaStreamWaitEvent(ws.s_copy, ws.ev[3], 0));
+        CU_TRY(cudaEventRecord(ws.ev[4], ws.s_copy));
+        d2h_segs(ws, segs, ws.s_copy);
+        res->d2h_bytes += 24.0 * (double)s.slab_e;
+        CU_TRY(cudaEventRecord(ws.ev[5], ws.s_copy));
+        d2h_timed = used > 0;
+      } else if (fast_ok && s.slab_e > 0) {
+        CU_TRY(cudaEventRecord(ws.ev_k0[0], ws.s_comp));
+        launch_fast<1>(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, nullptr, nullptr, nullptr, ws.counts.p, d_flags);
+        CU_TRY(cudaEventRecord(ws.ev_k1[0], ws.s_comp));
         res->launches++;
-        used = c + 1;
+        res->counts_ready = true;
+        used = 1;
       }
-      CU_TRY(cudaStreamWaitEvent(ws.s_copy, ws.ev[3], 0));
-      CU_TRY(cudaEventRecord(ws.ev[4], ws.s_copy));
-      std::vector<Seg> segs;
-      for (int c = 0; c < used; ++c) {
-        const long long clo = s.lo + c * rpc, chi = std::min(s.hi, clo + rpc);
-        const long long eo = (clo - s.lo) * k;
-        const size_t cb = (size_t)(chi - clo) * k * sizeof(double);
-        segs.push_back({(char*)(s.h_out + s.lo * k + eo), (char*)(d_from + eo), cb, ws.ev_chunk[c]});
-        segs.push_back({(char*)(s.h_out + s.E + s.lo * k + eo), (char*)(d_to + eo), cb, nullptr});
-        segs.push_back({(char*)(s.h_out + 2 * s.E + s.lo * k + eo), (char*)(d_w + eo), cb, nullptr});
-      }
-      d2h_segs(ws, segs, ws.s_copy);
-      res->d2h_bytes += 24.0 * (double)s.slab_e;
-      CU_TRY(cudaEventRecord(ws.ev[5], ws.s_copy));
-    } else if (fast_ok && s.slab_e > 0) {
-      ws.counts.need(std::max<size_t>(16, (size_t)s.slab_e * cbytes));
-      CU_TRY(cudaEventRecord(ws.ev_k0[0], ws.s_comp));
-      launch_fast<1>(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, nullptr, nullptr, nullptr, ws.counts.p, d_flags);
-      CU_TRY(cudaEventRecord(ws.ev_k1[0], ws.s_comp));
-      res->launches++;
-      res->counts_ready = true;
+      read_small(ws, res);
     }
-    read_small(ws, res);
     CU_TRY(cudaStreamSynchronize(ws.s_copy));
-    CU_TRY(cudaEventElapsedTime(&res->ms_h2d, ws.ev[0], ws.ev[1]));
-    CU_TRY(cudaEventElapsedTime(&res->ms_k0, ws.ev[1], ws.ev[2]));
-    CU_TRY(cudaEventElapsedTime(&res->ms_gather, ws.ev[2], ws.ev[3]));
-    for (int c = 0; c < std::max(used, res->counts_ready ? 1 : 0); ++c) {
-      float ms = 0;
-      CU_TRY(cudaEventElapsedTime(&ms, ws.ev_k0[c], ws.ev_k1[c]));
-      res->ms_k1 += ms;
-    }
-    if (used) CU_TRY(cudaEventElapsedTime(&res->ms_d2h, ws.ev[4], ws.ev[5]));
+    res->ms_h2d = event_ms(ws.ev[0], ws.ev[1]);
+    res->ms_k0 = event_ms(ws.ev[1], ws.ev[2]);
+    res->ms_gather = event_ms(ws.ev[2], ws.ev[3]);
+    for (int c = 0; c < used; ++c) res->ms_k1 += event_ms(ws.ev_k0[c], ws.ev_k1[c]);
+    if (d2h_timed) res->ms_d2h = event_ms(ws.ev[4], ws.ev[5]);
   } catch (const Err& e) {
     res->err = e;
   }
@@ -833,29 +811,22 @@ void device_phase2(Slab s, bool exact, SlabResult* res) {
     CU_TRY(cudaSetDevice(s.dev));
     if (s.slab_e <= 0) return;
     const int k = s.k;
-    const int cbytes = k <= 255 ? 1 : 2;
     const int* d_idx = (const int*)ws.idx.p;
     ws.out.need(std::max<size_t>(16, (size_t)s.slab_e * 3 * sizeof(double)));  // host mode kept it empty
-    double* d_from = (double*)ws.out.p;
-    double* d_to = d_from + s.slab_e;
-    double* d_w = d_to + s.slab_e;
     long long* d_nw = (long long*)((char*)ws.small.p + 8);
-    ws.counts.need(std::max<size_t>(16, (size_t)s.slab_e * cbytes));
-    ws.scratch.need(expand_scratch_bytes(s.slab_e));
+    s.need_counts(ws);
     CU_TRY(cudaEventRecord(ws.ev[6], ws.s_comp));
     if (exact || !res->counts_ready) {
       launch_exact(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, s.mode == GFICF_MODE_SERIAL ? 1 : 0, ws.counts.p);
       res->launches++;
     }
-    launch_expand(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, ws.counts.p, s.mode == GFICF_MODE_SERIAL, d_from, d_to,
-                  d_w, ws.scratch.p, d_nw);
+    launch_expand(jac_ctx(ws.s_comp), d_idx, k, s.lo, s.hi, ws.counts.p, s.mode == GFICF_MODE_SERIAL,
+                  s.d_col(ws, 0), s.d_col(ws, 1), s.d_col(ws, 2), ws.scratch.p, d_nw);
     res->launches += s.mode == GFICF_MODE_SERIAL ? 4 : 1;
     CU_TRY(cudaEventRecord(ws.ev[7], ws.s_comp));
     read_small(ws, res);
     if (s.mode == GFICF_MODE_SERIAL) res->n_written = *(long long*)((char*)ws.h_small + 8);
-    float ms = 0;
-    CU_TRY(cudaEventElapsedTime(&ms, ws.ev[6], ws.ev[7]));
-    res->ms_k1 += ms;
+    res->ms_k1 += event_ms(ws.ev[6], ws.ev[7]);
     d2h_slab(ws, s, res);
   } catch (const Err& e) {
     res->err = e;
@@ -1050,12 +1021,6 @@ struct DeviceRestore {
   }
 };
 
-float event_ms(cudaEvent_t a, cudaEvent_t b) {
-  float ms = 0;
-  CU_TRY(cudaEventElapsedTime(&ms, a, b));
-  return ms;
-}
-
 // One single-device host-buffer call: a device must be visible; the call holds g_call_mu and runs on device 0
 // with its workspace ready, and the caller's device is current again when it ends.
 struct SingleDeviceCall {
@@ -1079,20 +1044,129 @@ struct SingleDeviceCall {
   }
 };
 
-int jaccard_host_call(const void* idx, int elem, int64_t n, int32_t k, double* out, int32_t n_devices,
-                      int32_t mode, int64_t* n_written, char* err, size_t errlen) {
-  API_BEGIN
-  if (err && errlen) err[0] = 0;
+// The reference holds rows and nrow*ncol in `int` (rcpp_parallel_jaccard_coeff.cpp:28,67)
+void check_nk_limit(int64_t n, int32_t k) {
+  if (n >= 0x7fffffffLL - 2 || (long double)n * k >= 2147483647.0L)
+    throw Err{GFICF_E_LIMIT, "n*k must stay below 2^31 (the reference's int row index)"};
+}
+
+// Argument checks of the Jaccard host entries; false for an empty matrix (nothing to do, no device needed).
+bool jaccard_check_args(const void* idx, const double* out, int64_t n, int32_t k, int32_t mode, int64_t* n_written) {
   if (n < 0 || k < 0) throw Err{GFICF_E_ARG, "negative matrix dimension"};
   if (mode != GFICF_MODE_PARALLEL && mode != GFICF_MODE_SERIAL)
     throw Err{GFICF_E_ARG, "mode must be 0 (parallel, fixed slots) or 1 (serial, compacted)"};
   if (n_written) *n_written = 0;
-  if (n == 0 || k == 0) return GFICF_OK;
+  if (n == 0 || k == 0) return false;
   if (!idx || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
-  // the reference holds rows and nrow*ncol in `int` (rcpp_parallel_jaccard_coeff.cpp:28,67)
-  if (n >= 0x7fffffffLL - 2 || (long double)n * k >= 2147483647.0L)
-    throw Err{GFICF_E_LIMIT, "n*k must stay below 2^31 (the reference's int row index)"};
+  check_nk_limit(n, k);
   if (k > 65535) throw Err{GFICF_E_LIMIT, "k above 65535 is not supported"};
+  return true;
+}
+
+// fn(slab, &result) for every slab of this process: inline for one, one host thread per slab for several
+template <class F>
+void for_each_slab(const std::vector<Slab>& slabs, std::vector<SlabResult>& res, F fn) {
+  if (slabs.size() == 1) {
+    fn(slabs[0], &res[0]);
+    return;
+  }
+  std::vector<std::thread> th;
+  for (size_t r = 0; r < slabs.size(); ++r) th.emplace_back(fn, slabs[r], &res[r]);
+  for (auto& t : th) t.join();
+}
+
+// What the slabs agree on after a phase: the OR of their flags, returned.  The slabs of this process are
+// merged on the host; with a communicator of all ranks (one process per GPU) the merged bits then go
+// through one ncclAllReduce(max), which every rank enters whether it failed or not.  Unless some slab saw
+// a bad id (the caller raises GFICF_E_RANGE), a failure ends the call the same way everywhere: this
+// process's first error, else `peer_failed`.
+unsigned agree(const std::vector<Slab>& slabs, const std::vector<SlabResult>& res, ncclComm_t world,
+               const char* peer_failed) {
+  unsigned flags = 0;
+  bool failed = false;
+  for (auto& r : res) {
+    flags |= r.flags;
+    failed |= r.err.code != GFICF_OK;
+  }
+  bool peer = false;
+  if (world) {
+    DeviceWs& ws = g_ws[slabs[0].dev];
+    CU_TRY(cudaSetDevice(slabs[0].dev));
+    ws.ensure(slabs[0].dev);  // phase 0 may have failed before it
+    int* bits = (int*)((char*)ws.small.p + 32);
+    int h[4] = {(int)(flags & kFlagBadId) != 0, (int)(flags & kFlagDupId) != 0, (int)(flags & kFlagHashFail) != 0,
+                failed};
+    CU_TRY(cudaMemcpyAsync(bits, h, sizeof h, cudaMemcpyHostToDevice, ws.s_comp));
+    NCCL_TRY(nccl_dyn::get().AllReduce(bits, bits, 4, ncclInt32, ncclMax, world, ws.s_comp));
+    CU_TRY(cudaMemcpyAsync(h, bits, sizeof h, cudaMemcpyDeviceToHost, ws.s_comp));
+    CU_TRY(cudaStreamSynchronize(ws.s_comp));
+    flags = (h[0] ? kFlagBadId : 0u) | (h[1] ? kFlagDupId : 0u) | (h[2] ? kFlagHashFail : 0u);
+    peer = h[3] != 0;
+  }
+  if (flags & kFlagBadId) return flags;
+  for (auto& r : res)
+    if (r.err.code != GFICF_OK) throw r.err;
+  if (peer) throw Err{GFICF_E_CUDA, peer_failed};
+  return flags;
+}
+
+// One Jaccard call over the row slabs of this process: phase 0, agree, phase 1, agree, then phase 2 when
+// the exact path or the serial compaction is needed.  `world` is null when the slabs of this process are the
+// whole matrix (several of them exchange their index slabs over g_nccl's communicators), and the
+// communicator of all ranks when each process brings one slab.  Writes gficf_cuda_last_timings /
+// _last_output (thread-local: the caller reads them on this thread) and returns n_written of the serial
+// export.  A bad id anywhere -> GFICF_E_RANGE, on every rank.
+long long run_slabs(std::vector<Slab>& slabs, ncclComm_t world) {
+  std::lock_guard<std::mutex> lk(g_call_mu);
+  DeviceRestore restore;
+  const auto t0 = std::chrono::steady_clock::now();
+  const int ns = (int)slabs.size();
+  g_active_devices.store(ns);
+  if (!world && ns > 1) {
+    nccl_ensure(ns);
+    for (int r = 0; r < ns; ++r) slabs[r].comm = g_nccl.comms[r];
+  }
+  std::vector<SlabResult> res(ns);
+  for_each_slab(slabs, res, device_phase0);
+  // nobody has entered a collective yet: a slab that failed ends the call here, on every rank
+  agree(slabs, res, world, "another rank failed before the index exchange");
+  for_each_slab(slabs, res, device_phase1);
+  const unsigned flags = agree(slabs, res, world, "another rank failed");
+  if (!(flags & kFlagBadId)) {
+    const bool exact = slabs[0].k > kLargeMaxK || (flags & (kFlagDupId | kFlagHashFail));
+    if (exact || slabs[0].mode == GFICF_MODE_SERIAL) {
+      for_each_slab(slabs, res, [exact](Slab s, SlabResult* r) { device_phase2(s, exact, r); });
+      for (auto& r : res)
+        if (r.err.code != GFICF_OK) throw r.err;
+    }
+  }
+  const auto t1 = std::chrono::steady_clock::now();
+  double tm[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  double h2d_total = 0;
+  for (auto& r : res) {
+    tm[0] = std::max<double>(tm[0], r.ms_h2d);
+    tm[1] = std::max<double>(tm[1], r.ms_k0);
+    tm[2] = std::max<double>(tm[2], r.ms_k1);
+    tm[3] = std::max<double>(tm[3], r.ms_d2h);
+    tm[5] = std::max<double>(tm[5], r.ms_gather);
+    tm[6] += r.launches;
+    tm[7] += r.d2h_bytes;
+    h2d_total += r.h2d_bytes;
+  }
+  tm[4] = std::chrono::duration<double, std::milli>(t1 - t0).count();
+  memcpy(tl_timings, tm, sizeof tm);
+  tl_output = {res[0].out_mode, res[0].host_items, h2d_total};
+  if (flags & kFlagBadId)
+    throw Err{GFICF_E_RANGE,
+              "neighbour ids must be integers in [1, nrow] (NaN, fractional or out-of-range id found)"};
+  return res[0].n_written;
+}
+
+int jaccard_host_call(const void* idx, int elem, int64_t n, int32_t k, double* out, int32_t n_devices,
+                      int32_t mode, int64_t* n_written, char* err, size_t errlen) {
+  API_BEGIN
+  if (err && errlen) err[0] = 0;
+  if (!jaccard_check_args(idx, out, n, k, mode, n_written)) return GFICF_OK;
   int ndev = n_devices > 0 ? n_devices : default_devices();
   const int vis = visible_devices();
   if (vis < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
@@ -1101,80 +1175,13 @@ int jaccard_host_call(const void* idx, int elem, int64_t n, int32_t k, double* o
   if (ndev > kMaxDevices) throw Err{GFICF_E_ARG, "too many devices"};
   if (mode == GFICF_MODE_SERIAL) ndev = 1;  // global row compaction: one device
   if ((long long)ndev > n) ndev = 1;
-
-  std::lock_guard<std::mutex> lk(g_call_mu);
-  DeviceRestore restore;
-  const auto t0 = std::chrono::steady_clock::now();
   const long long rows_per = (n + ndev - 1) / ndev;
-  g_active_devices.store(ndev);
-  std::vector<SlabResult> res(ndev);
-  std::vector<Slab> slabs;
   const int out_mode = resolve_out_mode(out, (int)k, (int)mode);
-  for (int r = 0; r < ndev; ++r) {
-    slabs.emplace_back(r, ndev, idx, (long long)n, (int)k, rows_per, out, (int)mode);
-    slabs.back().elem = elem;
-    slabs.back().out_mode = out_mode;
-  }
-  auto first_error = [&]() {
-    for (auto& r : res)
-      if (r.err.code != GFICF_OK) throw r.err;
-  };
-  if (ndev == 1) {
-    device_phase0(slabs[0], &res[0]);
-    first_error();
-    device_phase1(slabs[0], &res[0]);
-  } else {
-    nccl_ensure(ndev);
-    for (int r = 0; r < ndev; ++r) slabs[r].comm = g_nccl.comms[r];
-    {
-      std::vector<std::thread> th;
-      for (int r = 0; r < ndev; ++r) th.emplace_back(device_phase0, slabs[r], &res[r]);
-      for (auto& t : th) t.join();
-    }
-    first_error();  // nobody has entered a collective yet
-    std::vector<std::thread> th;
-    for (int r = 0; r < ndev; ++r) th.emplace_back(device_phase1, slabs[r], &res[r]);
-    for (auto& t : th) t.join();
-  }
-  unsigned all_flags = 0;
-  for (auto& r : res) all_flags |= r.flags;
-  bool bad_id = (all_flags & kFlagBadId) != 0;
-  if (!bad_id) {
-    first_error();
-    const bool exact = k > kLargeMaxK || (all_flags & (kFlagDupId | kFlagHashFail));
-    if (exact || mode == GFICF_MODE_SERIAL) {
-      if (ndev == 1) {
-        device_phase2(slabs[0], exact, &res[0]);
-      } else {
-        std::vector<std::thread> th;
-        for (int r = 0; r < ndev; ++r) th.emplace_back(device_phase2, slabs[r], exact, &res[r]);
-        for (auto& t : th) t.join();
-      }
-    }
-  }
-  const auto t1 = std::chrono::steady_clock::now();
-  unsigned flags = 0;
-  double tm[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-  for (auto& r : res) {
-    if (!bad_id && r.err.code != GFICF_OK) throw r.err;
-    flags |= r.flags;
-    tm[0] = std::max<double>(tm[0], r.ms_h2d);
-    tm[1] = std::max<double>(tm[1], r.ms_k0);
-    tm[2] = std::max<double>(tm[2], r.ms_k1);
-    tm[3] = std::max<double>(tm[3], r.ms_d2h);
-    tm[5] = std::max<double>(tm[5], r.ms_gather);
-    tm[6] += r.launches;
-    tm[7] += r.d2h_bytes;
-  }
-  double h2d_total = 0;
-  for (auto& r : res) h2d_total += r.h2d_bytes;
-  tl_output = {res[0].out_mode, res[0].host_items, h2d_total};
-  tm[4] = std::chrono::duration<double, std::milli>(t1 - t0).count();
-  memcpy(tl_timings, tm, sizeof tm);
-  if (flags & kFlagBadId)
-    throw Err{GFICF_E_RANGE,
-              "neighbour ids must be integers in [1, nrow] (NaN, fractional or out-of-range id found)"};
-  if (n_written) *n_written = res[0].n_written;
+  std::vector<Slab> slabs;
+  for (int r = 0; r < ndev; ++r)
+    slabs.emplace_back(r, ndev, idx, elem, (long long)n, (int)k, rows_per, out, (int)mode, out_mode);
+  const long long nw = run_slabs(slabs, nullptr);
+  if (n_written) *n_written = nw;
   return GFICF_OK;
   API_END
 }
@@ -1238,67 +1245,14 @@ int gficf_cuda_jaccard_rank(const double* idx, int64_t n, int32_t k, double* out
   API_BEGIN
   if (err && errlen) err[0] = 0;
   if (!g_mp.comm) throw Err{GFICF_E_ARG, "gficf_cuda_comm_init_rank has not been called"};
-  if (n < 0 || k < 0) throw Err{GFICF_E_ARG, "negative matrix dimension"};
-  if (n == 0 || k == 0) return GFICF_OK;
-  if (!idx || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
-  if (n >= 0x7fffffffLL - 2 || (long double)n * k >= 2147483647.0L)
-    throw Err{GFICF_E_LIMIT, "n*k must stay below 2^31 (the reference's int row index)"};
-  if (k > 65535) throw Err{GFICF_E_LIMIT, "k above 65535 is not supported"};
-  std::lock_guard<std::mutex> lk(g_call_mu);
-  DeviceRestore restore;
-  const auto t0 = std::chrono::steady_clock::now();
+  if (!jaccard_check_args(idx, out, n, k, GFICF_MODE_PARALLEL, nullptr)) return GFICF_OK;
   const int nr = g_mp.nranks;
-  const long long rows_per = (n + nr - 1) / nr;
-  Slab s(g_mp.rank, nr, idx, (long long)n, (int)k, rows_per, out, GFICF_MODE_PARALLEL);
-  s.dev = g_mp.dev;
-  s.comm = g_mp.comm;
-  s.out_mode = resolve_out_mode(out, (int)k, GFICF_MODE_PARALLEL);
-  SlabResult res;
-  device_phase0(s, &res);
-  DeviceWs& ws = g_ws[s.dev];
-  {
-    // agree that every rank got through its local phase BEFORE the index all-gather: a rank that
-    // failed (out of memory ...) still takes part in this tiny all-reduce, then everybody leaves
-    CU_TRY(cudaSetDevice(s.dev));
-    ws.ensure(s.dev);
-    int* okbit = (int*)((char*)ws.small.p + 48);
-    int h = res.err.code != GFICF_OK;
-    CU_TRY(cudaMemcpyAsync(okbit, &h, sizeof h, cudaMemcpyHostToDevice, ws.s_comp));
-    NCCL_TRY(nccl_dyn::get().AllReduce(okbit, okbit, 1, ncclInt32, ncclMax, s.comm, ws.s_comp));
-    CU_TRY(cudaMemcpyAsync(&h, okbit, sizeof h, cudaMemcpyDeviceToHost, ws.s_comp));
-    CU_TRY(cudaStreamSynchronize(ws.s_comp));
-    if (res.err.code != GFICF_OK) throw res.err;
-    if (h) throw Err{GFICF_E_CUDA, "another rank failed before the index exchange"};
-  }
-  device_phase1(s, &res);
-  // flags of all ranks (every rank must reach this collective, error or not)
-  unsigned all_flags = res.flags;
-  {
-    CU_TRY(cudaSetDevice(s.dev));
-    int* bits = (int*)((char*)ws.small.p + 32);
-    int h[4] = {(int)(res.flags & 1u), (int)((res.flags >> 1) & 1u), (int)((res.flags >> 2) & 1u),
-                res.err.code != GFICF_OK};
-    CU_TRY(cudaMemcpyAsync(bits, h, sizeof h, cudaMemcpyHostToDevice, ws.s_comp));
-    NCCL_TRY(nccl_dyn::get().AllReduce(bits, bits, 4, ncclInt32, ncclMax, s.comm, ws.s_comp));
-    CU_TRY(cudaMemcpyAsync(h, bits, sizeof h, cudaMemcpyDeviceToHost, ws.s_comp));
-    CU_TRY(cudaStreamSynchronize(ws.s_comp));
-    all_flags = (unsigned)h[0] | ((unsigned)h[1] << 1) | ((unsigned)h[2] << 2);
-    if (res.err.code != GFICF_OK) throw res.err;
-    if (h[3]) throw Err{GFICF_E_CUDA, "another rank failed"};
-  }
-  if (all_flags & kFlagBadId)
-    throw Err{GFICF_E_RANGE,
-              "neighbour ids must be integers in [1, nrow] (NaN, fractional or out-of-range id found)"};
-  if (k > kLargeMaxK || (all_flags & (kFlagDupId | kFlagHashFail))) {
-    device_phase2(s, true, &res);
-    if (res.err.code != GFICF_OK) throw res.err;
-  }
-  const auto t1 = std::chrono::steady_clock::now();
-  double tm[8] = {res.ms_h2d, res.ms_k0, res.ms_k1, res.ms_d2h,
-                  std::chrono::duration<double, std::milli>(t1 - t0).count(), res.ms_gather,
-                  (double)res.launches, res.d2h_bytes};
-  memcpy(tl_timings, tm, sizeof tm);
-  tl_output = {res.out_mode, res.host_items, res.h2d_bytes};
+  std::vector<Slab> slabs;
+  slabs.emplace_back(g_mp.rank, nr, idx, 8, (long long)n, (int)k, (n + nr - 1) / nr, out, GFICF_MODE_PARALLEL,
+                     resolve_out_mode(out, (int)k, GFICF_MODE_PARALLEL));
+  slabs[0].dev = g_mp.dev;
+  slabs[0].comm = g_mp.comm;
+  run_slabs(slabs, g_mp.comm);
   return GFICF_OK;
   API_END
 }
@@ -1532,8 +1486,7 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   if (n == 0 || k == 0) return GFICF_OK;
   if (!idx_colmajor || !colptr || !row || !w || cap < 0) throw Err{GFICF_E_ARG, "null output pointer"};
   if (k > 127) throw Err{GFICF_E_LIMIT, "the graph build carries the mutual flag in bit 7 of the count byte: k <= 127"};
-  if (n >= 0x7fffffffLL - 2 || (long double)n * k >= 2147483647.0L)
-    throw Err{GFICF_E_LIMIT, "n*k must stay below 2^31 (the reference's int row index)"};
+  check_nk_limit(n, k);
   SingleDeviceCall call;
   DeviceWs& ws = call.ws;
   const long long E = (long long)n * k;
@@ -1558,15 +1511,7 @@ int gficf_cuda_snn_lower(const void* idx_colmajor, int32_t elem_bytes, int64_t n
   results((char*)ws.out.p);
   unsigned* d_flags = (unsigned*)ws.small.p;
   int64_t* d_nv = (int64_t*)((char*)ws.small.p + 16);
-  CU_TRY(cudaMemsetAsync(ws.small.p, 0, 64, ws.s_comp));
-  CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
-  const size_t dev_elem = h2d_block(ws, idx_colmajor, n, ws.in_raw.p, n, k, (size_t)elem_bytes, ws.s_comp);
-  CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
-  if (dev_elem == 8)
-    launch_layout(jac_ctx(ws.s_comp), (const double*)ws.in_raw.p, n, 0, n, k, 0, n, (int*)ws.idx.p, d_flags);
-  else
-    launch_layout(jac_ctx(ws.s_comp), (const int*)ws.in_raw.p, n, 0, n, k, 0, n, (int*)ws.idx.p, d_flags);
-  CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
+  upload_rows(ws, idx_colmajor, elem_bytes, n, k, 0, n);
   if (!launch_fast<2>(jac_ctx(ws.s_comp), (const int*)ws.idx.p, k, 0, n, nullptr, nullptr, nullptr, ws.counts.p,
                       d_flags))
     throw Err{GFICF_E_LIMIT, "k outside the range of the mutual-bit count kernel"};
