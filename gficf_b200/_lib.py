@@ -79,6 +79,8 @@ PROTOTYPES = {
     "gficf_cuda_wmu_markers": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, C.c_int32, _vp, C.c_char_p, C.c_size_t]),
     "gficf_cuda_wmu_markers_csc": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int64, _vp, C.c_int32, _vp, C.c_char_p,
                                              C.c_size_t]),
+    "gficf_cuda_wmu_markers_csc_devices": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int64, _vp, C.c_int32, C.c_int32,
+                                                     _vp, C.c_char_p, C.c_size_t]),
     "gficf_cuda_set_launch_ctas_per_sm": (C.c_int, [C.c_int32]),
     "gficf_cuda_last_launch": (C.c_int, [C.POINTER(C.c_int32)] * 4),
     "gficf_cuda_version": (C.c_char_p, []),

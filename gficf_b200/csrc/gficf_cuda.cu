@@ -204,8 +204,9 @@ struct DeviceWs {
   cudaStream_t s_comp = nullptr, s_copy = nullptr;
   cudaEvent_t ev[8] = {};
   cudaEvent_t ev_k0[kMaxChunks] = {}, ev_k1[kMaxChunks] = {};
-  // in_raw: device copy of the caller's rows (f64 or int32, column-major); small: flags + n_written
-  Buf in_raw, idx, out, counts, scratch, small;
+  // in_raw: device copy of the caller's rows (f64 or int32, column-major); small: flags + n_written;
+  // exch: what the sparse markers call on several devices receives, regroups and indexes it with
+  Buf in_raw, idx, out, counts, scratch, small, exch;
   PinBuf ring, h_counts;  // h_counts: the slab's 1-byte counts on the host (counts-over-PCIe output mode)
   cudaEvent_t ev_cnt_done = nullptr, ev_exp = nullptr, ev_dma[4] = {}, ev_ring = nullptr;
   bool ring_used = false;  // ev_ring marks the end of the last staged copy through `ring`
@@ -235,7 +236,7 @@ struct DeviceWs {
     if (!init) return;
     cudaSetDevice(dev);
     cudaDeviceSynchronize();
-    in_raw.drop(); idx.drop(); out.drop(); counts.drop(); scratch.drop(); small.drop();
+    in_raw.drop(); idx.drop(); out.drop(); counts.drop(); scratch.drop(); small.drop(); exch.drop();
     ring.drop();
     h_counts.drop();
     cudaEventDestroy(ev_cnt_done);
@@ -1577,6 +1578,22 @@ std::vector<long long> markers_cluster_sizes(const int32_t* cluster, int64_t n_c
   return size;
 }
 
+// Host checks of the compressed-column markers entries, before any device is touched; false when there are no
+// genes (nothing to do).  The row ids are checked on the device, by the transpose that reads them.
+bool markers_csc_check(const int32_t* colptr, const int32_t* row, const double* x, int64_t n_genes, int64_t n_cells,
+                       const int32_t* cluster, int32_t n_clusters, const double* out) {
+  markers_check_sizes(n_genes, n_cells, n_clusters);
+  if (n_genes == 0) return false;
+  if (n_genes >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 genes (R's int row ids)"};
+  if (!colptr || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  if (colptr[0] != 0) throw Err{GFICF_E_ARG, fmt("colptr[0] is %d, not 0", colptr[0])};
+  for (int64_t j = 0; j < n_cells; ++j)
+    if (colptr[j + 1] < colptr[j])
+      throw Err{GFICF_E_ARG, fmt("colptr decreases at column %lld (%d after %d)", (long long)j, colptr[j + 1], colptr[j])};
+  if (colptr[n_cells] > 0 && (!row || !x)) throw Err{GFICF_E_ARG, "null matrix pointer"};
+  return true;
+}
+
 // The end shared by the Mann-Whitney entries: launches checked, ev[2] recorded, z | ratio (n_clusters blocks of
 // n_genes) and the per-gene single flags read back and finished into out (wmu_finish).
 void wmu_read_and_finish(DeviceWs& ws, const double* d_z, const int* d_single, int64_t n_genes, int32_t n_clusters,
@@ -1749,16 +1766,8 @@ int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const 
                                size_t errlen) {
   API_BEGIN
   if (err && errlen) err[0] = 0;
-  markers_check_sizes(n_genes, n_cells, n_clusters);
-  if (n_genes == 0) return GFICF_OK;
-  if (n_genes >= 0x7fffffffLL) throw Err{GFICF_E_LIMIT, "more than 2^31 genes (R's int row ids)"};
-  if (!colptr || !cluster || !out) throw Err{GFICF_E_ARG, "null matrix pointer"};
-  if (colptr[0] != 0) throw Err{GFICF_E_ARG, fmt("colptr[0] is %d, not 0", colptr[0])};
-  for (int64_t j = 0; j < n_cells; ++j)
-    if (colptr[j + 1] < colptr[j])
-      throw Err{GFICF_E_ARG, fmt("colptr decreases at column %lld (%d after %d)", (long long)j, colptr[j + 1], colptr[j])};
+  if (!markers_csc_check(colptr, row, x, n_genes, n_cells, cluster, n_clusters, out)) return GFICF_OK;
   const long long nnz = colptr[n_cells];
-  if (nnz > 0 && (!row || !x)) throw Err{GFICF_E_ARG, "null matrix pointer"};
   const std::vector<long long> size = markers_cluster_sizes(cluster, n_cells, n_clusters);
   SingleDeviceCall call;
   DeviceWs& ws = call.ws;
@@ -1833,6 +1842,257 @@ int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const 
   call.timings(event_ms(ws.ev[0], ws.ev[1]), 0, event_ms(ws.ev[1], ws.ev[2]), 0,
                (double)(7 + 5 * ((bits_for(n_genes - 1) + 7) / 8)),
                (double)zc * 16 + (double)n_genes * 4 + 4 + (double)gptr.size() * 8);
+  return GFICF_OK;
+  API_END
+}
+
+}  // extern "C"
+
+// ---------------------------------------------------------------- the same on several devices
+namespace {
+// One device of gficf_cuda_wmu_markers_csc_devices: column slab r = [c0, c1) (stored values [v0, v0 + nnz)) on
+// device r, and after the exchange the genes [g0, g0 + ng).
+struct WmuDevice {
+  int dev;
+  long long c0, c1, v0, nnz;
+  std::vector<int> colptr;     // the slab's column pointers, rebased to 0
+  std::vector<long long> gptr;  // the slab's gene pointers (n_genes + 1)
+  unsigned flags = 0;
+  WmuCscScratch sc;
+  WmuGeneMajor slab;  // the slab's values gene-major, cells local to the slab
+  int *d_cl, *d_crank, *d_members;
+  long long *d_size, *d_cptr;
+  // after the gene ranges are known
+  long long g0 = 0, ng = 0, cap = 1;
+  int grid = 1;
+  std::vector<long long> src, dst, cell0;  // regroup tables (wmu_regroup_tables) and the slabs' first columns
+  unsigned *d_rcell, *d_ecell;
+  double *d_rx, *d_ex;
+  long long *d_src, *d_dst, *d_cell0;
+  float ms_h2d = 0, ms_transpose = 0, ms_exchange = 0, ms_rank = 0;
+  Err err;
+};
+
+// fn(device) on one host thread per device; every thread has joined before the first failure is raised
+template <class F>
+void on_devices(std::vector<WmuDevice>& devs, F fn) {
+  std::vector<std::thread> th;
+  for (auto& w : devs)
+    th.emplace_back([&fn, &w] {
+      try {
+        CU_TRY(cudaSetDevice(w.dev));
+        fn(w);
+      } catch (const Err& e) {
+        w.err = e;
+      } catch (const std::exception& e) {
+        w.err = Err{GFICF_E_CUDA, e.what()};
+      }
+    });
+  for (auto& t : th) t.join();
+  for (auto& w : devs)
+    if (w.err.code != GFICF_OK) throw w.err;
+}
+
+void wmu_csc_devices(const int32_t* colptr, const int32_t* row, const double* x, long long n_genes, long long N,
+                     const int32_t* cluster, int n_clusters, const std::vector<long long>& size, int D, double* out) {
+  std::lock_guard<std::mutex> lk(g_call_mu);
+  DeviceRestore restore;
+  const auto t0 = std::chrono::steady_clock::now();
+  const long long C = n_clusters;
+  g_active_devices.store(D);
+  nccl_ensure(D);
+  const WmuClusterLists cl = wmu_cluster_lists(cluster, N, n_clusters);
+  const std::vector<long long> c = wmu_cell_slabs(colptr, N, D);
+  std::vector<WmuDevice> devs((size_t)D);
+  for (int r = 0; r < D; ++r) {
+    WmuDevice& w = devs[(size_t)r];
+    w.dev = r;
+    w.c0 = c[(size_t)r];
+    w.c1 = c[(size_t)r + 1];
+    w.v0 = colptr[w.c0];
+    w.nnz = colptr[w.c1] - w.v0;
+  }
+
+  // upload of each slab and of the cluster lists, transpose; the flags and gene pointers come back to the host
+  on_devices(devs, [&](WmuDevice& w) {
+    DeviceWs& ws = g_ws[w.dev];
+    ws.ensure(w.dev);
+    const long long n = w.c1 - w.c0;
+    w.colptr.resize((size_t)n + 1);
+    for (long long j = 0; j <= n; ++j) w.colptr[(size_t)j] = colptr[w.c0 + j] - (int)w.v0;
+    int* d_colptr;
+    int* d_row;
+    double* d_x;
+    auto matrix = [&](char* base) {
+      ScratchCarver cv{base};
+      d_colptr = cv.take<int>(n + 1);
+      d_row = cv.take<int>(w.nnz);
+      d_x = cv.take<double>(w.nnz + 1);
+      return cv.bytes;
+    };
+    auto lists = [&](char* base) {
+      ScratchCarver cv{base};
+      w.d_cl = cv.take<int>(N);
+      w.d_crank = cv.take<int>(N);
+      w.d_members = cv.take<int>(N);
+      w.d_size = cv.take<long long>(C);
+      w.d_cptr = cv.take<long long>(C + 1);
+      return cv.bytes;
+    };
+    ws.in_raw.need(matrix(nullptr));
+    matrix((char*)ws.in_raw.p);
+    ws.idx.need(lists(nullptr));
+    lists((char*)ws.idx.p);
+    ws.scratch.need(wmu_csc_layout(nullptr, n_genes, w.nnz).bytes);
+    w.sc = wmu_csc_layout((char*)ws.scratch.p, n_genes, w.nnz);
+    CU_TRY(cudaEventRecord(ws.ev[0], ws.s_comp));
+    h2d_block(ws, w.colptr.data(), n + 1, d_colptr, n + 1, 1, 4, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, row + w.v0, w.nnz, d_row, w.nnz, 1, 4, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, x + w.v0, w.nnz, d_x, w.nnz, 1, 8, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, cluster, N, w.d_cl, N, 1, 4, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, cl.crank.data(), N, w.d_crank, N, 1, 4, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, cl.members.data(), N, w.d_members, N, 1, 4, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, size.data(), C, w.d_size, C, 1, 8, ws.s_comp, /*ids=*/false);
+    h2d_block(ws, cl.cptr.data(), C + 1, w.d_cptr, C + 1, 1, 8, ws.s_comp, /*ids=*/false);
+    CU_TRY(cudaEventRecord(ws.ev[1], ws.s_comp));
+    w.slab = wmu_csc_to_genes(ws.s_comp, w.sc, sm_count() * 8, d_colptr, d_row, d_x, n_genes, n, w.nnz);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaEventRecord(ws.ev[2], ws.s_comp));
+    w.gptr.resize((size_t)n_genes + 1);
+    CU_TRY(cudaMemcpyAsync(&w.flags, w.sc.flags, 4, cudaMemcpyDeviceToHost, ws.s_comp));
+    CU_TRY(cudaMemcpyAsync(w.gptr.data(), w.sc.gene_ptr, w.gptr.size() * 8, cudaMemcpyDeviceToHost, ws.s_comp));
+    CU_TRY(cudaStreamSynchronize(ws.s_comp));
+    w.ms_h2d = event_ms(ws.ev[0], ws.ev[1]);
+    w.ms_transpose = event_ms(ws.ev[1], ws.ev[2]);
+  });
+  for (auto& w : devs)
+    if (w.flags & kFlagCscRow)
+      throw Err{GFICF_E_ARG, "a row id is outside [0, n_genes) or row ids are not strictly increasing in a column"};
+
+  // gene ranges and exchange table; every buffer of the exchange and of the kernels is allocated before any
+  // device enters the exchange (a device that failed later would leave its peers waiting in it)
+  std::vector<const long long*> gptr;
+  for (auto& w : devs) gptr.push_back(w.gptr.data());
+  const WmuExchange xp = wmu_exchange_plan(gptr, n_genes);
+  on_devices(devs, [&](WmuDevice& w) {
+    DeviceWs& ws = g_ws[w.dev];
+    const int d = w.dev;
+    w.g0 = xp.g[(size_t)d];
+    w.ng = xp.g[(size_t)d + 1] - w.g0;
+    wmu_regroup_tables(xp, gptr, d, &w.src, &w.dst);
+    w.cell0.assign(c.begin(), c.end() - 1);
+    const long long nr = xp.nrecv[(size_t)d];
+    auto exch = [&](char* base) {
+      ScratchCarver cv{base};
+      w.d_rcell = cv.take<unsigned>(nr);
+      w.d_rx = cv.take<double>(nr);
+      w.d_ecell = cv.take<unsigned>(nr);
+      w.d_ex = cv.take<double>(nr);
+      w.d_src = cv.take<long long>(w.src.size());
+      w.d_dst = cv.take<long long>(w.dst.size());
+      w.d_cell0 = cv.take<long long>(D);
+      return cv.bytes;
+    };
+    ws.exch.need(exch(nullptr));
+    exch((char*)ws.exch.p);
+    CU_TRY(cudaMemcpyAsync(w.d_src, w.src.data(), w.src.size() * 8, cudaMemcpyHostToDevice, ws.s_comp));
+    CU_TRY(cudaMemcpyAsync(w.d_dst, w.dst.data(), w.dst.size() * 8, cudaMemcpyHostToDevice, ws.s_comp));
+    CU_TRY(cudaMemcpyAsync(w.d_cell0, w.cell0.data(), (size_t)D * 8, cudaMemcpyHostToDevice, ws.s_comp));
+    w.cap = wmu_gene_cap(w.dst.data(), w.ng);
+    CU_TRY(cudaFuncSetAttribute(wmu_markers_csr_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                kWmuMaxClusters * kWmuClusterSmemBytes));
+    int per_sm = 0;
+    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wmu_markers_csr_rank_kernel, kWmuThreads,
+                                                         (size_t)C * kWmuClusterSmemBytes));
+    w.grid = (int)std::min<long long>(w.ng, (long long)std::max(1, per_sm) * sm_count());
+    ws.counts.need((size_t)w.grid * 2 * w.cap * (sizeof(unsigned long long) + sizeof(unsigned)));
+    ws.out.need((size_t)w.ng * C * 16 + (size_t)w.ng * 4 + 64);
+    CU_TRY(cudaStreamSynchronize(ws.s_comp));
+  });
+
+  // exchange (NCCL point to point; a device's own block is a device-to-device copy), regroup, rank + means,
+  // and the finish of the device's rows of out
+  on_devices(devs, [&](WmuDevice& w) {
+    DeviceWs& ws = g_ws[w.dev];
+    const int d = w.dev;
+    const nccl_dyn::Api& nc = nccl_dyn::get();
+    ncclComm_t comm = g_nccl.comms[d];
+    CU_TRY(cudaEventRecord(ws.ev[3], ws.s_comp));
+    NCCL_TRY(nc.GroupStart());
+    for (int r = 0; r < D; ++r) {
+      if (r == d) continue;
+      const size_t out_i = (size_t)d * D + r, in_i = (size_t)r * D + d;
+      if (xp.cnt[out_i] > 0) {
+        NCCL_TRY(nc.Send(w.slab.ent_cell + xp.send[out_i], (size_t)xp.cnt[out_i], ncclUint32, r, comm, ws.s_comp));
+        NCCL_TRY(nc.Send(w.slab.ent_x + xp.send[out_i], (size_t)xp.cnt[out_i], ncclFloat64, r, comm, ws.s_comp));
+      }
+      if (xp.cnt[in_i] > 0) {
+        NCCL_TRY(nc.Recv(w.d_rcell + xp.recv[in_i], (size_t)xp.cnt[in_i], ncclUint32, r, comm, ws.s_comp));
+        NCCL_TRY(nc.Recv(w.d_rx + xp.recv[in_i], (size_t)xp.cnt[in_i], ncclFloat64, r, comm, ws.s_comp));
+      }
+    }
+    NCCL_TRY(nc.GroupEnd());
+    const size_t self = (size_t)d * D + d;
+    if (xp.cnt[self] > 0) {
+      CU_TRY(cudaMemcpyAsync(w.d_rcell + xp.recv[self], w.slab.ent_cell + xp.send[self], (size_t)xp.cnt[self] * 4,
+                             cudaMemcpyDeviceToDevice, ws.s_comp));
+      CU_TRY(cudaMemcpyAsync(w.d_rx + xp.recv[self], w.slab.ent_x + xp.send[self], (size_t)xp.cnt[self] * 8,
+                             cudaMemcpyDeviceToDevice, ws.s_comp));
+    }
+    CU_TRY(cudaEventRecord(ws.ev[4], ws.s_comp));
+    const WmuGeneMajor gm = wmu_regroup(ws.s_comp, sm_count() * 8, w.d_rcell, w.d_rx, w.d_src, w.d_dst, w.d_cell0, D,
+                                        w.ng, w.d_ecell, w.d_ex);
+    const size_t zc = (size_t)w.ng * C;
+    double* d_z = (double*)ws.out.p;
+    double* d_ratio = d_z + zc;
+    int* d_single = (int*)(d_ratio + zc);
+    unsigned long long* d_keys = (unsigned long long*)ws.counts.p;
+    unsigned* d_pay = (unsigned*)(d_keys + (size_t)w.grid * 2 * w.cap);
+    wmu_markers_csc_launch(ws.s_comp, w.grid, gm, w.d_dst, w.ng, N, w.d_cl, w.d_crank, w.d_members, w.d_size,
+                           w.d_cptr, n_clusters, w.cap, d_keys, d_pay, d_z, d_ratio, d_single);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaEventRecord(ws.ev[5], ws.s_comp));
+    std::vector<double> h(zc * 2);
+    std::vector<int> hs((size_t)w.ng);
+    CU_TRY(cudaMemcpyAsync(h.data(), d_z, zc * 16, cudaMemcpyDeviceToHost, ws.s_comp));
+    CU_TRY(cudaMemcpyAsync(hs.data(), d_single, (size_t)w.ng * 4, cudaMemcpyDeviceToHost, ws.s_comp));
+    CU_TRY(cudaStreamSynchronize(ws.s_comp));
+    wmu_finish(h.data(), hs.data(), w.ng, n_clusters, out, w.g0, n_genes);
+    w.ms_exchange = event_ms(ws.ev[3], ws.ev[4]);
+    w.ms_rank = event_ms(ws.ev[4], ws.ev[5]);
+  });
+  double tm[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  for (auto& w : devs) {
+    tm[0] = std::max<double>(tm[0], w.ms_h2d);
+    tm[1] = std::max<double>(tm[1], w.ms_transpose);
+    tm[2] = std::max<double>(tm[2], w.ms_rank);
+    tm[5] = std::max<double>(tm[5], w.ms_exchange);
+  }
+  tm[4] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  memcpy(tl_timings, tm, sizeof tm);
+}
+}  // namespace
+
+extern "C" {
+
+// gficf_cuda_wmu_markers_csc with the genes split over n_devices devices (0: gficf_cuda_set_devices' count)
+int gficf_cuda_wmu_markers_csc_devices(const int32_t* colptr, const int32_t* row, const double* x, int64_t n_genes,
+                                       int64_t n_cells, const int32_t* cluster, int32_t n_clusters,
+                                       int32_t n_devices, double* out, char* err, size_t errlen) {
+  API_BEGIN
+  if (err && errlen) err[0] = 0;
+  if (n_devices < 0) throw Err{GFICF_E_ARG, "n_devices must be 0 (the default count) or positive"};
+  if (!markers_csc_check(colptr, row, x, n_genes, n_cells, cluster, n_clusters, out)) return GFICF_OK;
+  const std::vector<long long> size = markers_cluster_sizes(cluster, n_cells, n_clusters);
+  const int ndev = n_devices > 0 ? n_devices : default_devices();
+  const int vis = visible_devices();
+  if (vis < 1) throw Err{GFICF_E_CUDA, "no CUDA device is visible (this path has no CPU fallback)"};
+  if (ndev > vis) throw Err{GFICF_E_ARG, fmt("%d devices requested but only %d visible", ndev, vis)};
+  if (ndev > kMaxDevices) throw Err{GFICF_E_ARG, "too many devices"};
+  const int D = (int)std::min<long long>(ndev, n_genes);
+  if (D == 1)
+    return gficf_cuda_wmu_markers_csc(colptr, row, x, n_genes, n_cells, cluster, n_clusters, out, err, errlen);
+  wmu_csc_devices(colptr, row, x, n_genes, n_cells, cluster, n_clusters, size, D, out);
   return GFICF_OK;
   API_END
 }

@@ -1,8 +1,9 @@
 // nccl_dyn.h -- NCCL bound at run time (dlopen), so the library loads on a
 // single-GPU host without libnccl and never conflicts with the NCCL a host
-// process (e.g. PyTorch) already carries.  Only the entry points the row-sharded
-// path needs: communicator setup for the GPUs of one process, all-gather of the
-// int32 index slabs, broadcast.
+// process (e.g. PyTorch) already carries.  Only the entry points the multi-GPU
+// paths need: communicator setup for the GPUs of one process, all-gather of the
+// int32 index slabs, broadcast, and the point-to-point exchange of the sparse
+// markers call's gene blocks.
 #pragma once
 #include <cuda_runtime.h>
 #include <dlfcn.h>
@@ -39,6 +40,8 @@ struct Api {
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*Broadcast)(const void*, void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
+  ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
   ncclResult_t (*GroupStart)() = nullptr;
   ncclResult_t (*GroupEnd)() = nullptr;
   const char* (*GetErrorString)(ncclResult_t) = nullptr;
@@ -68,6 +71,8 @@ struct Api {
     GFICF_NCCL_SYM(CommDestroy, "ncclCommDestroy")
     GFICF_NCCL_SYM(AllGather, "ncclAllGather")
     GFICF_NCCL_SYM(Broadcast, "ncclBroadcast")
+    GFICF_NCCL_SYM(Send, "ncclSend")
+    GFICF_NCCL_SYM(Recv, "ncclRecv")
     GFICF_NCCL_SYM(GroupStart, "ncclGroupStart")
     GFICF_NCCL_SYM(GroupEnd, "ncclGroupEnd")
     GFICF_NCCL_SYM(GetErrorString, "ncclGetErrorString")

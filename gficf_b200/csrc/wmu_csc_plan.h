@@ -1,7 +1,7 @@
 // wmu_csc_plan.h -- the Mann-Whitney calls' launch sequences (wmu_kernels.cuh) and host finish, shared by the product
 // and the CPU test suite: the rank + means launches of gficf_cuda_wmu_test, gficf_cuda_wmu_markers and
-// gficf_cuda_wmu_markers_csc, the cluster lists and device transpose of the compressed-column call, and the
-// p-value / log2 finish of all three.  Included by gficf_cuda.cu (after its error helpers) and by the
+// gficf_cuda_wmu_markers_csc, the cluster lists and device transpose of the compressed-column call, the slabs,
+// gene ranges, exchange table and regroup of its multi-device form, and the p-value / log2 finish of all of them.  Included by gficf_cuda.cu (after its error helpers) and by the
 // tests/cuda_emu/wmu*_emu.cpp harnesses with GFICF_CUDA_EMU defined.  Grids come from the caller (the product
 // sizes them from the occupancy of the rank kernels).
 //
@@ -159,21 +159,114 @@ inline void wmu_markers_csc_launch(net_stream_t st, int grid, const WmuGeneMajor
                   ratio);
 }
 
+// ---- several devices (gficf_cuda_wmu_markers_csc_devices).  A gene's result depends only on its own stored
+// values in cell order, so the genes are split over the devices.  The upload is split by cells instead: device
+// r receives the columns [c[r], c[r + 1]) and makes them gene-major (wmu_csc_to_genes).  Each device then owns
+// the genes [g[d], g[d + 1]) and receives from every slab r the block [gptr_r[g[d]], gptr_r[g[d + 1]]) of r's
+// gene-major values; wmu_regroup puts the blocks of a gene one after the other in slab order, which is cell
+// order, so the result is the single-device gene-major array restricted to the device's genes.
+
+// Column slabs: c[0 .. D], c[0] = 0, c[D] = n_cells; slab r holds about r's share of the nnz stored values
+// (c[r] = the first column that starts at or after r nnz / D).  A slab may hold no column or no stored value.
+inline std::vector<long long> wmu_cell_slabs(const int* colptr, long long n_cells, int D) {
+  std::vector<long long> c((size_t)D + 1, 0);
+  const long long nnz = colptr[n_cells];
+  for (int r = 1; r < D; ++r)
+    c[(size_t)r] = std::lower_bound(colptr, colptr + n_cells + 1, nnz * r / D,
+                                    [](int a, long long t) { return (long long)a < t; }) - colptr;
+  c[(size_t)D] = n_cells;
+  return c;
+}
+
+// Gene ranges: g[0 .. D], g[0] = 0, g[D] = n_genes (D <= n_genes), every range non-empty; range d is cut at
+// the first gene whose summed pointer G reaches d nnz / D, so it holds its share of the stored values to
+// within one gene's count, unless keeping every range non-empty moves the cut.
+inline std::vector<long long> wmu_gene_ranges(const long long* G, long long n_genes, int D) {
+  std::vector<long long> g((size_t)D + 1, 0);
+  const long long nnz = G[n_genes];
+  for (int d = 1; d < D; ++d) {
+    long long cut = std::lower_bound(G, G + n_genes + 1, nnz * d / D) - G;
+    cut = std::max(cut, g[(size_t)d - 1] + 1);
+    g[(size_t)d] = std::min(cut, n_genes - (D - d));
+  }
+  g[(size_t)D] = n_genes;
+  return g;
+}
+
+// The exchange of D devices, from the gene pointers of every slab (gptr[r]: n_genes + 1 entries each).
+// Block (r -> d): cnt[r D + d] values from offset send[r D + d] of r's gene-major arrays, received at offset
+// recv[r D + d] of d's receive buffer (the blocks of the sources before r come first); nrecv[d] in all.
+struct WmuExchange {
+  int D;
+  std::vector<long long> g, G;  // gene ranges; summed gene pointer (the single-device gene_ptr)
+  std::vector<long long> send, cnt, recv, nrecv;
+};
+
+inline WmuExchange wmu_exchange_plan(const std::vector<const long long*>& gptr, long long n_genes) {
+  WmuExchange x;
+  const int D = (int)gptr.size();
+  x.D = D;
+  x.G.assign((size_t)n_genes + 1, 0);
+  for (const long long* p : gptr)
+    for (long long j = 0; j <= n_genes; ++j) x.G[(size_t)j] += p[j];
+  x.g = wmu_gene_ranges(x.G.data(), n_genes, D);
+  x.send.resize((size_t)D * D);
+  x.cnt.resize((size_t)D * D);
+  x.recv.resize((size_t)D * D);
+  x.nrecv.assign((size_t)D, 0);
+  for (int d = 0; d < D; ++d)
+    for (int r = 0; r < D; ++r) {
+      const size_t i = (size_t)r * D + d;
+      x.send[i] = gptr[(size_t)r][x.g[(size_t)d]];
+      x.cnt[i] = gptr[(size_t)r][x.g[(size_t)d + 1]] - x.send[i];
+      x.recv[i] = x.nrecv[(size_t)d];
+      x.nrecv[(size_t)d] += x.cnt[i];
+    }
+  return x;
+}
+
+// Destination d's regroup tables, ng = g[d + 1] - g[d] genes: src[r (ng + 1) + j] = where local gene j's values
+// from slab r start in d's receive buffer (j = ng: where that block ends); dst[j] = where gene j starts in
+// d's gene-major array (the local gene pointer of the rank and means kernels); cell0[r] = c[r].
+inline void wmu_regroup_tables(const WmuExchange& x, const std::vector<const long long*>& gptr, int d,
+                               std::vector<long long>* src, std::vector<long long>* dst) {
+  const long long g0 = x.g[(size_t)d], ng = x.g[(size_t)d + 1] - g0;
+  src->resize((size_t)x.D * (ng + 1));
+  dst->resize((size_t)ng + 1);
+  for (int r = 0; r < x.D; ++r)
+    for (long long j = 0; j <= ng; ++j)
+      (*src)[(size_t)r * (ng + 1) + j] = x.recv[(size_t)r * x.D + d] + gptr[(size_t)r][g0 + j] - gptr[(size_t)r][g0];
+  for (long long j = 0; j <= ng; ++j) (*dst)[(size_t)j] = x.G[(size_t)(g0 + j)] - x.G[(size_t)g0];
+}
+
+// The received blocks (cells local to their slab, rcell / rx) into one gene-major array of ng genes (device
+// pointers to the tables of wmu_regroup_tables).
+inline WmuGeneMajor wmu_regroup(net_stream_t st, int max_ctas, const unsigned* rcell, const double* rx,
+                                const long long* src, const long long* dst, const long long* cell0, int D,
+                                long long ng, unsigned* ent_cell, double* ent_x) {
+  const long long warps = 256 / 32;
+  const long long grid = std::max(1LL, std::min<long long>((ng + warps - 1) / warps, max_ctas));
+  GFICF_LAUNCH(st, wmu_regroup_kernel, grid, 256, rcell, rx, src, dst, cell0, D, ng, ent_cell, ent_x);
+  return WmuGeneMajor{ent_cell, ent_x};
+}
+
 // Host finish of the three calls: the two transcendental steps per (gene, cluster), getPvalue
 // (mann_whitney.cpp:101-110) and log2 (:100).  z_ratio = z | ratio, each n_clusters blocks of n_genes;
-// block c of out is cluster c's n_genes x 2 result (one split: n_clusters = 1).  Clusters are spread over
-// host threads when there are many values.
-inline void wmu_finish(const double* z_ratio, const int* single, long long n_genes, int n_clusters, double* out) {
+// block c of out is cluster c's ld x 2 result (one split: n_clusters = 1), and the n_genes go to its rows
+// [row0, row0 + n_genes) (ld = 0: n_genes).  Clusters are spread over host threads when there are many values.
+inline void wmu_finish(const double* z_ratio, const int* single, long long n_genes, int n_clusters, double* out,
+                       long long row0 = 0, long long ld = 0) {
   const long long C = n_clusters;
   const size_t zc = (size_t)n_genes * C;
+  if (ld == 0) ld = n_genes;
   auto finish = [&](long long c_lo, long long c_hi) {
     for (long long c = c_lo; c < c_hi; ++c) {
       const double* z = z_ratio + (size_t)c * n_genes;
       const double* ratio = z_ratio + zc + (size_t)c * n_genes;
-      double* o = out + (size_t)c * 2 * n_genes;
+      double* o = out + (size_t)c * 2 * ld + row0;
       for (long long g = 0; g < n_genes; ++g) {
         o[g] = single[g] ? 1.0 : gficf_host::wmu_pvalue(z[g]);
-        o[n_genes + g] = log2(ratio[g]);
+        o[ld + g] = log2(ratio[g]);
       }
     }
   };

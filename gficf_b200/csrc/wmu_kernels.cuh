@@ -741,6 +741,31 @@ wmu_csc_gather_kernel(const unsigned* __restrict__ vals, const unsigned* __restr
   }
 }
 
+// Several devices (wmu_csc_plan.h): the blocks one device received from every column slab, slab-major, into
+// one gene-major array.  Warp per local gene j: its values from slab r are rcell / rx[src[r (ng + 1) + j] ..
+// src[r (ng + 1) + j + 1]) with cells local to the slab; they go, slab after slab, to ent_cell / ent_x from
+// dst[j] on, each cell id plus the slab's first column cell0[r].  Slabs are in cell order and a slab's cells
+// ascend inside a gene, so the gene's cells ascend.
+__global__ void __launch_bounds__(256)
+wmu_regroup_kernel(const unsigned* __restrict__ rcell, const double* __restrict__ rx, const long long* __restrict__ src,
+                   const long long* __restrict__ dst, const long long* __restrict__ cell0, int D, long long ng,
+                   unsigned* __restrict__ ent_cell, double* __restrict__ ent_x) {
+  const int lane = threadIdx.x & 31;
+  const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
+  for (long long j = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); j < ng; j += nwarps) {
+    long long o = dst[j];
+    for (int r = 0; r < D; ++r) {
+      const long long s = src[(size_t)r * (ng + 1) + j], n = src[(size_t)r * (ng + 1) + j + 1] - s;
+      const unsigned base = (unsigned)cell0[r];
+      for (long long i = lane; i < n; i += 32) {
+        ent_cell[o + i] = rcell[s + i] + base;
+        ent_x[o + i] = rx[s + i];
+      }
+      o += n;
+    }
+  }
+}
+
 // s + 1.0 + 1.0 + ... (m additions, each rounded), replayed in O(binades) steps.  While ulp(s) <= 1, adding
 // an integer is exact as long as the result stays within s's binade or reaches its upper end 2^(e+1)
 // (s >= 0), or does not pass 0 (s < 0): those steps are taken in one addition.  The step that leaves that

@@ -86,12 +86,13 @@ def _int32_index(a, what):
     return np.ascontiguousarray(a, dtype=np.int32)
 
 
-def rcpp_parallel_WMU_markers_sparse(mat, cluster, printOutput: bool = False) -> np.ndarray:
+def rcpp_parallel_WMU_markers_sparse(mat, cluster, printOutput: bool = False, n_devices: int = 1) -> np.ndarray:
     """rcpp_parallel_WMU_markers for a scipy.sparse CSC matrix or array (genes x cells; R's dgCMatrix has
     the same slots).  Only the stored values are uploaded and read; the result equals, bit for bit,
     rcpp_parallel_WMU_markers(mat.toarray(), cluster).  Stored zeros are zeros.  Other sparse formats and
     dense arrays raise TypeError (convert with .tocsc() first); index arrays that do not fit in int32 raise
-    ValueError."""
+    ValueError.  n_devices > 1 splits the genes over that many GPUs (0: the count of set_devices); the
+    result is the same, bit for bit."""
     import scipy.sparse as sp
 
     if not sp.issparse(mat) or mat.format != "csc":
@@ -107,8 +108,13 @@ def rcpp_parallel_WMU_markers_sparse(mat, cluster, printOutput: bool = False) ->
         sys.stdout.write(_BANNER)
     out = np.empty((g, 2, k), dtype=np.float64, order="F")
     err = C.create_string_buffer(512)
-    rc = _lib.lib().gficf_cuda_wmu_markers_csc(colptr.ctypes.data, row.ctypes.data, x.ctypes.data, g, n,
-                                               ids.ctypes.data, k, out.ctypes.data, err, 512)
+    if n_devices == 1:
+        rc = _lib.lib().gficf_cuda_wmu_markers_csc(colptr.ctypes.data, row.ctypes.data, x.ctypes.data, g, n,
+                                                   ids.ctypes.data, k, out.ctypes.data, err, 512)
+    else:
+        rc = _lib.lib().gficf_cuda_wmu_markers_csc_devices(colptr.ctypes.data, row.ctypes.data, x.ctypes.data, g, n,
+                                                           ids.ctypes.data, k, int(n_devices), out.ctypes.data, err,
+                                                           512)
     _lib.check(rc, err)
     if printOutput:
         sys.stdout.write(_BANNER_DONE)

@@ -355,6 +355,26 @@ int gficf_cuda_wmu_markers_csc(const int32_t* colptr, const int32_t* row, const 
                                int64_t n_cells, const int32_t* cluster, int32_t n_clusters, double* out, char* err,
                                size_t errlen);
 
+/* gficf_cuda_wmu_markers_csc on several devices of this process: the same arguments and result, bit for bit,
+ * for every n_devices (0 = the count set by gficf_cuda_set_devices / GFICF_CUDA_DEVICES).  D = min(n_devices,
+ * n_genes) devices, 0 .. D - 1, take part, so each owns at least one gene; D = 1 is gficf_cuda_wmu_markers_csc.
+ * The cells are cut into D column slabs of about nnz / D stored values each; device r uploads its slab (and the
+ * per-cell cluster arrays) and makes it gene-major.  The genes are cut into D ranges balanced by stored values;
+ * each device receives its genes' blocks from every slab (NCCL point to point), puts them back in cell order and
+ * runs the rank and means kernels on its genes alone.  A gene's result depends only on its own values in cell
+ * order, which is why the result does not change.
+ * Device memory per device: the single-device figure above with its slab's stored values, cells, and its own
+ * genes (results and sort scratch), plus 24 bytes per stored value of its genes (the blocks received, then
+ * regrouped) and the 12 bytes per cell of the cluster arrays, which every device holds.
+ * Timings (gficf_cuda_last_timings; the maximum over the devices): [0] upload, [1] transpose, [2] regroup +
+ * rank + means, [4] wall time of the call, [5] exchange.
+ * Errors as gficf_cuda_wmu_markers_csc (a bad row id in any slab is GFICF_E_ARG, raised before the exchange),
+ * and GFICF_E_ARG for n_devices < 0 or more devices than are visible; GFICF_E_NCCL when D > 1 and libnccl
+ * cannot be loaded.  A failure on any device fails the call; the next call works. */
+int gficf_cuda_wmu_markers_csc_devices(const int32_t* colptr, const int32_t* row, const double* x, int64_t n_genes,
+                                       int64_t n_cells, const int32_t* cluster, int32_t n_clusters,
+                                       int32_t n_devices, double* out, char* err, size_t errlen);
+
 /* ---- the data-parallel pieces of the community detection that reads the graph (SURVEY 8f row 3;
  * reference src/ModularityOptimizer.cpp).  The sequential, RNG-ordered local moving loop (:484-583)
  * stays on the host; these are the steps around it that touch every edge:

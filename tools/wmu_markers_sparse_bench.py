@@ -5,6 +5,10 @@ bitwise comparison of the two; then a scale case the dense call cannot take (its
 clocks around calls that return with the result on the host; the kernel split comes from torch.profiler in a
 pass of its own.
     python tools/wmu_markers_sparse_bench.py [out.json] [scale_genes scale_cells scale_density]
+With --devices 1,2,4,8 it runs only the scale case, once per device count (gficf_cuda_wmu_markers_csc_devices;
+1 is the single-device call), in rounds that alternate the order of the counts, and checks that every count gives
+the bits of the single-device call:
+    python tools/wmu_markers_sparse_bench.py --devices 1,2,4,8 [out.json] [scale_genes scale_cells scale_density]
 """
 import json, os, resource, subprocess, sys, time
 import numpy as np
@@ -12,6 +16,11 @@ import scipy.sparse as sp
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import gficf_b200
 
+DEVICES = None
+if "--devices" in sys.argv:
+    i = sys.argv.index("--devices")
+    DEVICES = [int(v) for v in sys.argv[i + 1].split(",")]
+    del sys.argv[i:i + 2]
 out_json = sys.argv[1] if len(sys.argv) > 1 else None
 S_GENES = int(sys.argv[2]) if len(sys.argv) > 2 else 20_000
 S_CELLS = int(sys.argv[3]) if len(sys.argv) > 3 else 500_000
@@ -56,7 +65,85 @@ def profile_kernels(fn):
     return dict(sorted(ms.items(), key=lambda kv: -kv[1]))
 
 
+def scale_matrix():
+    """The scale case, generated column by column in CSC form (geometric gaps between stored rows), never dense.
+    Generation peaks at about 30 bytes of host memory per stored value: fewer cells when the host lacks it."""
+    global S_CELLS
+    avail = int(open("/proc/meminfo").read().split("MemAvailable:")[1].split()[0]) * 1024
+    while S_GENES * S_CELLS * S_DENS * 30 > 0.6 * avail:
+        S_CELLS //= 2
+    rng = np.random.default_rng(2)
+    lib = rng.uniform(0.5, 2.0, size=S_CELLS)
+    indptr = np.zeros(S_CELLS + 1, dtype=np.int64)
+    rows_chunks, x_chunks = [], []
+    chunk = 2000
+    L = int(S_GENES * S_DENS + 8 * np.sqrt(S_GENES * S_DENS) + 64)
+    for j0 in range(0, S_CELLS, chunk):
+        j1 = min(S_CELLS, j0 + chunk)
+        r = np.cumsum(rng.geometric(S_DENS, size=(j1 - j0, L)), axis=1) - 1
+        keep = r < S_GENES
+        cnt = keep.sum(axis=1)
+        rr = r[keep].astype(np.int32)
+        vals = (1 + rng.poisson(0.5, size=rr.size)) * (1e6 / 5000.0) / np.repeat(lib[j0:j1], cnt)
+        rows_chunks.append(rr)
+        x_chunks.append(vals)
+        indptr[j0 + 1:j1 + 1] = cnt
+    indptr = np.cumsum(indptr)
+    rows = np.concatenate(rows_chunks)
+    del rows_chunks
+    x = np.concatenate(x_chunks)
+    del x_chunks
+    return sp.csc_matrix((x, rows, indptr.astype(np.int32)), shape=(S_GENES, S_CELLS)), labels(rng, S_CELLS)
+
+
+def device_scaling(devices, rounds=3):
+    """Every device count on the scale case, warmed up once each (workspaces, NCCL communicators), then `rounds`
+    rounds in alternating order.  Phases from gficf_cuda_last_timings (maximum over the devices): upload,
+    transpose, exchange, regroup + rank + means; the single-device call reports its transpose inside `kernels`."""
+    vis = gficf_b200.lib().gficf_cuda_device_count()
+    skipped = [d for d in devices if d > vis]
+    devices = [d for d in devices if d <= vis]
+    t_gen = time.perf_counter()
+    big, cl = scale_matrix()
+    t_gen = time.perf_counter() - t_gen
+    run = lambda d: gficf_b200.rcpp_parallel_WMU_markers_sparse(big, cl, n_devices=d)  # noqa: E731
+    ref = run(1)
+    same = {}
+    for d in devices:
+        same[d] = bool(np.array_equal(run(d).view(np.int64), ref.view(np.int64)))
+    calls = {d: [] for d in devices}
+    for rep in range(rounds):
+        for d in (devices if rep % 2 == 0 else devices[::-1]):
+            t0 = time.perf_counter()
+            out = run(d)
+            dt = (time.perf_counter() - t0) * 1e3
+            tm = gficf_b200.last_timings()
+            same[d] = same[d] and bool(np.array_equal(out.view(np.int64), ref.view(np.int64)))
+            calls[d].append({"call_ms": dt, "wall_ms": tm["wall_ms"], "h2d_ms": tm["h2d_ms"],
+                             "transpose_ms": tm["layout_ms"], "exchange_ms": tm["allgather_ms"],
+                             "kernels_ms": tm["jaccard_ms"],
+                             "device_ms": tm["layout_ms"] + tm["allgather_ms"] + tm["jaccard_ms"]})
+    best = {d: min(calls[d], key=lambda r: r["call_ms"]) for d in devices}
+    return {"genes": S_GENES, "cells": S_CELLS, "clusters": K, "nnz": int(big.nnz),
+            "density": big.nnz / (S_GENES * S_CELLS), "generation_s": t_gen, "visible_devices": vis,
+            "skipped_devices": skipped, "calls": calls, "best": best,
+            "speedup_call": {d: best[1]["call_ms"] / best[d]["call_ms"] for d in devices} if 1 in devices else None,
+            "speedup_device": {d: best[1]["device_ms"] / best[d]["device_ms"] for d in devices} if 1 in devices else None,
+            "bitwise_equal_to_one_device": same,
+            "timing": "host clock around each call (call_ms); the library's CUDA events, the maximum over the devices "
+                      "of each phase (device_ms = transpose + exchange + regroup/rank/means; for one device the "
+                      "transpose is inside kernels_ms); best of the rounds by call_ms"}
+
+
 res = {"card": card()}
+if DEVICES:
+    res["devices"] = device_scaling(DEVICES)
+    print(json.dumps(res), flush=True)
+    if out_json:
+        os.makedirs(os.path.dirname(os.path.abspath(out_json)), exist_ok=True)
+        with open(out_json, "w") as f:
+            json.dump(res, f, indent=1)
+    sys.exit(0)
 
 # ---- r03 workload: 2000 x 100 000, 20 clusters (tools/wmu_markers_bench.py, seed 1)
 genes, N = 2000, 100_000
@@ -81,37 +168,11 @@ res["r03"] = {
 del m, mat, dense_out, sparse_out
 print(json.dumps(res["r03"]), flush=True)
 
-# ---- scale case: generated column by column in CSC form (geometric gaps between stored rows), never dense.
-#      Generation peaks at about 30 bytes of host memory per stored value: fewer cells when the host lacks it.
+# ---- scale case
 import torch
-avail = int(open("/proc/meminfo").read().split("MemAvailable:")[1].split()[0]) * 1024
-while S_GENES * S_CELLS * S_DENS * 30 > 0.6 * avail:
-    S_CELLS //= 2
-rng = np.random.default_rng(2)
-lib = rng.uniform(0.5, 2.0, size=S_CELLS)
-indptr = np.zeros(S_CELLS + 1, dtype=np.int64)
-rows_chunks, x_chunks = [], []
-chunk = 2000
-L = int(S_GENES * S_DENS + 8 * np.sqrt(S_GENES * S_DENS) + 64)
 t_gen = time.perf_counter()
-for j0 in range(0, S_CELLS, chunk):
-    j1 = min(S_CELLS, j0 + chunk)
-    r = np.cumsum(rng.geometric(S_DENS, size=(j1 - j0, L)), axis=1) - 1
-    keep = r < S_GENES
-    cnt = keep.sum(axis=1)
-    rr = r[keep].astype(np.int32)
-    vals = (1 + rng.poisson(0.5, size=rr.size)) * (1e6 / 5000.0) / np.repeat(lib[j0:j1], cnt)
-    rows_chunks.append(rr)
-    x_chunks.append(vals)
-    indptr[j0 + 1:j1 + 1] = cnt
-indptr = np.cumsum(indptr)
-rows = np.concatenate(rows_chunks)
-del rows_chunks
-x = np.concatenate(x_chunks)
-del x_chunks
-big = sp.csc_matrix((x, rows, indptr.astype(np.int32)), shape=(S_GENES, S_CELLS))
+big, cl = scale_matrix()
 t_gen = time.perf_counter() - t_gen
-cl = labels(rng, S_CELLS)
 assert gficf_b200.lib().gficf_cuda_release() == 0  # empty the workspace so that its growth below is the call's
 free0, total = torch.cuda.mem_get_info()
 calls = []
